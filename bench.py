@@ -45,6 +45,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
+sys.dont_write_bytecode = True          # the benchmark may run from a read-only tree: no __pycache__ beside the sources
 
 H, W, C, R, LEVELS, GR = 48, 64, 128, 3, 4, 4
 P = H * W
@@ -148,6 +149,24 @@ class ClockSampler(threading.Thread):
             return {"sm_mhz": None, "sm_max_mhz": self.max_mhz, "reasons": ["nvml unavailable"]}
         return {"sm_mhz": statistics.median(self.samples), "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons),
                 "samples": len(self.samples)}
+
+
+DUMP_BYTES = 64_000_000                 # --dump-outputs writes at most this much in all
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir, results):
+    """Write each result as out_dir/<name>.npy in float32.  The arrays share DUMP_BYTES equally; one with more entries
+    than its share is written as a 1-D sample: the entries of its flattened form at sorted positions drawn without
+    replacement by numpy.random.default_rng(DUMP_SEED), the same positions on every run with the same arguments."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (DUMP_BYTES - 4096 * len(results)) // (4 * len(results))      # 4096: room for each .npy header
+    for name, t in results.items():
+        a = t.detach().float().cpu().numpy()
+        if a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(DUMP_SEED).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peak():
@@ -767,12 +786,19 @@ def main():
     ap.add_argument("--cpu-edges", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-cuda", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last timed step (corr, offset / mean / cov / den "
+                         "gradients) as DIR/<name>.npy; inputs are seeded, so runs with the same arguments are comparable")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
 
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
+    if a.dump_outputs and (a.impl != "ours" or world > 1):
+        ap.error("--dump-outputs is implemented for the single-GPU step of --impl ours")
     n_gpus = max(world, a.gpus)
     config = {"workload": "frontend_w20_e48" if (a.edges, a.frames) == (48, 20) else f"frontend_w{a.frames}_e{a.edges}",
               "edges_per_gpu": a.edges, "keyframes": a.frames, "fmap": [C, H, W], "levels": LEVELS, "radius": R,
@@ -832,19 +858,26 @@ def main():
     records = []
     t_start, t_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_start.record()
-    for _ in range(a.steps):
+    for i in range(a.steps):
         rec = []
-        wl.step(record=rec)
+        out = wl.step(record=rec)
         records.append(rec)
+        if i + 1 < a.steps:
+            del out                       # only the last step's results outlive the step
     t_end.record()
     torch.cuda.synchronize()
     total_ms = t_start.elapsed_time(t_end)
+    last = {k: out[k] for k in Workload.RESULT_KEYS} if a.dump_outputs else None
+    del out
     # keep the GPU under the same load a little longer so that NVML has something to sample (20 steps are ~30 ms)
     t_load = time.perf_counter()
     while time.perf_counter() - t_load < 0.25:
         wl.step()
         torch.cuda.synchronize()
     sampler.stop_flag = True
+    if last is not None:
+        dump_outputs(a.dump_outputs, last)
+        del last
     per_op = {}
     for rec in records:
         for (n0, e0), (n1, e1) in zip(rec[:-1], rec[1:]):
