@@ -213,6 +213,34 @@ LGU_API int lgu_altcorr_lookup_fused_into(const float* lvl0, const float* lvl1, 
                                   int E, int H, int W, int num_levels, int radius,
                                   int shared_offsets, int apply_mask, void* stream);
 
+/* The backend lookup with its CONSUMER's first layer folded in: update_op's corr_encoder[0:2] = Conv2d(196, 128, 1) + ReLU
+ * (droid_net.py:74-76,115), which factor_graph.py:281-286 runs under fp16 autocast, is evaluated on the 196 x 32 tile
+ * while it is still in shared memory, and only enc [E_out,128,H,W] leaves the SM (786 KB per 48 x 64 edge in fp16
+ * instead of the 1.2 MB of 196-channel rows -- what a rank of the sharded backend ships to the destination).
+ * Precision contract (that of the autocast conv, up to summation order):
+ *   - W and b are rounded to fp16 (round to nearest even) by lgu_pack_conv1x1_f16;
+ *   - every corr value is rounded to fp16 (round to nearest even, as Tensor.half());
+ *   - products are exact in fp32 and accumulated in fp32 (m16n8k16 fp16 tensor-core MMAs, K = 196 padded to 208 with
+ *     zeros); the bias is added in fp32; ReLU propagates NaN like torch.relu;
+ *   - the result is rounded once: to fp16 (round to nearest even) with out_half = 1, or stored as fp32 with out_half = 0.
+ *
+ * lgu_pack_conv1x1_f16: weight [128,196] (out_channels = 128, in_channels = 196 only), bias [128] or NULL (zero) ->
+ *   packed, LGU_CONV1X1_F16_BYTES bytes, 16-byte aligned: the fp16 m16n8k16 A fragments [8 warps][13 k-steps][32 lanes]
+ *   (16 B each), then the fp16-rounded bias as 128 floats.
+ * lgu_altcorr_lookup_enc_into: lgu_altcorr_lookup_fused_into (per-corner gating, shared_offsets, apply_mask, mask_out,
+ *   out_index rows) writing enc instead of corr; boxes0 / boxes1 as in lgu_altcorr_lookup_boxes_into (boxes0 != NULL
+ *   replaces lvl0, which is then ignored; boxes1 != NULL replaces lvl1 and needs boxes0).  enc must be 8-byte aligned.
+ * Both return LGU_ERR_BAD_ARG for null or misaligned pointers and bad sizes before any device work, and
+ * lgu_altcorr_lookup_enc_into returns LGU_ERR_UNSUPPORTED unless num_levels = 4, radius = 3, W % 32 = 0 and H % 8 = 0. */
+#define LGU_CONV1X1_F16_BYTES 53760
+LGU_API int lgu_pack_conv1x1_f16(const float* weight, const float* bias, void* packed, int out_channels, int in_channels,
+                                 void* stream);
+LGU_API int lgu_altcorr_lookup_enc_into(const float* boxes0, const float* boxes1, const float* lvl0, const float* lvl1,
+                                const float* lvl2, const float* lvl3, const float* coords, const float* off0, float* off1,
+                                const void* packed, void* enc, const int32_t* out_index, int out_half, float* mask_out,
+                                int E, int H, int W, int num_levels, int radius,
+                                int shared_offsets, int apply_mask, void* stream);
+
 /* Backward of lgu_corr_lookup_fused = what autograd runs for corr.py:88-109 in training (4 x
  * defCorr_index_backward, the offset[1]*mask / sigmoid / var chain, corr_index_backward), in one launch:
  *   gv0..gv3      dense gradients of the pyramid levels (each written exactly once; level 1 includes the mask path)

@@ -13,6 +13,7 @@ instead.  What differs is underneath:
 
 The learned heads (ofsMap / ofs_residual convs, the GaussianMask MLP) stay torch modules, as in the reference.
 """
+import functools
 import math
 import os
 import weakref
@@ -376,6 +377,15 @@ class _Offsets(list):
         return base, self.cum
 
 
+def _encoder_conv(corr_encoder):
+    """UpdateModule.corr_encoder (droid_net.py:74-78) or its first layer -> that Conv2d(196, 128, 1)."""
+    conv = corr_encoder[0] if isinstance(corr_encoder, nn.Sequential) else corr_encoder
+    if not (isinstance(conv, nn.Conv2d) and conv.kernel_size == (1, 1) and conv.in_channels == 196
+            and conv.out_channels == 128):
+        raise RuntimeError("lookup_encoded needs the 196 -> 128 1x1 corr_encoder conv")
+    return conv
+
+
 # ------------------------------------------------------------------------------------------------
 # CorrBlock
 # ------------------------------------------------------------------------------------------------
@@ -478,10 +488,7 @@ class CorrBlock:
         UpdateModule.corr_encoder (droid_net.py:74-78) or its first conv; returns (enc, mean_n, theta) with
         enc = relu(conv1x1(corr)) [b,n,128,h,w] -- feed it to corr_encoder[2:] -- or (corr, enc, mean_n, theta) with
         keep_corr=True.  The 196-channel tensor is not written unless asked for."""
-        conv = corr_encoder[0] if isinstance(corr_encoder, nn.Sequential) else corr_encoder
-        if not (isinstance(conv, nn.Conv2d) and conv.kernel_size == (1, 1) and conv.in_channels == 196
-                and conv.out_channels == 128):
-            raise RuntimeError("lookup_encoded needs the 196 -> 128 1x1 corr_encoder conv")
+        conv = _encoder_conv(corr_encoder)
         batch, num, ht, wd, _ = coords.shape
         E = batch * num
         if not self._can_fuse_lookup(coords):
@@ -750,7 +757,10 @@ class AltCorrBlock:
         t = torch.cat(((f1 * 4.0).permute(0, 3, 1, 2), (f2 * 4.0).permute(0, 3, 1, 2)), dim=1).float()
         return _generate_offsets(self.ofsMap, self.ofs_residual, t)
 
-    def _corr_materialized(self, coords, ii, jj, out=None, out_index=None, pass_edges=None, pass_hook=None, key=None):
+    def _corr_materialized(self, coords, ii, jj, out=None, out_index=None, pass_edges=None, pass_hook=None, key=None,
+                           enc=None):
+        """enc: fp16 operands of the consumer's first layer (ops.pack_conv1x1_f16); the lookup then returns / writes
+        relu(conv1x1(corr)) [.., 128, H, W] instead of corr."""
         B, N, H, W, S, _ = coords.shape
         # pass_edges: an int (edges per pass) or a sequence of pass sizes (the sharded engine tapers the passes of a rank's
         # last chunk so that only a small shipment is left exposed at the end of the step)
@@ -792,6 +802,7 @@ class AltCorrBlock:
             m0, = ops.altcorr_forward(f1, f2, (c[:1] / 2).view(1, 1, H, W, 2).contiguous(), MASK_RADIUS)
             mask0 = torch.sigmoid(torch.var(m0.permute(0, 1, 3, 4, 2).reshape(1, H, W, 9), dim=3))
             slab0 = (off0[:1].contiguous(), (off1[:1] * mask0.view(1, H, W, 1)).contiguous())
+        lookup = ops.altcorr_lookup_fused if enc is None else functools.partial(ops.altcorr_lookup_encoded, packed=enc)
         outs, masks, new_off1 = [], [], []
         for s, s_end in bounds:
             e = slice(s, s_end)
@@ -823,12 +834,12 @@ class AltCorrBlock:
                                            torch.arange(e.start, e.stop, dtype=torch.int32, device=c.device))) \
                 if out is not None else {}
             if self.strict_ref:
-                o, m = ops.altcorr_lookup_fused(vols, c[e], slab0[0], slab0[1], self.radius, shared_offsets=True,
-                                                apply_mask=False, return_mask=True, boxes0=boxes0, boxes1=boxes1, **dst)
+                o, m = lookup(vols, c[e], slab0[0], slab0[1], self.radius, shared_offsets=True,
+                              apply_mask=False, return_mask=True, boxes0=boxes0, boxes1=boxes1, **dst)
             else:
                 o1 = off1[e].clone()                                      # updated in place: offset[1] * mask
-                o, m = ops.altcorr_lookup_fused(vols, c[e], off0[e].contiguous(), o1, self.radius, shared_offsets=False,
-                                                apply_mask=True, return_mask=True, boxes0=boxes0, boxes1=boxes1, **dst)
+                o, m = lookup(vols, c[e], off0[e].contiguous(), o1, self.radius, shared_offsets=False,
+                              apply_mask=True, return_mask=True, boxes0=boxes0, boxes1=boxes1, **dst)
                 new_off1.append(o1)
             outs.append(o)
             masks.append(m)
@@ -897,3 +908,31 @@ class AltCorrBlock:
         if squeeze:
             corr = corr.squeeze(dim=-1)
         return corr.contiguous()
+
+    @torch.no_grad()
+    def lookup_encoded(self, coords, ii, jj, corr_encoder, out=None, out_index=None, pass_edges=None, pass_hook=None,
+                       key=None):
+        """__call__ with the consumer's first layer folded into the lookup kernel (inference): corr_encoder is
+        UpdateModule.corr_encoder (droid_net.py:74-78) or its first conv.  Returns relu(conv1x1(corr)) [1,E,128,H,W] fp16,
+        evaluated as update_op does under fp16 autocast (factor_graph.py:281-286: operands rounded to fp16, fp32
+        accumulation, relu keeps NaN) -- feed it to corr_encoder[2:].  With out ([E_out,128,H,W], fp16 or fp32) / out_index
+        the rows are written there and `out` is returned, like __call__; pass_edges / pass_hook / key as there, so a
+        ShardedBackendCorr can use this (with corr_encoder bound) as its compute and ship 128 instead of 196 channels per
+        pixel.  Leaves the same `offset` attribute as __call__.  Needs the materialised path (B = S = 1, 4 levels, r = 3,
+        C = 128, W % 32 == 0, H % 8 == 0)."""
+        conv = _encoder_conv(corr_encoder)
+        if coords.dim() == 5:
+            coords = coords.unsqueeze(dim=-2)
+        B, N, H, W, S, _ = coords.shape
+        if not (self.materialize and B == 1 and S == 1):
+            raise RuntimeError("lookup_encoded needs the materialised backend lookup (B = S = 1, 4 levels, r = 3, C = 128, "
+                               "W % 32 == 0, H % 8 == 0)")
+        bias = conv.bias
+        pkey = (id(conv), conv.weight._version, conv.weight.data_ptr(),
+                None if bias is None else (bias._version, bias.data_ptr()))
+        if getattr(self, "_enc_key", None) != pkey:
+            w = conv.weight.detach().to(coords.device, torch.float32)
+            b = bias.detach().to(coords.device, torch.float32) if bias is not None else None
+            self._enc_key, self._enc_packed = pkey, ops.pack_conv1x1_f16(w, b)
+        res = self._corr_materialized(coords, ii, jj, out, out_index, pass_edges, pass_hook, key, enc=self._enc_packed)
+        return res if out is not None else res.view(B, N, -1, H, W)

@@ -125,7 +125,22 @@ __device__ __forceinline__ uint32_t flf_tf32(float x) {
   return r;
 }
 
-template <bool PC, bool HALF, bool CONV = false>
+// CONV: the consumer's first layer evaluated on the staged tile (see FusedLookupParams::conv_w)
+enum ConvMode : int { kConvNone = 0, kConvTF32 = 1, kConvF16 = 2 };
+
+// m16n8k16 fp16 tensor-core MMA on register fragments (D += A * B, fp32 accumulate)
+__device__ __forceinline__ void flf_mma_f16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  asm volatile(
+      "mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
+      : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+__device__ __forceinline__ uint32_t flf_h2(float lo, float hi) {     // round-to-nearest-even, like Tensor.half()
+  const __half2 h = __floats2half2_rn(lo, hi);
+  return *reinterpret_cast<const uint32_t*>(&h);
+}
+
+template <bool PC, bool HALF, int CONV = kConvNone>
 __global__ void __launch_bounds__(fl::kThreads, 2)
 lookup_fused_kernel(const __grid_constant__ FusedMaps maps, const FusedLookupParams prm) {
   using namespace fl;
@@ -419,21 +434,60 @@ lookup_fused_kernel(const __grid_constant__ FusedMaps maps, const FusedLookupPar
     __syncwarp();
     if (has_next && lane == 0) fetch_offsets(npw, nns);
 
+    // kConvF16: the first kPre weight fragments are requested before the barrier and kPre loads stay in flight through
+    // the k-loop (the TMA buffers leave too little L1 for the 53 KB of fragments, so every tile re-reads them from L2;
+    // measured on a B200 at 1000 W: 280.7 against 283.4 us per 48-edge lookup with one load per k-step)
+    constexpr int kPre = 4;
+    uint4 wpre[kPre];
+    if constexpr (CONV == kConvF16) {
+      const uint4* wf = reinterpret_cast<const uint4*>(prm.conv_w) + (size_t)warp * ((CH + 15) / 16) * 32 + lane;
+#pragma unroll
+      for (int d = 0; d < kPre; ++d) wpre[d] = __ldg(wf + d * 32);
+    }
     __syncthreads();
-    if (CONV) {
+    if (CONV != kConvNone) {
       // ---- corr_encoder[0:2] on the staged tile: enc[oc, pixel] = relu(b[oc] + sum_k W[oc, k] * corr[k, pixel]).
-      // Warp w owns output channels 16 w .. 16 w + 15 for all 32 pixels: 4 n-tiles x 25 k-steps of m16n8k8 TF32 MMAs on
-      // register fragments, 3-term split (W = W_hi + W_lo pre-split by lgu_pack_conv1x1, corr = hi + lo split here;
+      // Warp w owns output channels 16 w .. 16 w + 15 for all 32 pixels (4 n-tiles of 8 pixels).
+      // kConvTF32: 25 k-steps of m16n8k8 TF32 MMAs on register fragments, 3-term split (W = W_hi + W_lo pre-split by lgu_pack_conv1x1, corr = hi + lo split here;
       // lo*lo dropped: ~2^-22 relative per product, fp32 accumulation) -> <= 1e-5 of F.conv2d in fp32 for O(1..10) values.
       // (tcgen05 would want W_hi / W_lo in tensor memory -- 392 of the 512 columns an SM shares between its two resident
       // CTAs -- and UMMA-layout copies of the tile next to a 107 KB TMA ring: neither fits, and 3.7 GFLOP-equivalent per
       // 48-edge lookup is far from the legacy tensor path's limit.)
-      constexpr int KS = (CH + 7) / 8;                          // 25 k-steps; rows 196..199 are zero
+      // kConvF16 (the backend lookup): what the consumer's conv computes under fp16 autocast (factor_graph.py:281-286) --
+      // W and b rounded to fp16 by lgu_pack_conv1x1_f16, the staged corr values rounded to fp16 here (round to nearest
+      // even), products exact in fp32, fp32 accumulation, one rounding of the output: 13 k-steps of m16n8k16 MMAs
+      // (52 per warp and tile), K padded to 208 with zero rows.  (tcgen05 .kind::f16 with W in tensor memory needs
+      // 104 + 32 columns per CTA, which fits; but its B operand is an fp16 UMMA-layout copy of the tile in shared memory:
+      // 13,312 B more per CTA is 2 x 120,912 B, beyond the SM's 228 KB at two CTAs, and writing the pass loop's results
+      // in that layout instead would change the code every other instantiation shares.)
       float acc[4][4];
 #pragma unroll
       for (int nt = 0; nt < 4; ++nt) { acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.0f; }
-      const float4* wf = prm.conv_w + ((size_t)warp * KS * 32 + lane) * 2;
       const int kq = lane & 3, nq = lane >> 2;
+      if constexpr (CONV == kConvF16) {
+        constexpr int KS16 = (CH + 15) / 16;                    // 13 k-steps; rows 196..207 are zero
+        const uint4* wf = reinterpret_cast<const uint4*>(prm.conv_w) + (size_t)warp * KS16 * 32 + lane;
+#pragma unroll
+        for (int ks = 0; ks < KS16; ++ks) {
+          const uint4 w = wpre[ks % kPre];
+          if (ks + kPre < KS16) wpre[ks % kPre] = __ldg(wf + (ks + kPre) * 32);
+          const uint32_t a[4] = {w.x, w.y, w.z, w.w};
+          // B fragment: rows k0, k0 + 1 (b0) and k0 + 8, k0 + 9 (b1) of pixel column nt * 8 + nq; CH is even, so a pair
+          // is either inside the 196 channels or entirely padding
+          const int k0 = ks * 16 + 2 * kq, k1 = k0 + 8;
+          const bool v0 = k0 < CH, v1 = k1 < CH;
+          const float* r0 = s_out + (v0 ? k0 : 0) * kOutPitch + nq;
+          const float* r1 = s_out + (v1 ? k1 : 0) * kOutPitch + nq;
+#pragma unroll
+          for (int nt = 0; nt < 4; ++nt) {
+            const uint32_t b0 = v0 ? flf_h2(r0[nt * 8], r0[kOutPitch + nt * 8]) : 0u;
+            const uint32_t b1 = v1 ? flf_h2(r1[nt * 8], r1[kOutPitch + nt * 8]) : 0u;
+            flf_mma_f16(acc[nt], a, b0, b1);
+          }
+        }
+      } else {
+      constexpr int KS = (CH + 7) / 8;                          // 25 k-steps; rows 196..199 are zero
+      const float4* wf = prm.conv_w + ((size_t)warp * KS * 32 + lane) * 2;
 #pragma unroll 1
       for (int ks = 0; ks < KS; ++ks) {
         const float4 whi = __ldg(wf + (size_t)ks * 64), wlo = __ldg(wf + (size_t)ks * 64 + 1);
@@ -453,6 +507,7 @@ lookup_fused_kernel(const __grid_constant__ FusedMaps maps, const FusedLookupPar
           flf_mma_tf32(acc[nt], ahi, h0, h1);
         }
       }
+      }
       // C fragment: rows oc0 + nq (c0, c1) and oc0 + nq + 8 (c2, c3), pixels nt * 8 + 2 kq + {0, 1}
       const int p0 = pw - warp * kPixPerWarp;
       const int oc_a = warp * 16 + nq, oc_b = oc_a + 8;
@@ -462,7 +517,11 @@ lookup_fused_kernel(const __grid_constant__ FusedMaps maps, const FusedLookupPar
 #pragma unroll
       for (int nt = 0; nt < 4; ++nt) {
         float e0 = acc[nt][0] + ba, e1 = acc[nt][1] + ba, e2 = acc[nt][2] + bb, e3 = acc[nt][3] + bb;
-        if (prm.conv_relu) { e0 = fmaxf(e0, 0.0f); e1 = fmaxf(e1, 0.0f); e2 = fmaxf(e2, 0.0f); e3 = fmaxf(e3, 0.0f); }
+        if (CONV == kConvF16) {                                 // torch.relu: NaN stays NaN
+          e0 = e0 < 0.0f ? 0.0f : e0; e1 = e1 < 0.0f ? 0.0f : e1; e2 = e2 < 0.0f ? 0.0f : e2; e3 = e3 < 0.0f ? 0.0f : e3;
+        } else if (prm.conv_relu) {
+          e0 = fmaxf(e0, 0.0f); e1 = fmaxf(e1, 0.0f); e2 = fmaxf(e2, 0.0f); e3 = fmaxf(e3, 0.0f);
+        }
         if (HALF) {
           __half* enc = reinterpret_cast<__half*>(prm.enc) + erow + nt * 8;
           *reinterpret_cast<__half2*>(enc + (size_t)oc_a * P) = __floats2half2_rn(e0, e1);
@@ -474,7 +533,7 @@ lookup_fused_kernel(const __grid_constant__ FusedMaps maps, const FusedLookupPar
         }
       }
     }
-    if (!CONV || prm.out != nullptr) {
+    if (CONV == kConvNone || prm.out != nullptr) {
       const int p0 = pw - warp * kPixPerWarp;
       const size_t row = (size_t)(prm.out_index != nullptr ? __ldg(prm.out_index + n) : n) * CH * P + p0 + lane;
       const float* srow = s_out + lane;
@@ -501,6 +560,7 @@ struct ConvArgs {
   const float* b;
   void* enc;
   int relu;
+  int f16;       // 1: fp16 fragments of lgu_pack_conv1x1_f16 (kConvF16), 0: TF32 hi/lo fragments (kConvTF32)
 };
 static int launch_lookup_fused(const float* lvl0, const float* lvl1, const float* lvl2, const float* lvl3,
                                const float* coords, const float* off0, float* off1, float* corr, float* mask_out, int E,
@@ -527,6 +587,60 @@ __global__ void pack_conv1x1_kernel(const float* __restrict__ W, float4* __restr
   frag[(size_t)t * 2 + 1] = make_float4(lo[0], lo[1], lo[2], lo[3]);
 }
 }
+namespace lgu {
+constexpr int kF16FragBytes = 8 * 13 * 32 * 16;                     // 53,248 B; the fp16-rounded bias follows as 128 floats
+static_assert(kF16FragBytes + 128 * 4 == LGU_CONV1X1_F16_BYTES, "lgu_corr.h: LGU_CONV1X1_F16_BYTES");
+// W [128, K] (K <= 208), b [128] or null -> the m16n8k16 fp16 A fragments of the kConvF16 epilogue, [8 warps][13 k-steps]
+// [32 lanes]{a0..a3} (a_r = halves (row, col), (row, col + 1): rows g, g + 8, g, g + 8 and columns 2 t, 2 t, 2 t + 8,
+// 2 t + 8 of the warp's 16 x 16 block; g = lane / 4, t = lane % 4), then fp32(fp16(b)) for the 128 channels
+__global__ void pack_conv1x1_f16_kernel(const float* __restrict__ W, const float* __restrict__ b, uint4* __restrict__ frag,
+                                        float* __restrict__ bias16, int K) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < 128) bias16[t] = b != nullptr ? __half2float(__float2half_rn(b[t])) : 0.0f;
+  if (t >= 8 * 13 * 32) return;
+  const int lane = t & 31, ks = (t >> 5) % 13, w = t / (13 * 32);
+  const int g = lane >> 2, c0 = ks * 16 + 2 * (lane & 3);
+  uint32_t r[4];
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    const int row = w * 16 + g + (q & 1) * 8, col = c0 + (q >> 1) * 8;
+    const float lo = col < K ? W[(size_t)row * K + col] : 0.0f, hi = col + 1 < K ? W[(size_t)row * K + col + 1] : 0.0f;
+    const __half2 h = __floats2half2_rn(lo, hi);
+    r[q] = *reinterpret_cast<const uint32_t*>(&h);
+  }
+  frag[t] = make_uint4(r[0], r[1], r[2], r[3]);
+}
+}  // namespace lgu
+extern "C" int lgu_pack_conv1x1_f16(const float* weight, const float* bias, void* packed, int out_channels, int in_channels,
+                                    void* stream) {
+  LGU_REQUIRE(weight && packed, "lgu_pack_conv1x1_f16: null pointer");
+  LGU_REQUIRE((reinterpret_cast<uintptr_t>(packed) & 15) == 0, "lgu_pack_conv1x1_f16: packed must be 16-byte aligned");
+  LGU_REQUIRE(out_channels == 128 && in_channels == 196,
+              "lgu_pack_conv1x1_f16: only the 196 -> 128 corr_encoder is implemented (got %d -> %d)", in_channels, out_channels);
+  uint8_t* p = static_cast<uint8_t*>(packed);
+  lgu::pack_conv1x1_f16_kernel<<<(8 * 13 * 32 + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
+      weight, bias, reinterpret_cast<uint4*>(p), reinterpret_cast<float*>(p + lgu::kF16FragBytes), in_channels);
+  return lgu::check_launch("lgu_pack_conv1x1_f16");
+}
+extern "C" int lgu_altcorr_lookup_enc_into(const float* boxes0, const float* boxes1, const float* lvl0, const float* lvl1,
+                                           const float* lvl2, const float* lvl3, const float* coords, const float* off0,
+                                           float* off1, const void* packed, void* enc, const int32_t* out_index, int out_half,
+                                           float* mask_out, int E, int H, int W, int num_levels, int radius,
+                                           int shared_offsets, int apply_mask, void* stream) {
+  LGU_REQUIRE(E >= 0, "lgu_altcorr_lookup_enc_into: bad sizes E=%d", E);
+  if (E == 0) return LGU_OK;
+  LGU_REQUIRE(packed != nullptr && enc != nullptr, "lgu_altcorr_lookup_enc_into: null pointer");
+  LGU_REQUIRE((reinterpret_cast<uintptr_t>(packed) & 15) == 0 && (reinterpret_cast<uintptr_t>(enc) & 7) == 0,
+              "lgu_altcorr_lookup_enc_into: packed must be 16-byte and enc 8-byte aligned");
+  LGU_REQUIRE(boxes0 != nullptr || lvl0 != nullptr, "lgu_altcorr_lookup_enc_into: null pointer (level 0 needs boxes or a volume)");
+  LGU_REQUIRE(boxes1 != nullptr || lvl1 != nullptr, "lgu_altcorr_lookup_enc_into: null pointer (level 1 needs boxes or a volume)");
+  const uint8_t* p = static_cast<const uint8_t*>(packed);
+  const lgu::ConvArgs conv = {reinterpret_cast<const float4*>(p), reinterpret_cast<const float*>(p + lgu::kF16FragBytes), enc,
+                              1, 1};
+  return lgu::launch_lookup_fused(boxes0 != nullptr ? nullptr : lvl0, lvl1, lvl2, lvl3, coords, off0, off1, nullptr,
+                                  mask_out, E, H, W, num_levels, radius, 1, shared_offsets, apply_mask, nullptr, E, nullptr,
+                                  out_index, out_half, stream, &conv, boxes0, boxes1);
+}
 extern "C" int lgu_pack_conv1x1(const float* weight, float* wfrag, int out_channels, int in_channels, void* stream) {
   LGU_REQUIRE(weight && wfrag, "lgu_pack_conv1x1: null pointer");
   LGU_REQUIRE(out_channels == 128 && in_channels == 196, "lgu_pack_conv1x1: only the 196 -> 128 corr_encoder is implemented");
@@ -544,7 +658,7 @@ extern "C" int lgu_corr_lookup_fused_enc(const float* lvl0, const float* lvl1, c
   LGU_REQUIRE((reinterpret_cast<uintptr_t>(wfrag) & 15) == 0 && (reinterpret_cast<uintptr_t>(enc) & 7) == 0,
               "lgu_corr_lookup_fused_enc: wfrag must be 16-byte and enc 8-byte aligned");
   LGU_REQUIRE(!(out_half && corr != nullptr), "lgu_corr_lookup_fused_enc: fp16 output applies to enc only (pass corr = NULL)");
-  const lgu::ConvArgs conv = {reinterpret_cast<const float4*>(wfrag), bias, enc, relu};
+  const lgu::ConvArgs conv = {reinterpret_cast<const float4*>(wfrag), bias, enc, relu, 0};
   return lgu::launch_lookup_fused(lvl0, lvl1, lvl2, lvl3, coords, off0, const_cast<float*>(off1), corr, mask_out, E, H, W,
                                   num_levels, radius, 0, 0, 1, slots, slots != nullptr ? num_slots : E, cum_mask, nullptr,
                                   out_half, stream, &conv);
@@ -668,9 +782,12 @@ static int lgu::launch_lookup_fused(const float* lvl0, const float* lvl1, const 
   LGU_REQUIRE(!(shared_offsets && apply_mask), "lgu_*_lookup_fused: apply_mask needs per-edge offsets");
   auto kern = per_corner ? (out_half ? lookup_fused_kernel<true, true> : lookup_fused_kernel<true, false>)
                          : (out_half ? lookup_fused_kernel<false, true> : lookup_fused_kernel<false, false>);
-  if (conv != nullptr) {
+  if (conv != nullptr && conv->f16) {
+    LGU_REQUIRE(per_corner, "lgu_*_lookup_enc: the fp16 encoder is implemented for the backend lookup");
+    kern = out_half ? lookup_fused_kernel<true, true, kConvF16> : lookup_fused_kernel<true, false, kConvF16>;
+  } else if (conv != nullptr) {
     LGU_REQUIRE(!per_corner, "lgu_corr_lookup_fused_enc: the fused encoder is implemented for the CorrBlock lookup");
-    kern = out_half ? lookup_fused_kernel<false, true, true> : lookup_fused_kernel<false, false, true>;
+    kern = out_half ? lookup_fused_kernel<false, true, kConvTF32> : lookup_fused_kernel<false, false, kConvTF32>;
   }
   if (int rc = optin_smem(reinterpret_cast<const void*>(kern), flf::kFwdSmemBytes, "lgu_corr_lookup_fused")) return rc;
   kern<<<(unsigned)nblk, fl::kThreads, flf::kFwdSmemBytes, (cudaStream_t)stream>>>(maps, prm);

@@ -727,15 +727,8 @@ def build_volume(f1_hi, f1_lo, f2_hi, f2_lo, ii, jj, half_mask=None):
     return vol
 
 
-def altcorr_lookup_fused(volumes, coords, off0, off1, radius=3, shared_offsets=False, apply_mask=True,
-                         return_mask=False, out=None, out_index=None, boxes0=None, boxes1=None):
-    """corr_lookup_fused with the backend samplers' semantics (per-corner gating, quirk Q4; lowMem_defSample.cu /
-    altcorr_kernel.cu).  volumes: 4 tensors [E,H,W,H>>l,W>>l] from build_volume.  shared_offsets: every edge reads
-    offset slab 0 (quirk Q2; off0/off1 then hold >= 1 slab); apply_mask=False: off1 is used as given.
-    out: destination [E_out,196,H,W], fp32 or fp16 (rounded to nearest), possibly peer memory of another GPU mapped
-    into this process; out_index int32 [E]: row of `out` that receives edge e (default: e).  Returns `out` then.
-    boxes0 [E,H*W,16,20] (build_boxes): level 0 as compact per-pixel boxes; volumes[0] is then ignored (may be None);
-    boxes1: the same for level 1 (needs boxes0)."""
+def _check_altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1):
+    """Shapes / dtypes / layout of the backend lookup's inputs; returns (E, H, W)."""
     E, H, W = volumes[2].shape[:3]
     if boxes1 is not None and boxes0 is None:
         raise RuntimeError("boxes1 needs boxes0")
@@ -756,17 +749,35 @@ def altcorr_lookup_fused(volumes, coords, off0, off1, radius=3, shared_offsets=F
         if not (isinstance(o, torch.Tensor) and o.is_cuda and o.is_contiguous() and o.dtype == torch.float32
                 and o.numel() >= need):
             raise RuntimeError(f"{name} must be a contiguous fp32 CUDA tensor with >= {need} elements")
+    return E, H, W
+
+
+def _check_out_rows(out, out_index, E, C, H, W, device):
+    """A caller-owned destination [E_out,C,H,W] (fp32 / fp16) and its optional int32 row index, one row per edge."""
+    if not (isinstance(out, torch.Tensor) and out.is_cuda and out.is_contiguous() and out.dim() == 4
+            and tuple(out.shape[1:]) == (C, H, W) and out.dtype in (torch.float32, torch.float16)):
+        raise RuntimeError(f"out must be a contiguous CUDA tensor [E_out,{C},H,W], fp32 or fp16")
+    if out_index is not None:
+        if not (out_index.is_cuda and out_index.dtype == torch.int32 and out_index.is_contiguous()
+                and out_index.numel() == E and out_index.device == device):
+            raise RuntimeError("out_index must be a contiguous CUDA int32 vector with one row per edge")
+    elif out.shape[0] < E:
+        raise RuntimeError(f"out has {out.shape[0]} rows, {E} edges")
+
+
+def altcorr_lookup_fused(volumes, coords, off0, off1, radius=3, shared_offsets=False, apply_mask=True,
+                         return_mask=False, out=None, out_index=None, boxes0=None, boxes1=None):
+    """corr_lookup_fused with the backend samplers' semantics (per-corner gating, quirk Q4; lowMem_defSample.cu /
+    altcorr_kernel.cu).  volumes: 4 tensors [E,H,W,H>>l,W>>l] from build_volume.  shared_offsets: every edge reads
+    offset slab 0 (quirk Q2; off0/off1 then hold >= 1 slab); apply_mask=False: off1 is used as given.
+    out: destination [E_out,196,H,W], fp32 or fp16 (rounded to nearest), possibly peer memory of another GPU mapped
+    into this process; out_index int32 [E]: row of `out` that receives edge e (default: e).  Returns `out` then.
+    boxes0 [E,H*W,16,20] (build_boxes): level 0 as compact per-pixel boxes; volumes[0] is then ignored (may be None);
+    boxes1: the same for level 1 (needs boxes0)."""
+    E, H, W = _check_altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1)
     mask = torch.empty(E, H, W, dtype=torch.float32, device=coords.device) if return_mask else None
     if out is not None:
-        if not (isinstance(out, torch.Tensor) and out.is_cuda and out.is_contiguous() and out.dim() == 4
-                and tuple(out.shape[1:]) == (196, H, W) and out.dtype in (torch.float32, torch.float16)):
-            raise RuntimeError("out must be a contiguous CUDA tensor [E_out,196,H,W], fp32 or fp16")
-        if out_index is not None:
-            if not (out_index.is_cuda and out_index.dtype == torch.int32 and out_index.is_contiguous()
-                    and out_index.numel() == E and out_index.device == coords.device):
-                raise RuntimeError("out_index must be a contiguous CUDA int32 vector with one row per edge")
-        elif out.shape[0] < E:
-            raise RuntimeError(f"out has {out.shape[0]} rows, {E} edges")
+        _check_out_rows(out, out_index, E, 196, H, W, coords.device)
         null = ctypes.c_void_p(0)
         if boxes0 is not None:
             head = (_p(boxes0), _p(boxes1) if boxes1 is not None else null, _p(volumes[1]) if boxes1 is None else null)
@@ -801,3 +812,63 @@ def altcorr_lookup_fused(volumes, coords, off0, off1, radius=3, shared_offsets=F
                                                  _i(1 if apply_mask else 0), _stream(coords))
     _lib.check(st, "altcorr_lookup_fused")
     return (corr, mask) if return_mask else corr
+
+
+CONV1X1_F16_BYTES = 53760            # LGU_CONV1X1_F16_BYTES
+
+
+def pack_conv1x1_f16(weight, bias=None):
+    """corr_encoder[0] weight [128,196] (or [128,196,1,1]) and bias [128] (or None) -> the fp16 operands of the backend
+    lookup's encoder epilogue (altcorr_lookup_encoded): both rounded to fp16 as autocast does, weight in m16n8k16
+    A-fragment order.  A uint8 CUDA tensor of CONV1X1_F16_BYTES bytes."""
+    if not (isinstance(weight, torch.Tensor) and weight.is_cuda and weight.dtype == torch.float32):
+        raise RuntimeError("weight must be a CUDA fp32 tensor")
+    w = weight.detach().reshape(weight.shape[0], -1).contiguous()
+    if tuple(w.shape) != (128, 196):
+        raise RuntimeError(f"only the 196 -> 128 corr_encoder is implemented, got weight {tuple(weight.shape)}")
+    if bias is not None:
+        if not (isinstance(bias, torch.Tensor) and bias.is_cuda and bias.dtype == torch.float32 and bias.numel() == 128
+                and bias.device == w.device):
+            raise RuntimeError("bias must be a CUDA fp32 vector of 128 on the weight's device")
+        bias = bias.detach().contiguous()
+    packed = torch.empty(CONV1X1_F16_BYTES, dtype=torch.uint8, device=w.device)
+    with torch.cuda.device(w.device):
+        st = _lib.lib().lgu_pack_conv1x1_f16(_p(w), _p(bias) if bias is not None else ctypes.c_void_p(0), _p(packed),
+                                             _i(128), _i(196), _stream(w))
+    _lib.check(st, "pack_conv1x1_f16")
+    return packed
+
+
+def altcorr_lookup_encoded(volumes, coords, off0, off1, radius=3, shared_offsets=False, apply_mask=True,
+                           return_mask=False, out=None, out_index=None, boxes0=None, boxes1=None, packed=None):
+    """altcorr_lookup_fused with update_op's corr_encoder[0:2] = relu(Conv2d(196,128,1)) folded into the kernel, evaluated
+    as under fp16 autocast (operands rounded to fp16, fp32 accumulation, one rounding of the output; relu keeps NaN):
+    only the 128-channel result leaves the SM.  packed: from pack_conv1x1_f16.  Same inputs, side effects and row
+    placement as altcorr_lookup_fused; out: [E_out,128,H,W] fp16 or fp32.  Without out, returns a new
+    [E,128,H,W] fp16 tensor."""
+    E, H, W = _check_altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1)
+    if not (isinstance(packed, torch.Tensor) and packed.is_cuda and packed.dtype == torch.uint8 and packed.is_contiguous()
+            and packed.numel() == CONV1X1_F16_BYTES and packed.device == coords.device):
+        raise RuntimeError("packed must come from pack_conv1x1_f16 (on the coords' device)")
+    if packed.data_ptr() % 16:
+        raise RuntimeError("packed must be 16-byte aligned")
+    if out is None:
+        out = torch.empty(E, 128, H, W, dtype=torch.float16, device=coords.device)
+        out_index = None
+    else:
+        _check_out_rows(out, out_index, E, 128, H, W, coords.device)
+    if out.data_ptr() % 8:
+        raise RuntimeError("out must be 8-byte aligned")
+    mask = torch.empty(E, H, W, dtype=torch.float32, device=coords.device) if return_mask else None
+    null = ctypes.c_void_p(0)
+    vol = lambda l: null if volumes[l] is None or (l == 0 and boxes0 is not None) or (l == 1 and boxes1 is not None) \
+        else _p(volumes[l])
+    with torch.cuda.device(coords.device):
+        st = _lib.lib().lgu_altcorr_lookup_enc_into(
+            _p(boxes0) if boxes0 is not None else null, _p(boxes1) if boxes1 is not None else null, vol(0), vol(1), vol(2),
+            vol(3), _p(coords), _p(off0), _p(off1), _p(packed), _p(out),
+            _p(out_index) if out_index is not None else null, _i(out.dtype == torch.float16),
+            _p(mask) if return_mask else null, _i(E), _i(H), _i(W), _i(4), _i(radius), _i(1 if shared_offsets else 0),
+            _i(1 if apply_mask else 0), _stream(coords))
+    _lib.check(st, "altcorr_lookup_encoded")
+    return (out, mask) if return_mask else out
