@@ -253,8 +253,7 @@ LGU_API int lgu_altcorr_lookup_enc_into(const float* boxes0, const float* boxes1
  * e = exponent of the pixel's largest upstream |gradient|; native integer shared-memory adds, order-independent, no
  * overflow even if all 196 corners collide): |error| <= 2^-24 * max|g| per contribution, i.e. <= 1e-5 abs for the
  * O(1)..O(10) gradients of training, and bit-reproducible from run to run.  Pixels with non-finite gradients or NaN
- * sampling positions take the fp32 compare-and-swap path (NaNs propagate as in the reference).
- * LGU_BWD_FLOAT_ATOMICS=1 selects that path everywhere. */
+ * sampling positions take the fp32 compare-and-swap path (NaNs propagate as in the reference). */
 LGU_API int lgu_corr_lookup_fused_backward(const float* lvl0, const float* lvl1, const float* coords,
                                    const float* off0, const float* off1_out, const float* mask,
                                    const float* corr_grad, const float* off1_out_grad,

@@ -15,7 +15,6 @@ The learned heads (ofsMap / ofs_residual convs, the GaussianMask MLP) stay torch
 """
 import functools
 import math
-import os
 import weakref
 
 import torch
@@ -701,10 +700,10 @@ class AltCorrBlock:
         `clear_cache()` drops everything (call it when the feature maps change)."""
         self.cache = bool(cache)
         self.sparse_volumes = bool(sparse_volumes)
-        # 0: volumes only; 1 (default): level 0 as compact boxes; 2: levels 0 and 1 -- measured slower (46.6 against 44.5 ms
-        # per 4096-edge step: a level-1 slice is only 3 KB, its mask keeps 90 % of the halves, and the box rows leave as
-        # scattered 16-byte stores instead of full lines)  (LGU_COMPACT_BOXES overrides)
-        self.compact_boxes = int(os.environ.get("LGU_COMPACT_BOXES", 1 if compact_boxes is True else int(compact_boxes)))
+        # level 0 as compact boxes (default) or as volume rows.  Level 1 as compact boxes too was measured slower (46.6
+        # against 44.5 ms per 4096-edge step: a level-1 slice is only 3 KB, its mask keeps 90 % of the halves, and the box
+        # rows leave as scattered 16-byte stores instead of full lines)
+        self.compact_boxes = bool(compact_boxes)
         self._cache = {}
         self._vol_bytes = 0
         if volume_cache_gb is None and self.cache and fmaps.is_cuda:
@@ -807,7 +806,7 @@ class AltCorrBlock:
         for s, s_end in bounds:
             e = slice(s, s_end)
             vols = ent["vols"].get(s) if ent is not None else None
-            boxes0 = boxes1 = None
+            boxes0 = None
             if vols is None:
                 # Level 0 is 3/4 of the volume bytes, and the lookup below reads it only inside a 20 x 16 box per source
                 # pixel (offsets are 4 * tanh, corr.py:121-128): build only the row bands those boxes touch.  Not when the
@@ -816,12 +815,9 @@ class AltCorrBlock:
                 hm = ops.volume_half_mask(c[e], 0) if sparse else None
                 # ... and with fp16-valued maps (the backend's buffer) and W = 64 level 0 is not written as rows at all:
                 # every source pixel keeps just the 16 x 20 box the lookup stages (1.3 KB instead of 7.6 KB of rows)
-                boxes0 = boxes1 = None
                 if sparse and self.compact_boxes and W == 64 and H % 4 == 0 and planes[0][1] is None:
                     boxes0 = ops.build_boxes(planes[0][0], planes[0][0], ii32[e], jj32[e], c[e], half_mask=hm)
-                    if (H * W // 4) % 256 == 0 and self.compact_boxes > 1:
-                        boxes1 = ops.build_boxes(planes[0][0], planes[1][0], ii32[e], jj32[e], c[e], level=1)
-                vols = [None if ((l == 0 and boxes0 is not None) or (l == 1 and boxes1 is not None)) else
+                vols = [None if (l == 0 and boxes0 is not None) else
                         ops.build_volume(planes[0][0], planes[0][1], planes[l][0], planes[l][1], ii32[e], jj32[e],
                                          half_mask=hm if l == 0 else None).view(-1, H, W, H >> l, W >> l)
                         for l in range(self.num_levels)]
@@ -835,15 +831,15 @@ class AltCorrBlock:
                 if out is not None else {}
             if self.strict_ref:
                 o, m = lookup(vols, c[e], slab0[0], slab0[1], self.radius, shared_offsets=True,
-                              apply_mask=False, return_mask=True, boxes0=boxes0, boxes1=boxes1, **dst)
+                              apply_mask=False, return_mask=True, boxes0=boxes0, **dst)
             else:
                 o1 = off1[e].clone()                                      # updated in place: offset[1] * mask
                 o, m = lookup(vols, c[e], off0[e].contiguous(), o1, self.radius, shared_offsets=False,
-                              apply_mask=True, return_mask=True, boxes0=boxes0, boxes1=boxes1, **dst)
+                              apply_mask=True, return_mask=True, boxes0=boxes0, **dst)
                 new_off1.append(o1)
             outs.append(o)
             masks.append(m)
-            del vols, boxes0, boxes1
+            del vols, boxes0
             if pass_hook is not None:                             # rows e.start .. e.stop of this call are enqueued
                 pass_hook(e.start, e.stop)
         # the attribute the reference leaves behind: offset[1] * mask (corr.py:206)

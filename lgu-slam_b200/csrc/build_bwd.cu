@@ -16,18 +16,17 @@
 // representable inputs.  Hence chunked accumulation: the issuer alternates between two TMEM accumulators every kChunk
 // k-blocks (K = 128, 48 MMAs) and four drain warps add each finished chunk into fp32 REGISTER sums with
 // round-to-nearest adds (thread == output row, 128 sums per thread).  The small operand (feature planes, pre-scaled
-// by 1/16) is split once by lgu_tf32_split; the big one (G) is split on the fly in shared memory by the converter warps,
-// which for the second product also TRANSPOSE the tile (G is q-contiguous, the contraction runs over p) into the
-// K-major 128B-swizzled layout the validated descriptors of build_pyramid.cu describe.
+// by 1/16) is split once by lgu_tf32_split; the big one (G) is split on the fly by the converter warps, which read it
+// from shared memory -- for the second product TRANSPOSED (G is q-contiguous, the contraction runs over p) -- and write
+// the hi / lo rows to tensor memory.
 //
 // One CTA per output tile (128 rows x 128 channels), 320 threads:
-//   warp 0    : TMA producer (A k-block 128 x 32 fp32 or raw 32 x 128, B_hi / B_lo k-blocks), ring of kStages (4 in the
-//               default .ts form, where A_hi / A_lo live in tensor memory: 64 columns per stage next to the accumulators)
-//   warp 1    : tcgen05.mma issuer (M128 N128 K8, 12 MMAs per k-block) + TMEM allocation (2 x 128 columns)
-//   warps 2-5 : converters (thread == tile row: mask / subtract / (transpose), fence.proxy.async)
+//   warp 0    : TMA producer (A k-block 128 x 32 fp32 or raw 32 x 128, B_hi / B_lo k-blocks), ring of 4 stages
+//   warp 1    : tcgen05.mma issuer (M128 N128 K8, 12 MMAs per k-block, .ts form: A from tensor memory) + TMEM allocation
+//               (2 x 128 accumulator columns, then 64 columns of A_hi / A_lo per stage)
+//   warps 2-5 : converters (thread == tile row == TMEM lane: mask / subtract / (transpose), tcgen05.st)
 //   warps 6-9 : drain + epilogue (tcgen05.ld 32x32b.x32 of every finished chunk -> register sums -> 128-byte
 //               coalesced stores along the pixel axis of the [E, C, P] output)
-#include <cstdlib>
 #include "tc_common.cuh"
 
 namespace lgu {
@@ -39,18 +38,15 @@ constexpr int kTile = 128;                 // M and N
 constexpr int kKB = 32;                    // k-block: 32 fp32 = one 128-byte swizzle atom row
 constexpr int kTileBytes = kTile * 128;    // 16 KB operand k-block
 constexpr int kMaxSeg = 4;
-// TS = false: A_hi / A_lo k-blocks live in shared memory (SS form of tcgen05.mma).
-// TS = true : the converters write A_hi / A_lo into TENSOR MEMORY (tcgen05.st, thread == lane == tile row) and the MMAs
-//             take A from there (.ts form): a stage is raw A | B_hi | B_lo = 48 KB (4 stages), and per k-block 80 KB
-//             less crosses the SM's shared memory (the SS form is shared-memory-bandwidth bound).
-template <bool TR, bool TS>
-struct Cfg {
-  static constexpr int kStages = TS ? 4 : (TR ? 2 : 3);
-  static constexpr int kStageBytes = (TS ? 3 : (TR ? 5 : 4)) * kTileBytes;   // [raw] | A_hi | A_lo | B_hi | B_lo
-  static constexpr int kBarOffset = kStages * kStageBytes;
-  static constexpr int kSmemBytes = kBarOffset + 256 + 1024;      // + barriers + alignment slack
-  static constexpr int kTmemCols = TS ? 512 : 256;                // accumulators 0..255, A ring 256 + 64 * stage
-};
+// The converters write A_hi / A_lo into TENSOR MEMORY (tcgen05.st, thread == lane == tile row) and the MMAs take A from
+// there (.ts form): a stage is raw A | B_hi | B_lo = 48 KB, and per k-block 80 KB less crosses the SM's shared memory
+// than with A_hi / A_lo in shared memory (that SS form is shared-memory-bandwidth bound: 1.63 + 2.4 ms against
+// 1.25 + 1.3 ms for the two products).
+constexpr int kStages = 4;
+constexpr int kStageBytes = 3 * kTileBytes;                     // raw A | B_hi | B_lo
+constexpr int kBarOffset = kStages * kStageBytes;
+constexpr int kSmemBytes = kBarOffset + 256 + 1024;             // + barriers + alignment slack
+constexpr int kTmemCols = 512;                                  // accumulators 0..255, A ring 256 + 64 * stage
 }  // namespace bb
 
 struct BbMaps {
@@ -69,16 +65,6 @@ struct BbParams {
 __host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
-__device__ __forceinline__ void tc_mma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 __device__ __forceinline__ void tc_mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc,
                                                uint32_t accumulate) {
   asm volatile(
@@ -93,36 +79,33 @@ constexpr uint32_t kTf32Mask = 0xFFFFE000u;   // sign, exponent, 10 mantissa bit
 
 // TR = false: A k-block = rows [row0, row0+128) x columns [kb*32, +32) of the segment's tensor (K contiguous).
 // TR = true : A k-block = TRANSPOSE of rows [edge_row0 + kb*32, +32) x columns [mt*128, +128) (K = rows).
-template <bool TR, bool TS>
+template <bool TR>
 __global__ void __launch_bounds__(bb::kThreads, 1)
 build_bwd_kernel(const __grid_constant__ BbMaps maps, const BbParams prm) {
   using namespace bb;
-  using C_ = Cfg<TR, TS>;
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment by POINTER arithmetic on the shared array: an integer round trip makes every derived pointer
   // generic, and all staging accesses compile to generic LD.E / ST.E instead of LDS / STS (ncu: the top stall site)
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C_::kBarOffset);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kBarOffset);
   uint64_t* full = bars;                         // [kStages]  TMA bytes landed
-  uint64_t* conv = bars + C_::kStages;           // [kStages]  converted tiles visible to the tensor core
-  uint64_t* empty = bars + 2 * C_::kStages;      // [kStages]  MMAs have read the stage
-  uint64_t* chunk_full = bars + 3 * C_::kStages;   // [2]  accumulator chunk complete (tcgen05.commit)
-  uint64_t* chunk_empty = chunk_full + 2;         // [2]  drained by the four drain warps
+  uint64_t* conv = bars + kStages;               // [kStages]  converted tiles visible to the tensor core
+  uint64_t* empty = bars + 2 * kStages;          // [kStages]  MMAs have read the stage
+  uint64_t* chunk_full = bars + 3 * kStages;     // [2]  accumulator chunk complete (tcgen05.commit)
+  uint64_t* chunk_empty = chunk_full + 2;        // [2]  drained by the four drain warps
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(chunk_empty + 2);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int e = blockIdx.x / prm.tiles_m, mt = blockIdx.x - e * prm.tiles_m;
-  constexpr int kRawOff = 0;
-  constexpr int kAhiOff = (TR && !TS) ? kTileBytes : 0;            // TS: the raw tile is the only A copy in shared memory
-  constexpr int kAloOff = kAhiOff + kTileBytes;
-  constexpr int kBhiOff = TS ? kTileBytes : kAloOff + kTileBytes;
+  constexpr int kAOff = 0;                                         // the raw tile is the only A copy in shared memory
+  constexpr int kBhiOff = kTileBytes;
   constexpr int kBloOff = kBhiOff + kTileBytes;
 
   if (warp == 0 && lane == 0) {
 #pragma unroll
     for (int l = 0; l < kMaxSeg; ++l)
       if (l < prm.nseg) { prefetch_tmap(&maps.a[l]); prefetch_tmap(&maps.bh[l]); prefetch_tmap(&maps.bl[l]); }
-    for (int s = 0; s < C_::kStages; ++s) {
+    for (int s = 0; s < kStages; ++s) {
       mbar_init(full + s, 1);
       mbar_init(conv + s, 4);                    // one arrival per converter warp
       mbar_init(empty + s, 1);
@@ -133,7 +116,7 @@ build_bwd_kernel(const __grid_constant__ BbMaps maps, const BbParams prm) {
     }
     mbar_fence_init();
   }
-  if (warp == 1) tmem_alloc(tmem_ptr, C_::kTmemCols);
+  if (warp == 1) tmem_alloc(tmem_ptr, kTmemCols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -149,13 +132,13 @@ build_bwd_kernel(const __grid_constant__ BbMaps maps, const BbParams prm) {
         const int a_edge_row = e * prm.a_rows_per_edge;
         const int b_row = e * prm.C;
         for (int kb = 0; kb < prm.kblocks[l]; ++kb, ++it) {
-          const int s = it % C_::kStages;
-          const uint32_t use = it / C_::kStages;
+          const int s = it % kStages;
+          const uint32_t use = it / kStages;
           mbar_wait(empty + s, (use & 1) ^ 1);
-          uint8_t* st = smem + s * C_::kStageBytes;
+          uint8_t* st = smem + s * kStageBytes;
           mbar_expect_tx(full + s, 3 * kTileBytes);
-          if (TR) tma_load_2d(st + kRawOff, &maps.a[l], full + s, mt * kTile, a_edge_row + kb * kKB);
-          else tma_load_2d(st + kAhiOff, &maps.a[l], full + s, kb * kKB, a_edge_row + mt * kTile);
+          if (TR) tma_load_2d(st + kAOff, &maps.a[l], full + s, mt * kTile, a_edge_row + kb * kKB);
+          else tma_load_2d(st + kAOff, &maps.a[l], full + s, kb * kKB, a_edge_row + mt * kTile);
           tma_load_2d(st + kBhiOff, &maps.bh[l], full + s, kb * kKB, b_row);
           tma_load_2d(st + kBloOff, &maps.bl[l], full + s, kb * kKB, b_row);
         }
@@ -171,8 +154,8 @@ build_bwd_kernel(const __grid_constant__ BbMaps maps, const BbParams prm) {
       for (int l = 0; l < kMaxSeg; ++l)
         if (l < prm.nseg) total += prm.kblocks[l];
       for (int i = 0; i < total; ++i, ++it) {
-        const int s = it % C_::kStages;
-        const uint32_t use = it / C_::kStages;
+        const int s = it % kStages;
+        const uint32_t use = it / kStages;
         const uint32_t chunk = it / kChunk, buf = chunk & 1;
         if (it % kChunk == 0) {                                   // new chunk: its accumulator must have been drained
           mbar_wait(chunk_empty + buf, ((chunk >> 1) & 1) ^ 1);
@@ -181,25 +164,17 @@ build_bwd_kernel(const __grid_constant__ BbMaps maps, const BbParams prm) {
         }
         mbar_wait(conv + s, use & 1);
         tc_fence_after();
-        const uint32_t st = smem_u32(smem + s * C_::kStageBytes);
+        const uint32_t st = smem_u32(smem + s * kStageBytes);
         const uint32_t d_tmem = tmem_base + buf * kTile;
 #pragma unroll
         for (int kk = 0; kk < kKB / 8; ++kk) {
           const uint32_t off = kk * 32;                           // K = 8 tf32 = 32 bytes inside the swizzle atom
-          const uint64_t ahi = make_kmajor_sw128_desc(st + kAhiOff + off), alo = make_kmajor_sw128_desc(st + kAloOff + off);
           const uint64_t bhi = make_kmajor_sw128_desc(st + kBhiOff + off), blo = make_kmajor_sw128_desc(st + kBloOff + off);
-          if (TS) {
-            const uint32_t a_t = tmem_base + 256 + s * 64 + kk * 8;   // A_hi columns; A_lo 32 columns further
-            tc_mma_tf32_ts(d_tmem, a_t, bhi, idesc, acc);
-            acc = 1;
-            tc_mma_tf32_ts(d_tmem, a_t, blo, idesc, 1);
-            tc_mma_tf32_ts(d_tmem, a_t + 32, bhi, idesc, 1);
-          } else {
-            tc_mma_tf32(d_tmem, ahi, bhi, idesc, acc);
-            acc = 1;
-            tc_mma_tf32(d_tmem, ahi, blo, idesc, 1);
-            tc_mma_tf32(d_tmem, alo, bhi, idesc, 1);
-          }
+          const uint32_t a_t = tmem_base + 256 + s * 64 + kk * 8;     // A_hi columns; A_lo 32 columns further
+          tc_mma_tf32_ts(d_tmem, a_t, bhi, idesc, acc);
+          acc = 1;
+          tc_mma_tf32_ts(d_tmem, a_t, blo, idesc, 1);
+          tc_mma_tf32_ts(d_tmem, a_t + 32, bhi, idesc, 1);
         }
         tc_commit(empty + s);
         if ((it % kChunk) == kChunk - 1 || i == total - 1) tc_commit(chunk_full + buf);
@@ -207,79 +182,43 @@ build_bwd_kernel(const __grid_constant__ BbMaps maps, const BbParams prm) {
     }
   } else if (warp < 6) {
     // =============================== converters (warps 2..5) ===============================
-    // tile row owned by this thread; with TS it is also the TMEM lane, which a warp may only touch in its own quadrant
-    const int row = TS ? ((warp & 3) * 32 + lane) : (threadIdx.x - 64);
+    // tile row owned by this thread; it is also the TMEM lane, which a warp may only touch in its own quadrant
+    const int row = (warp & 3) * 32 + lane;
     const int rsw = row & 7;                                      // 128B swizzle phase of the row
     int total = 0;
 #pragma unroll
     for (int l = 0; l < kMaxSeg; ++l)
       if (l < prm.nseg) total += prm.kblocks[l];
     for (int it = 0; it < total; ++it) {
-      const int s = it % C_::kStages;
-      const uint32_t use = it / C_::kStages;
+      const int s = it % kStages;
+      const uint32_t use = it / kStages;
       mbar_wait(full + s, use & 1);
-      uint8_t* st = smem + s * C_::kStageBytes;
-      float4* hi_row = reinterpret_cast<float4*>(st + kAhiOff + row * 128);
-      float4* lo_row = reinterpret_cast<float4*>(st + kAloOff + row * 128);
-      if (TS) {
-        // this row's 32 k values in K order (non-TR: undo the TMA's chunk swizzle; TR: one raw column), split, and
-        // written to the stage's tensor-memory columns
-        uint32_t h[32], l[32];
+      uint8_t* st = smem + s * kStageBytes;
+      // this row's 32 k values in K order (non-TR: undo the TMA's chunk swizzle; TR: one raw column), split, and written
+      // to the stage's tensor-memory columns
+      uint32_t h[32], l[32];
 #pragma unroll
-        for (int c = 0; c < 8; ++c) {
-          float v[4];
-          if (TR) {
-            const float* raw = reinterpret_cast<const float*>(st + kRawOff) + row;
+      for (int c = 0; c < 8; ++c) {
+        float v[4];
+        if (TR) {
+          const float* raw = reinterpret_cast<const float*>(st + kAOff) + row;
 #pragma unroll
-            for (int q = 0; q < 4; ++q) v[q] = raw[(4 * c + q) * kTile];
-          } else {
-            const float4 t = hi_row[c ^ rsw];
-            v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
-          }
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            h[4 * c + q] = __float_as_uint(v[q]) & kTf32Mask;
-            l[4 * c + q] = __float_as_uint(__fsub_rn(v[q], __uint_as_float(h[4 * c + q])));
-          }
+          for (int q = 0; q < 4; ++q) v[q] = raw[(4 * c + q) * kTile];
+        } else {
+          const float4 t = reinterpret_cast<const float4*>(st + kAOff + row * 128)[c ^ rsw];
+          v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
         }
-        const uint32_t ta = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + 256 + s * 64;
-        tmem_st32(ta, h);
-        tmem_st32(ta + 32, l);
-        tmem_wait_st();
-        tc_fence_before();
-      } else if (!TR) {
-        // in place and elementwise, so the TMA's chunk swizzle does not matter for correctness -- but the eight rows
-        // of a swizzle group must touch eight DIFFERENT chunks per access (visiting chunk c of every row at once is a
-        // 32-way bank conflict: measured 2.4 us per k-block instead of 0.8)
 #pragma unroll
-        for (int cc = 0; cc < 8; ++cc) {
-          const int c = cc ^ rsw;
-          const float4 v = hi_row[c];
-          float4 h, l;
-          h.x = __uint_as_float(__float_as_uint(v.x) & kTf32Mask); l.x = __fsub_rn(v.x, h.x);
-          h.y = __uint_as_float(__float_as_uint(v.y) & kTf32Mask); l.y = __fsub_rn(v.y, h.y);
-          h.z = __uint_as_float(__float_as_uint(v.z) & kTf32Mask); l.z = __fsub_rn(v.z, h.z);
-          h.w = __uint_as_float(__float_as_uint(v.w) & kTf32Mask); l.w = __fsub_rn(v.w, h.w);
-          hi_row[c] = h;
-          lo_row[c] = l;
-        }
-      } else {
-        // raw tile [32 k][128 m] (row-major, unswizzled): this thread owns column m == row; consecutive threads read
-        // consecutive words (conflict-free) and write their own 128-byte K-major row with the TMA's chunk swizzle
-        const float* raw = reinterpret_cast<const float*>(st + kRawOff) + row;
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {
-          float v[4], h[4];
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            v[q] = raw[(4 * c + q) * kTile];
-            h[q] = __uint_as_float(__float_as_uint(v[q]) & kTf32Mask);
-          }
-          hi_row[c ^ rsw] = make_float4(h[0], h[1], h[2], h[3]);
-          lo_row[c ^ rsw] = make_float4(__fsub_rn(v[0], h[0]), __fsub_rn(v[1], h[1]), __fsub_rn(v[2], h[2]),
-                                        __fsub_rn(v[3], h[3]));
+        for (int q = 0; q < 4; ++q) {
+          h[4 * c + q] = __float_as_uint(v[q]) & kTf32Mask;
+          l[4 * c + q] = __float_as_uint(__fsub_rn(v[q], __uint_as_float(h[4 * c + q])));
         }
       }
+      const uint32_t ta = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + 256 + s * 64;
+      tmem_st32(ta, h);
+      tmem_st32(ta + 32, l);
+      tmem_wait_st();
+      tc_fence_before();
       fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(conv + s);
@@ -321,7 +260,7 @@ build_bwd_kernel(const __grid_constant__ BbMaps maps, const BbParams prm) {
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, C_::kTmemCols);
+  if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
 }
 
 // x * scale -> hi (low 13 mantissa bits cleared) and lo = x * scale - hi (exact).
@@ -336,20 +275,12 @@ __global__ void __launch_bounds__(256) tf32_split_kernel(const float* __restrict
   }
 }
 
-template <bool TR, bool TS>
-static int launch_bb_impl(const BbMaps& maps, const BbParams& prm, int E, cudaStream_t st) {
-  using C_ = bb::Cfg<TR, TS>;
-  auto kern = build_bwd_kernel<TR, TS>;
-  if (int rc = optin_smem(reinterpret_cast<const void*>(kern), C_::kSmemBytes, "lgu_build_backward_fmaps")) return rc;
-  kern<<<(unsigned)(E * prm.tiles_m), bb::kThreads, C_::kSmemBytes, st>>>(maps, prm);
-  return check_launch("lgu_build_backward_fmaps");
-}
-
 template <bool TR>
 static int launch_bb(const BbMaps& maps, const BbParams& prm, int E, cudaStream_t st) {
-  const char* v = getenv("LGU_BBWD_SS");                           // 1: keep the A operand in shared memory (SS form)
-  if (v != nullptr && v[0] != '\0' && v[0] != '0') return launch_bb_impl<TR, false>(maps, prm, E, st);
-  return launch_bb_impl<TR, true>(maps, prm, E, st);
+  auto kern = build_bwd_kernel<TR>;
+  if (int rc = optin_smem(reinterpret_cast<const void*>(kern), bb::kSmemBytes, "lgu_build_backward_fmaps")) return rc;
+  kern<<<(unsigned)(E * prm.tiles_m), bb::kThreads, bb::kSmemBytes, st>>>(maps, prm);
+  return check_launch("lgu_build_backward_fmaps");
 }
 
 }  // namespace lgu

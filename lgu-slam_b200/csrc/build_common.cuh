@@ -1,7 +1,6 @@
 // build_common.cuh -- parameter block and Gaussian residual shared by build_pyramid.cu (8 epilogue warps; every
 // precision / flat volumes) and build_pyramid16.cu (16 epilogue warps; the fp16-input pyramid build).
 #pragma once
-#include <cstdlib>
 #include "tc_common.cuh"
 
 namespace lgu {
@@ -18,14 +17,12 @@ struct BpParams {
   const float* means;   // [E,P,2] or null
   const float* covs;    // [E,P,2]
   const float* den;     // [E,P]
-  float* lvl0;          // [E,P,Q] (LSU store experiments of the 16-warp kernel; the production path stores through the TMA map)
-  float* lvl1;          // [E,P,Q/4] or null (direct-store path)
+  float* lvl0;          // [E,P,Q] (stored to directly by the 16-warp kernel; the 8-warp kernel stores through its TMA map)
+  float* lvl1;          // [E,P,Q/4] or null (as lvl0)
   float* lvl2;          // [E,P,Q/16] or null
   float* lvl3;          // [E,P,Q/64] or null
   int E, P, H, gauss_radius, round_half, num_units, has_l1;
   const int32_t* out_slots;   // [E] or null: edge e is written to pyramid slot out_slots[e] (edge-slot pool)
-  unsigned long long* trace;   // LGU_BP_TRACE builds: 4 cycle counters (null otherwise)
-  int wide;     // 1: level-0 rows leave as pair-shared 16 KB boxes (512 contiguous bytes per source pixel; PREC 1, Q % 64 == 0)
   int Q;        // target pixels per map (== P for the pyramid build; any multiple of 4 in flat volume mode)
   int halves;   // 256-column accumulator halves per unit: ceil(Q / 256)
   const uint32_t* half_mask;   // [num_units] or null: bit h set = accumulator half h (256 target columns) of the unit is built
@@ -33,8 +30,6 @@ struct BpParams {
   float* boxes;               // FLAT 16-warp kernel: [E,P,16,20] or null -- write each source pixel's lookup box (rows
   const float* box_coords;    //   box_origin_y(floor(cy),7,H) .. +15, cols box_origin_x(floor(cx),7,64) .. +19 around box_coords [E,P,2],
                               //   zeros outside the target grid) INSTEAD of the volume rows (lgu_build_boxes)
-  int l0_lsu;   // 16-warp kernel: bit 0 / 1 = upper / lower row of a pair leaves through the LSU instead of the TMA store engine
-  int dbg;      // experiment switches of build_pyramid16_kernel (LGU_BUILD_DBG; 0 in production)
 };
 
 // Gaussian residual of one element (gaussianAttn.cu:58-64 + gaussianMask_cuda.py:85-86), fp32, no contraction.
@@ -48,16 +43,9 @@ __device__ __forceinline__ float gauss_residual(float v, int x1, int y1, float m
   return __fadd_rn(__fdiv_rn(masked, den), v);
 }
 
-
-static inline bool env_flag(const char* name) {   // experiment switches of the build kernels
-  const char* v = getenv(name);
-  return v != nullptr && v[0] != '\0' && v[0] != '0';
-}
-
 // (Forming the row-invariant ddy / cov_y once per window row instead of per tap was measured: 542 -> 553 us, reverted.)
 
 // The 16-epilogue-warp kernel (build_pyramid16.cu).  Returns LGU_OK / an error code.
-int launch_build16(const CUtensorMap& mh, const CUtensorMap& mb, const CUtensorMap& m0, const CUtensorMap& m1, const BpParams& prm,
-                   bool flat, cudaStream_t st);
+int launch_build16(const CUtensorMap& mh, const CUtensorMap& mb, const BpParams& prm, bool flat, cudaStream_t st);
 
 }  // namespace lgu

@@ -28,42 +28,8 @@
 // Precision: PREC 1 = one fp16 product (exact for fp16-valued feature maps: the inference path);
 //            PREC 2 = hi/lo fp16 split of both operands, 3 MMAs (hi*hi + hi*lo + lo*hi): ~2^-21 relative
 //            per product, for fp32-valued feature maps (the training path).
-#include <cstdlib>
 #include "build_common.cuh"
 #include "fused_common.cuh"
-
-// LGU_BP_TRACE (diagnostic builds only): per epilogue warp, cycles spent waiting for (0) the accumulator half, (1) a
-// free staging buffer (the TMA store engine), (2) the quadrant's pair barriers, and (3) in total.  lane 0 of every
-// epilogue warp adds its four counters to prm.trace[4] with atomics at kernel end (tools/diag/bp_trace.py).
-#ifdef LGU_BP_TRACE
-#define BP_T0() const long long _t0 = clock64()
-#define BP_ADD(slot) tr[slot] += clock64() - _t0
-#else
-#define BP_T0()
-#define BP_ADD(slot)
-#endif
-// LGU_BP_TRACE == 2: the slots are re-used for (0) the tcgen05.ld pairs, (1) staging writes + Gaussian patch,
-// (2) fence.proxy.async + __syncwarp + store issue
-#if defined(LGU_BP_TRACE) && LGU_BP_TRACE == 2
-#define BP2_T0() const long long _u0 = clock64()
-#define BP2_ADD(slot) tr[slot] += clock64() - _u0
-#undef BP_ADD
-#define BP_ADD(slot)
-#else
-#define BP2_T0()
-#define BP2_ADD(slot)
-#endif
-// LGU_BP_TRACE == 3: (0) 2x2 pooling of the row pair, (1) the whole level-1 path (pair barriers, staging, store),
-// (2) levels 2 / 3 (pooling + direct stores)
-#if defined(LGU_BP_TRACE) && LGU_BP_TRACE == 3
-#define BP3_T0() const long long _w0 = clock64()
-#define BP3_ADD(slot) tr[slot] += clock64() - _w0
-#undef BP_ADD
-#define BP_ADD(slot)
-#else
-#define BP3_T0()
-#define BP3_ADD(slot)
-#endif
 
 namespace lgu {
 
@@ -90,12 +56,12 @@ struct BpCfg {
   static constexpr int kSmemBytes = kBarOffset + 256 + 1024;  // + barriers + 1 KB alignment slack
 };
 
-template <int PREC, bool WIDE>
+template <int PREC>
 __global__ void __launch_bounds__(kBpThreads, 1)
 build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo,
                      const __grid_constant__ CUtensorMap map_bhi, const __grid_constant__ CUtensorMap map_blo,
                      const __grid_constant__ CUtensorMap map_l0, const __grid_constant__ CUtensorMap map_l1,
-                     const __grid_constant__ CUtensorMap map_l0w, const BpParams prm) {
+                     const BpParams prm) {
   using Cfg = BpCfg<PREC>;
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment by POINTER arithmetic on the shared array: an integer round trip makes every derived pointer
@@ -125,7 +91,6 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
     prefetch_tmap(&map_bhi);
     if (PREC == 2) { prefetch_tmap(&map_lo); prefetch_tmap(&map_blo); }
     prefetch_tmap(&map_l0);
-    if (WIDE) prefetch_tmap(&map_l0w);
     if (prm.has_l1) prefetch_tmap(&map_l1);
     mbar_init(a_full, 1);
     mbar_init(a_empty, 1);
@@ -225,10 +190,6 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
     }
   } else {
     // =============================== epilogue (warps 2..9) ===============================
-#ifdef LGU_BP_TRACE
-    long long tr[4] = {0, 0, 0, 0};
-    const long long tr_begin = clock64();
-#endif
     const int quad = warp & 3;                          // TMEM lane quadrant this warp may read (warp id % 4)
     const int xs = (warp - 2) >> 2;                     // which 32-column half of the 64 target columns
     const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
@@ -245,18 +206,13 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
     // stage one 32-float row segment per lane and hand the 32x32 tile to the TMA store engine
     auto store_tile = [&](float (&v)[32], int col, int row0, bool patch, int yy, float mx, float my, float c1, float c2,
                           float den, unsigned bx) {
-      {
-        BP_T0();
-        if (lane == 0) {
-          // the tile staged in this buffer two level-0 stores ago must have been read; the issuer warp has one
-          // level-1 group between them, so it may leave one more group pending
-          if (l1_issuer) tma_wait_read<Cfg::kStoreBufs>();
-          else tma_wait_read<Cfg::kStoreBufs - 1>();
-        }
-        __syncwarp();
-        BP_ADD(1);
+      if (lane == 0) {
+        // the tile staged in this buffer two level-0 stores ago must have been read; the issuer warp has one
+        // level-1 group between them, so it may leave one more group pending
+        if (l1_issuer) tma_wait_read<Cfg::kStoreBufs>();
+        else tma_wait_read<Cfg::kStoreBufs - 1>();
       }
-      BP2_T0();
+      __syncwarp();
       float4* rowp = reinterpret_cast<float4*>(my_store + sbuf * 4096 + lane * 128);
 #pragma unroll
       for (int c = 0; c < 8; ++c) rowp[c ^ rsw] = make_float4(v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
@@ -281,49 +237,13 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
           }
         }
       }
-      BP2_ADD(1);
-      {
-        BP2_T0();
-        fence_proxy_async();
-        __syncwarp();
-        if (lane == 0) {
-          tma_store_2d(&map_l0, my_store + sbuf * 4096, col, row0);
-          tma_commit();
-        }
-        BP2_ADD(2);
+      fence_proxy_async();
+      __syncwarp();
+      if (lane == 0) {
+        tma_store_2d(&map_l0, my_store + sbuf * 4096, col, row0);
+        tma_commit();
       }
       sbuf = (sbuf + 1 == Cfg::kStoreBufs) ? 0 : sbuf + 1;
-    };
-    // Wide path (PREC 1, Q % 64 == 0): the two warps of a lane quadrant fill ONE 16 KB tile per target-row pair --
-    // chunks [ya | x0..31], [ya | x32..63], [yb | x0..31], [yb | x32..63], i.e. 512 CONTIGUOUS bytes per source pixel
-    // -- and one elected lane stores it with a single 3-D box.  Measured on the store stream alone
-    // (tools/micro/tma_store.cu): 5.7-5.9 TB/s against 5.2 TB/s for 32-row x 128-byte boxes, single-buffered.
-    uint8_t* pair_l0 = sStore + quad * 4 * 4096;
-    auto stage_row = [&](float (&v)[32], int chunk, bool patch, int yy, float mx, float my, float c1, float c2,
-                         float den, unsigned bx) {
-      float4* rowp = reinterpret_cast<float4*>(pair_l0 + chunk * 4096 + lane * 128);
-#pragma unroll
-      for (int c = 0; c < 8; ++c) rowp[c ^ rsw] = make_float4(v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
-      if (patch) {
-        float* rowf = reinterpret_cast<float*>(rowp);
-        bool touched = false;
-        for (unsigned k = 0; k < rdg; ++k) {
-          const int x = (int)(bx + k);
-          const unsigned idx = (unsigned)(x - x0);
-          if (idx < 32u) {
-            const unsigned pos = (((idx >> 2) ^ (unsigned)rsw) << 2) | (idx & 3u);
-            rowf[pos] = gauss_residual(rowf[pos], x, yy, mx, my, c1, c2, den);
-            touched = true;
-          }
-        }
-        if (touched) {
-#pragma unroll
-          for (int c = 0; c < 8; ++c) {
-            const float4 t = rowp[c ^ rsw];
-            v[4 * c] = t.x; v[4 * c + 1] = t.y; v[4 * c + 2] = t.z; v[4 * c + 3] = t.w;
-          }
-        }
-      }
     };
     // level 1: 16 floats (64 B) per lane, 64B-swizzled 32-row tile (2 KB of a staging buffer)
     auto store_l1 = [&](const float (&v)[16], int col, int row0) {
@@ -368,23 +288,15 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
         if (!((hmask >> h) & 1u)) continue;               // (flat volumes only: the pooled levels need every half)
         const uint32_t buf = half_it & 1, buf_use = half_it >> 1;
         ++half_it;
-        {
-          BP_T0();
-          mbar_wait(t_full + buf, buf_use & 1);
-          BP_ADD(0);
-        }
+        mbar_wait(t_full + buf, buf_use & 1);
         tc_fence_after();
         const uint32_t tcol = tmem_base + lane_base + buf * 256 + xs * 32;
         float l1[2][16];
 #pragma unroll
         for (int rp = 0; rp < 2; ++rp) {
           float a[32], b[32];
-          {
-            BP2_T0();
-            tmem_ld32(tcol + (2 * rp) * 64, a);
-            tmem_ld32(tcol + (2 * rp + 1) * 64, b);
-            BP2_ADD(0);
-          }
+          tmem_ld32(tcol + (2 * rp) * 64, a);
+          tmem_ld32(tcol + (2 * rp + 1) * 64, b);
           if (rp == 1) {
             // last TMEM read of this half: hand the accumulator back to the MMA issuer
             tc_fence_before();
@@ -401,42 +313,13 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
           const int ya = 4 * h + 2 * rp, yb = ya + 1;
           const bool pa = gr > 0 && ((unsigned)ya - by) < rdg;
           const bool pb = gr > 0 && ((unsigned)yb - by) < rdg;
-          constexpr bool wide = Cfg::kPairL1 && WIDE;
-          if (wide) {
-            // A: the engine has read the pair's tiles of the previous row pair (the issuer waited), both warps may restage
-            if (xs == 0 && lane == 0) tma_wait_read<0>();
-            asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");
-            stage_row(a, xs, pa, ya, mx, my, c1, c2, den, bx);
-            stage_row(b, 2 + xs, pb, yb, mx, my, c1, c2, den, bx);
-          } else {
-            if (ya * 64 + x0 < Q) store_tile(a, ya * 64 + x0, row0, pa, ya, mx, my, c1, c2, den, bx);   // flat mode: Q may
-            if (yb * 64 + x0 < Q) store_tile(b, yb * 64 + x0, row0, pb, yb, mx, my, c1, c2, den, bx);   // end mid-half
-          }
+          if (ya * 64 + x0 < Q) store_tile(a, ya * 64 + x0, row0, pa, ya, mx, my, c1, c2, den, bx);   // flat mode: Q may
+          if (yb * 64 + x0 < Q) store_tile(b, yb * 64 + x0, row0, pb, yb, mx, my, c1, c2, den, bx);   // end mid-half
           // 2x2 average, ATen order: ((a0 + a1) + b0) + b1, then / 4   (corr.py:86)
-          {
-            BP3_T0();
 #pragma unroll
-            for (int i = 0; i < 16; ++i)
-              l1[rp][i] = __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(a[2 * i], a[2 * i + 1]), b[2 * i]), b[2 * i + 1]), 0.25f);
-            BP3_ADD(0);
-          }
-          BP3_T0();
-          if (wide) {
-            if (prm.has_l1) {
-              float4* rowp = reinterpret_cast<float4*>(pair_l1 + l1buf * 4096 + lane * 128);
-#pragma unroll
-              for (int c = 0; c < 4; ++c)
-                rowp[(xs * 4 + c) ^ rsw] = make_float4(l1[rp][4 * c], l1[rp][4 * c + 1], l1[rp][4 * c + 2], l1[rp][4 * c + 3]);
-            }
-            fence_proxy_async();
-            asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");        // B: both warps' halves are staged
-            if (xs == 0 && lane == 0) {
-              tma_store_3d(&map_l0w, pair_l0, 0, row0, 2 * ya);                 // chunks beyond Q / 32 are clipped
-              if (prm.has_l1) tma_store_2d(&map_l1, pair_l1 + l1buf * 4096, (2 * h + rp) * 32, row0);
-              tma_commit();
-            }
-            l1buf ^= 1;
-          } else if (prm.has_l1) {
+          for (int i = 0; i < 16; ++i)
+            l1[rp][i] = __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(a[2 * i], a[2 * i + 1]), b[2 * i]), b[2 * i + 1]), 0.25f);
+          if (prm.has_l1) {
             if (kL1Direct) {   // 64-byte rows cost the TMA store engine a full row slot each: use the idle LSU instead
               float4* o1 = reinterpret_cast<float4*>(prm.lvl1 + pix * (size_t)(Q >> 2) + (2 * h + rp) * 32 + xs * 16);
 #pragma unroll
@@ -445,21 +328,13 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
             } else if (Cfg::kPairL1) {
               // named barrier of the quadrant's two warps (ids 1..4).  A: the issuer's waits before its two level-0
               // stores of this row pair guarantee that the tile stored from this buffer two rows ago has been read.
-              {
-                BP_T0();
-                asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");
-                BP_ADD(2);
-              }
+              asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");
               float4* rowp = reinterpret_cast<float4*>(pair_l1 + l1buf * 4096 + lane * 128);
 #pragma unroll
               for (int c = 0; c < 4; ++c)
                 rowp[(xs * 4 + c) ^ rsw] = make_float4(l1[rp][4 * c], l1[rp][4 * c + 1], l1[rp][4 * c + 2], l1[rp][4 * c + 3]);
               fence_proxy_async();
-              {
-                BP_T0();
-                asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");    // B: both halves are in the tile
-                BP_ADD(2);
-              }
+              asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");    // B: both halves are in the tile
               if (xs == 0 && lane == 0) {
                 tma_store_2d(&map_l1, pair_l1 + l1buf * 4096, (2 * h + rp) * 32, row0);
                 tma_commit();
@@ -469,9 +344,7 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
               store_l1(l1[rp], (2 * h + rp) * 32 + xs * 16, row0);
             }
           }
-          BP3_ADD(1);
         }
-        BP3_T0();
         if (prm.lvl2 != nullptr) {
           float l2[8];
 #pragma unroll
@@ -494,16 +367,10 @@ build_pyramid_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_co
                 make_float4(l3[0], l3[1], l3[2], l3[3]);
           }
         }
-        BP3_ADD(2);
       }
     }
     if (lane == 0) tma_wait_all();                      // all bulk stores complete before the CTA exits
     __syncwarp();
-#ifdef LGU_BP_TRACE
-    tr[3] = clock64() - tr_begin;
-    if (lane == 0 && prm.trace != nullptr)
-      for (int q = 0; q < 4; ++q) atomicAdd(prm.trace + q, (unsigned long long)tr[q]);
-#endif
   }
 
   tc_fence_before();
@@ -578,16 +445,15 @@ __global__ void __launch_bounds__(256) pack_fmaps_vec_kernel(const SRC* __restri
 
 template <int PREC>
 static int launch_build(const CUtensorMap& mh, const CUtensorMap& ml, const CUtensorMap& mbh, const CUtensorMap& mbl,
-                        const CUtensorMap& m0, const CUtensorMap& m1, const CUtensorMap& m0w, const BpParams& prm,
-                        cudaStream_t st) {
+                        const CUtensorMap& m0, const CUtensorMap& m1, const BpParams& prm, cudaStream_t st) {
   using Cfg = BpCfg<PREC>;
-  auto kern = (PREC == 1 && prm.wide) ? build_pyramid_kernel<PREC, PREC == 1> : build_pyramid_kernel<PREC, false>;
+  auto kern = build_pyramid_kernel<PREC>;
   if (int rc = optin_smem(reinterpret_cast<const void*>(kern), Cfg::kSmemBytes, "lgu_build_pyramid")) return rc;
   int dev = 0, sms = kNumSMs;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int grid = prm.num_units < sms ? prm.num_units : sms;
-  kern<<<grid, kBpThreads, Cfg::kSmemBytes, st>>>(mh, ml, mbh, mbl, m0, m1, m0w, prm);
+  kern<<<grid, kBpThreads, Cfg::kSmemBytes, st>>>(mh, ml, mbh, mbl, m0, m1, prm);
   return check_launch("lgu_build_pyramid");
 }
 
@@ -678,38 +544,23 @@ static int build_pyramid_impl(const void* fmaps_hi, const void* fmaps_lo, const 
                    precision == 1 ? 32 : 16, precision == 1 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
   if (rc) return rc;
 
-  CUtensorMap m0w = m0;
-  // measured at E = 48 (bench.py): the pair-shared 16 KB level-0 boxes do not pay in the pyramid build (593 vs 582 us:
-  // its epilogue, not the store shape, is the limit) -- opt-in only; the flat volumes below use them by default
-  const int wide = (precision == 1 && env_flag("LGU_BUILD_WIDE")) ? 1 : 0;
-  if (wide) {
-    rc = make_map_chunked(&m0w, lvl0, (uint64_t)S * P, P, 32, 4);
-    if (rc) return rc;
-  }
   BpParams prm;
-  prm.wide = wide;
-  prm.trace = nullptr;
-#if defined(LGU_BP_TRACE) || defined(LGU_B16_TRACE)
-  if (const char* tp = getenv("LGU_BP_TRACE_PTR")) prm.trace = reinterpret_cast<unsigned long long*>(strtoull(tp, nullptr, 0));
-#endif
   prm.ii = ii; prm.jj = jj; prm.means = means; prm.covs = covs; prm.den = den;
   prm.lvl0 = lvl0; prm.lvl1 = lvl1; prm.lvl2 = lvl2; prm.lvl3 = lvl3;
   prm.E = E; prm.P = P; prm.H = H; prm.gauss_radius = gauss_radius; prm.round_half = round_half;
   prm.num_units = E * (P / kTileM);
   prm.has_l1 = lvl1 != nullptr;
-  prm.dbg = getenv("LGU_BUILD_DBG") ? atoi(getenv("LGU_BUILD_DBG")) : 0;
   prm.half_mask = nullptr;
   prm.boxes = nullptr; prm.box_coords = nullptr; prm.box_W = 64; prm.box_level = 0;
-  // level-0 rows of the 16-warp kernel through the LSU (default, 537 -> 505 us at E = 48); LGU_BUILD_L0_TMA=1: TMA stores
-  prm.l0_lsu = env_flag("LGU_BUILD_L0_TMA") ? 0 : 3;
   prm.out_slots = out_slots;
   prm.Q = P;
   prm.halves = H / 4;
-  // fp16-valued maps, all four levels: the 16-epilogue-warp kernel (build_pyramid16.cu); LGU_BUILD_EPI8=1 keeps this one
-  if (precision == 1 && lvl1 != nullptr && lvl2 != nullptr && lvl3 != nullptr && !wide && !env_flag("LGU_BUILD_EPI8"))
-    return launch_build16(mh, mh, m0, m1, prm, false, (cudaStream_t)stream);
-  if (precision == 1) return launch_build<1>(mh, ml, mh, ml, m0, m1, m0w, prm, (cudaStream_t)stream);
-  return launch_build<2>(mh, ml, mh, ml, m0, m1, m0w, prm, (cudaStream_t)stream);
+  // fp16-valued maps, all four levels: the 16-epilogue-warp kernel (build_pyramid16.cu; 573-580 us with this one at E = 48,
+  // 503 us there)
+  if (precision == 1 && lvl1 != nullptr && lvl2 != nullptr && lvl3 != nullptr)
+    return launch_build16(mh, mh, prm, false, (cudaStream_t)stream);
+  if (precision == 1) return launch_build<1>(mh, ml, mh, ml, m0, m1, prm, (cudaStream_t)stream);
+  return launch_build<2>(mh, ml, mh, ml, m0, m1, prm, (cudaStream_t)stream);
 }
 
 static int build_volume_impl(const void* fmaps1_hi, const void* fmaps1_lo, const void* fmaps2_hi,
@@ -742,36 +593,22 @@ static int build_volume_impl(const void* fmaps1_hi, const void* fmaps1_lo, const
   if (rc) return rc;
   rc = make_map_2d(&m0, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, volume, (uint64_t)E * P, Q, 32, 32);
   if (rc) return rc;
-  CUtensorMap m0w = m0;
-  // flat volumes (no Gaussian patch, no pooled levels): 512 contiguous bytes per source pixel and store, -10 % on the
-  // backend's volume builds (tools/bench_backend.py: 41.7 -> 39.5 ms per step at 2048 edges)
-  const int wide = (precision == 1 && (Q % 64) == 0 && !env_flag("LGU_BUILD_NARROW")) ? 1 : 0;
-  if (wide) {
-    rc = make_map_chunked(&m0w, volume, (uint64_t)E * P, Q, 32, 4);
-    if (rc) return rc;
-  }
   BpParams prm;
-  prm.wide = wide;
-  prm.trace = nullptr;
   prm.ii = ii; prm.jj = jj; prm.means = nullptr; prm.covs = nullptr; prm.den = nullptr;
   prm.lvl0 = volume; prm.lvl1 = nullptr; prm.lvl2 = nullptr; prm.lvl3 = nullptr;
   prm.E = E; prm.P = P; prm.H = 0; prm.gauss_radius = 0; prm.round_half = 0;
   prm.num_units = E * (P / kTileM);
   prm.has_l1 = 0;
-  prm.dbg = 0;
-  prm.l0_lsu = 0;
   prm.half_mask = half_mask;
   prm.boxes = boxes; prm.box_coords = box_coords; prm.box_W = box_W; prm.box_level = box_level;
   prm.H = boxes != nullptr ? Q / box_W : 0;
   prm.out_slots = nullptr;
   prm.Q = Q;
   prm.halves = (Q + 255) / 256;
-  // fp16-valued maps (the backend's buffer): the 16-warp kernel with its barrier-free flat epilogue; LGU_VOLUME_EPI8=1 keeps
-  // the 8-warp kernel with the pair-shared 16 KB TMA boxes
-  if (precision == 1 && (boxes != nullptr || !env_flag("LGU_VOLUME_EPI8")))
-    return launch_build16(mh, mbh, m0, m0, prm, true, (cudaStream_t)stream);
-  if (precision == 1) return launch_build<1>(mh, ml, mbh, mbl, m0, m0, m0w, prm, (cudaStream_t)stream);
-  return launch_build<2>(mh, ml, mbh, mbl, m0, m0, m0w, prm, (cudaStream_t)stream);
+  // fp16-valued maps (the backend's buffer): the 16-warp kernel with its barrier-free flat epilogue (2 % faster on the backend
+  // step than this kernel with pair-shared 16 KB TMA boxes)
+  if (precision == 1) return launch_build16(mh, mbh, prm, true, (cudaStream_t)stream);
+  return launch_build<2>(mh, ml, mbh, mbl, m0, m0, prm, (cudaStream_t)stream);
 }
 
 extern "C" int lgu_build_volume(const void* fmaps1_hi, const void* fmaps1_lo, const void* fmaps2_hi,

@@ -2,7 +2,7 @@
 // maps, all four levels; the frontend / CorrBlock.__init__ case).  Same producer, same tcgen05 issuer, same outputs
 // bit for bit; what changes is who drains the accumulator.
 //
-// Why: a clock64 trace of the 8-warp kernel (-DLGU_BP_TRACE, tools/diag/bp_trace.py) shows its epilogue warps waiting
+// Why: a clock64 trace of the 8-warp kernel (DESIGN.md; a diagnostic build up to commit b094b8a) shows its epilogue warps waiting
 // 3 % of their time for a free staging buffer, 4-8 % for the accumulator and 2 % at barriers -- the other ~90 % is their
 // own, latency-bound instruction stream (two epilogue warps per scheduler, 24 % issue slots used), while the TMA store
 // engine has >= 20 % headroom.  More warps per TMEM lane quadrant is the lever.
@@ -10,26 +10,15 @@
 // Epilogue split: the four warps of a TMEM lane quadrant (warp id % 4) take (column half xs) x (row pair rp) of every
 // accumulator half (4 target rows x 64 columns):
 //   * one row at a time: tcgen05.ld 32 columns -> [fp16 rounding] -> staged in the warp's 4 KB swizzled tile (Gaussian
-//     window patched in shared memory) -> TMA store; the horizontal pair sums a[2i] + a[2i+1] of the upper row are kept
-//     (16 registers) so the 2x2 average keeps ATen's order ((a0 + a1) + b0) + b1 without holding both rows;
-//   * level 1: the two xs-warps of a row pair fill one 32-row x 128-byte tile; the quadrant's two tiles (rp = 0, 1) are
-//     stored by one elected lane after a quadrant barrier;
+//     window patched in shared memory) -> full-line LSU stores; the horizontal pair sums a[2i] + a[2i+1] of the upper row
+//     are kept (16 registers) so the 2x2 average keeps ATen's order ((a0 + a1) + b0) + b1 without holding both rows;
+//   * level 1: the two xs-warps of a row pair fill one 32-row x 128-byte tile; after a quadrant barrier every warp stores
+//     8 rows of the quadrant's two tiles (rp = 0, 1) through the LSU;
 //   * levels 2 / 3: after that barrier every warp reads the two level-1 tiles back from shared memory and produces a
 //     quarter of the level-2 row (4 columns, one 16-byte store per lane) and, every second half, 2 columns of level 3.
 // Shared memory: A 32 KB + 3 x 32 KB operand stages + 16 x 4 KB level-0 staging + 8 x 4 KB level-1 tiles = 224 KB.
 #include "build_common.cuh"
 #include "fused_common.cuh"
-
-// LGU_B16_TRACE (diagnostic builds only, tools/diag/b16_trace.py): per epilogue warp, cycles in (0) waiting for the
-// accumulator half, (1) the two tcgen05.ld, (2) waiting for the staging tile to be free, (3) staging writes + Gaussian patch,
-// (4) fence + syncwarp + store issue, (5) quadrant barrier A, (6) level-1 staging + barrier B, (7) in total.
-#ifdef LGU_B16_TRACE
-#define B16_T0() const long long _t0 = clock64()
-#define B16_ADD(slot) tr[slot] += clock64() - _t0
-#else
-#define B16_T0()
-#define B16_ADD(slot)
-#endif
 
 namespace lgu {
 
@@ -47,10 +36,9 @@ constexpr int kSmemBytes = kBarOffset + 256 + 1024;
 
 // FLAT: one [E,P,Q] volume of level-0 source maps x the maps behind map_b (lgu_build_volume: no Gaussian patch, no pooled
 // levels, any Q % 4 == 0, optional half mask) -- the epilogue is then barrier-free: tcgen05.ld -> staging tile -> LSU.
-template <bool L1_LSU, bool FLAT>
+template <bool FLAT>
 __global__ void __launch_bounds__(b16::kThreads, 1)
 build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_b,
-                       const __grid_constant__ CUtensorMap map_l0, const __grid_constant__ CUtensorMap map_l1,
                        const BpParams prm) {
   using namespace b16;
   extern __shared__ uint8_t smem_raw[];
@@ -79,8 +67,6 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&map_hi);
     prefetch_tmap(&map_b);
-    prefetch_tmap(&map_l0);
-    prefetch_tmap(&map_l1);
     mbar_init(a_full, 1);
     mbar_init(a_empty, 1);
     for (int s = 0; s < kStages; ++s) {
@@ -172,28 +158,15 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
     uint8_t* my_store = sStore + (warp - 2) * 4096;
     uint8_t* l1_mine = sL1 + (quad * 2 + rp) * 4096;    // the level-1 tile this warp half-fills
     const uint8_t* l1_rows[2] = {sL1 + (quad * 2 + 0) * 4096, sL1 + (quad * 2 + 1) * 4096};
-    const bool l1_issuer = sub == 0;                    // issues the quadrant's two level-1 tiles
     const int gr = prm.gauss_radius;
     const unsigned rdg = 2u * (unsigned)gr + 1u;
     const int rsw = lane & 7;                           // 128B swizzle phase of this thread's staging row
     const int x0 = xs * 32;
     const int bar_id = 1 + quad;                        // named barrier of the quadrant's four warps (128 threads)
-#ifdef LGU_B16_TRACE
-    long long tr[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    const long long tr_begin = clock64();
-#endif
 
-    // stage_tile: one 32-float row segment per lane into the warp's swizzled staging tile (the previous flush must have read
-    // it), Gaussian window patched in shared memory, patched values read back into v (they feed the pooled levels).
-    auto stage_tile = [&](float (&v)[32], bool patch, int yy, float mx, float my, float c1, float c2, float den, unsigned bx,
-                          bool lsu) {
-      if (!lsu || (!FLAT && prm.l0_lsu != 3)) {                  // a TMA store of this tile may still be reading it
-        B16_T0();
-        if (lane == 0) tma_wait_read<0>();
-        __syncwarp();
-        B16_ADD(2);
-      }
-      B16_T0();
+    // stage_tile: one 32-float row segment per lane into the warp's swizzled staging tile (the previous flush has read it),
+    // Gaussian window patched in shared memory, patched values read back into v (they feed the pooled levels).
+    auto stage_tile = [&](float (&v)[32], bool patch, int yy, float mx, float my, float c1, float c2, float den, unsigned bx) {
       float4* rowp = reinterpret_cast<float4*>(my_store + lane * 128);
 #pragma unroll
       for (int c = 0; c < 8; ++c) rowp[c ^ rsw] = make_float4(v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
@@ -217,41 +190,29 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
           }
         }
       }
-      B16_ADD(3);
     };
-    // flush_tile: the staged 32 x 32 tile to global memory.  LSU (default): a store instruction covers 4 rows x 128
-    // contiguous bytes (lane = row % 4 x 16-byte chunk) -- full lines, no proxy fence, no bulk-group wait before the tile is
-    // staged again (537 -> 505 us at E = 48 against TMA tile stores); loads in batches of four so that the stores do not
-    // serialise on one register quad.  Otherwise: one TMA tile store.
-    auto flush_tile = [&](int col, int row0, bool lsu) {
-      if (lsu) {
-        __syncwarp();
+    // flush_tile: the staged 32 x 32 tile to global memory.  A store instruction covers 4 rows x 128 contiguous bytes
+    // (lane = row % 4 x 16-byte chunk) -- full lines, no proxy fence, no bulk-group wait before the tile is staged again
+    // (537 -> 505 us at E = 48 against TMA tile stores); loads in batches of four so that the stores do not serialise on
+    // one register quad.
+    auto flush_tile = [&](int col, int row0) {
+      __syncwarp();
 #pragma unroll
-        for (int it0 = 0; it0 < 8; it0 += 4) {
-          float4 q[4];
+      for (int it0 = 0; it0 < 8; it0 += 4) {
+        float4 q[4];
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const int row = (it0 + j) * 4 + (lane >> 3), ch = lane & 7;
-            q[j] = *reinterpret_cast<const float4*>(my_store + row * 128 + ((ch ^ (row & 7)) << 4));
-          }
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const int row = (it0 + j) * 4 + (lane >> 3), ch = lane & 7;
-            if (!FLAT || col + ch * 4 < Q)                       // flat volumes: Q may end inside the last half
-              __stcs(reinterpret_cast<float4*>(prm.lvl0 + (size_t)(row0 + row) * (size_t)Q + col + ch * 4), q[j]);
-          }
+        for (int j = 0; j < 4; ++j) {
+          const int row = (it0 + j) * 4 + (lane >> 3), ch = lane & 7;
+          q[j] = *reinterpret_cast<const float4*>(my_store + row * 128 + ((ch ^ (row & 7)) << 4));
         }
-        __syncwarp();
-      } else {
-        B16_T0();
-        fence_proxy_async();
-        __syncwarp();
-        if (lane == 0 && !(prm.dbg & 1)) {
-          tma_store_2d(&map_l0, my_store, col, row0);
-          tma_commit();
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const int row = (it0 + j) * 4 + (lane >> 3), ch = lane & 7;
+          if (!FLAT || col + ch * 4 < Q)                         // flat volumes: Q may end inside the last half
+            __stcs(reinterpret_cast<float4*>(prm.lvl0 + (size_t)(row0 + row) * (size_t)Q + col + ch * 4), q[j]);
         }
-        B16_ADD(4);
       }
+      __syncwarp();
     };
 
     uint32_t half_it = 0;
@@ -320,30 +281,21 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
         if (!((hmask >> h) & 1u)) continue;
         const uint32_t buf = half_it & 1, buf_use = half_it >> 1;
         ++half_it;
-        {
-          B16_T0();
-          mbar_wait(t_full + buf, buf_use & 1);
-          B16_ADD(0);
-        }
+        mbar_wait(t_full + buf, buf_use & 1);
         tc_fence_after();
         const uint32_t tcol = tmem_base + lane_base + buf * 256 + xs * 32;
         const int ya = 4 * h + 2 * rp, yb = ya + 1;
         float ha[16], l1[16];
-        const bool lsu_a = FLAT || (prm.l0_lsu & 1) != 0, lsu_b = FLAT || (prm.l0_lsu & 2) != 0;
         uint32_t braw[32];
         {
           float a[32];
-          {
-            B16_T0();
-            tmem_ld32(tcol + (2 * rp) * 64, a);
-            B16_ADD(1);
-          }
+          tmem_ld32(tcol + (2 * rp) * 64, a);
           if (prm.round_half) {
 #pragma unroll
             for (int i = 0; i < 32; ++i) a[i] = __half2float(__float2half_rn(a[i]));
           }
           const bool pa = gr > 0 && ((unsigned)ya - by) < rdg;
-          stage_tile(a, pa, ya, mx, my, c1, c2, den, bx, lsu_a);
+          stage_tile(a, pa, ya, mx, my, c1, c2, den, bx);
           if (!FLAT) {
 #pragma unroll
             for (int i = 0; i < 16; ++i) ha[i] = __fadd_rn(a[2 * i], a[2 * i + 1]);
@@ -355,17 +307,13 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
           box_row(ya * 64 + x0);
           __syncwarp();
         } else {
-          flush_tile(ya * 64 + x0, row0, lsu_a);
+          flush_tile(ya * 64 + x0, row0);
         }
         {
           float b[32];
-          {
-            B16_T0();
-            tmem_ld32_wait(braw);
+          tmem_ld32_wait(braw);
 #pragma unroll
-            for (int i = 0; i < 32; ++i) b[i] = __uint_as_float(braw[i]);
-            B16_ADD(1);
-          }
+          for (int i = 0; i < 32; ++i) b[i] = __uint_as_float(braw[i]);
           tc_fence_before();                            // last TMEM read of this half by this warp
           __syncwarp();
           if (lane == 0) mbar_arrive(t_empty + buf);
@@ -374,14 +322,14 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
             for (int i = 0; i < 32; ++i) b[i] = __half2float(__float2half_rn(b[i]));
           }
           const bool pb = gr > 0 && ((unsigned)yb - by) < rdg;
-          stage_tile(b, pb, yb, mx, my, c1, c2, den, bx, lsu_b);
+          stage_tile(b, pb, yb, mx, my, c1, c2, den, bx);
           if (FLAT) {                                           // no pooled levels: nothing to exchange, no barrier
             if (cbox != nullptr) {
               __syncwarp();
               box_row(yb * 64 + x0);
               __syncwarp();
             } else {
-              flush_tile(yb * 64 + x0, row0, lsu_b);
+              flush_tile(yb * 64 + x0, row0);
             }
             continue;
           }
@@ -389,43 +337,28 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
 #pragma unroll
           for (int i = 0; i < 16; ++i) l1[i] = __fmul_rn(__fadd_rn(__fadd_rn(ha[i], b[2 * i]), b[2 * i + 1]), 0.25f);
         }
-        flush_tile(yb * 64 + x0, row0, lsu_b);
-        // ---- level 1: quadrant barrier A (the tiles of the previous half were read by the engine -- the issuer's
-        // wait_read before its level-0 stores of this half -- and by every warp's level-2 pass), stage, barrier B, store
-        {
-          B16_T0();
-          asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
-          B16_ADD(5);
-        }
-        B16_T0();
+        flush_tile(yb * 64 + x0, row0);
+        // ---- level 1: quadrant barrier A (every warp has stored its rows of the previous half's tiles and read them for
+        // its level-2 pass), stage, barrier B, store
+        asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
         {
           float4* rowp = reinterpret_cast<float4*>(l1_mine + lane * 128);
 #pragma unroll
           for (int c = 0; c < 4; ++c)
             rowp[(xs * 4 + c) ^ rsw] = make_float4(l1[4 * c], l1[4 * c + 1], l1[4 * c + 2], l1[4 * c + 3]);
         }
-        if (!L1_LSU) fence_proxy_async();
         asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
-        B16_ADD(6);
-        if (prm.dbg & 2) {
-        } else if (L1_LSU) {
-          // The TMA store engine is what bounds this kernel (one 128-byte row segment per ~7 cycles and SM): the level-1
-          // tiles -- a fifth of its row segments -- leave through the LSU instead.  Each warp takes 8 rows of both tiles;
-          // a store instruction covers 4 rows x 128 contiguous bytes (lane = row % 4 x 16-byte chunk), i.e. full lines.
+        // Each warp stores 8 rows of both tiles through the LSU (559 -> 543 us at E = 48 against TMA tile stores); a store
+        // instruction covers 4 rows x 128 contiguous bytes (lane = row % 4 x 16-byte chunk), i.e. full lines.
 #pragma unroll
-          for (int tix = 0; tix < 2; ++tix) {
+        for (int tix = 0; tix < 2; ++tix) {
 #pragma unroll
-            for (int rr = 0; rr < 2; ++rr) {
-              const int row = sub * 8 + rr * 4 + (lane >> 3), ch = lane & 7;
-              const float4 vv = *reinterpret_cast<const float4*>(l1_rows[tix] + row * 128 + ((ch ^ (row & 7)) << 4));
-              float* dst = prm.lvl1 + (size_t)(row0 + row) * (size_t)(Q >> 2) + (2 * h + tix) * 32 + ch * 4;
-              __stcs(reinterpret_cast<float4*>(dst), vv);
-            }
+          for (int rr = 0; rr < 2; ++rr) {
+            const int row = sub * 8 + rr * 4 + (lane >> 3), ch = lane & 7;
+            const float4 vv = *reinterpret_cast<const float4*>(l1_rows[tix] + row * 128 + ((ch ^ (row & 7)) << 4));
+            float* dst = prm.lvl1 + (size_t)(row0 + row) * (size_t)(Q >> 2) + (2 * h + tix) * 32 + ch * 4;
+            __stcs(reinterpret_cast<float4*>(dst), vv);
           }
-        } else if (l1_issuer && lane == 0) {
-          tma_store_2d(&map_l1, l1_rows[0], (2 * h) * 32, row0);
-          tma_store_2d(&map_l1, l1_rows[1], (2 * h + 1) * 32, row0);
-          tma_commit();
         }
         // ---- level 2 (and 3): this warp's quarter of the row, from the two level-1 tiles in shared memory
         {
@@ -438,7 +371,6 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
           l2[1] = __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(u0.z, u0.w), w0.z), w0.w), 0.25f);
           l2[2] = __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(u1.x, u1.y), w1.x), w1.y), 0.25f);
           l2[3] = __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(u1.z, u1.w), w1.z), w1.w), 0.25f);
-          if (!(prm.dbg & 4))
           *reinterpret_cast<float4*>(prm.lvl2 + pix * (size_t)(Q >> 4) + h * 16 + sub * 4) =
               make_float4(l2[0], l2[1], l2[2], l2[3]);
           if ((h & 1) == 0) {
@@ -447,19 +379,11 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
           } else {
             const float l3a = __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(l2_prev[0], l2_prev[1]), l2[0]), l2[1]), 0.25f);
             const float l3b = __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(l2_prev[2], l2_prev[3]), l2[2]), l2[3]), 0.25f);
-            if (!(prm.dbg & 4))
             *reinterpret_cast<float2*>(prm.lvl3 + pix * (size_t)(Q >> 6) + (h >> 1) * 8 + sub * 2) = make_float2(l3a, l3b);
           }
         }
       }
     }
-    if (lane == 0) tma_wait_all();
-    __syncwarp();
-#ifdef LGU_B16_TRACE
-    tr[7] = clock64() - tr_begin;
-    if (lane == 0 && prm.trace != nullptr)
-      for (int q = 0; q < 8; ++q) atomicAdd(prm.trace + q, (unsigned long long)tr[q]);
-#endif
   }
 
   tc_fence_before();
@@ -467,18 +391,14 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-int launch_build16(const CUtensorMap& mh, const CUtensorMap& mb, const CUtensorMap& m0, const CUtensorMap& m1, const BpParams& prm,
-                   bool flat, cudaStream_t st) {
-  // level-1 tiles through the LSU (default; 559 -> 540 us at E = 48); LGU_BUILD_L1_TMA=1: through the TMA store engine
-  const bool l1_lsu = !env_flag("LGU_BUILD_L1_TMA") && prm.lvl1 != nullptr;
-  auto kern = flat ? build_pyramid16_kernel<true, true>
-                   : (l1_lsu ? build_pyramid16_kernel<true, false> : build_pyramid16_kernel<false, false>);
+int launch_build16(const CUtensorMap& mh, const CUtensorMap& mb, const BpParams& prm, bool flat, cudaStream_t st) {
+  auto kern = flat ? build_pyramid16_kernel<true> : build_pyramid16_kernel<false>;
   if (int rc = optin_smem(reinterpret_cast<const void*>(kern), b16::kSmemBytes, "lgu_build_pyramid")) return rc;
   int dev = 0, sms = kNumSMs;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int grid = prm.num_units < sms ? prm.num_units : sms;
-  kern<<<grid, b16::kThreads, b16::kSmemBytes, st>>>(mh, mb, m0, m1, prm);
+  kern<<<grid, b16::kThreads, b16::kSmemBytes, st>>>(mh, mb, prm);
   return check_launch(flat ? "lgu_build_volume(16)" : "lgu_build_pyramid(16)");
 }
 

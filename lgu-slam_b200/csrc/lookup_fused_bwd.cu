@@ -25,7 +25,6 @@
 //   g_var     = g_m * m * (1 - m)                             (sigmoid, corr.py:97)
 //   g_v[k]    = g_var * 2 (v[k] - mean) / 8                   (unbiased 9-tap variance, corr.py:96)
 //   gV_1     += corr_index_backward(g_v)                      (corrSample_kernel.cu:84-136)
-#include <cstdlib>
 #include "fused_common.cuh"
 #include "gauss_window.cuh"
 
@@ -322,7 +321,7 @@ __device__ __forceinline__ void emit_window(float* __restrict__ gw, float (&out)
 // finished HERE: the merged window gradient is in registers (emit_window), the 81 window values of level 0 are fetched at
 // the top of the pixel, and gauss_window_grads -- the arithmetic of lgu_build_backward_gauss, shared code -- gives the
 // pixel's (means, covs, den) gradients.  The separate kernel was bound by its window gathers from the dense gradients.
-template <bool ACC, bool BULK, bool FXP, bool GAUSS = false>
+template <bool ACC, bool BULK, bool GAUSS = false>
 __global__ void __launch_bounds__(fl::kThreads, 2)
 lookup_fused_bwd_kernel(const __grid_constant__ FusedMaps maps, const FusedLookupBwdParams prm) {
   using namespace flb;
@@ -553,7 +552,7 @@ lookup_fused_bwd_kernel(const __grid_constant__ FusedMaps maps, const FusedLooku
     // fixed-point scale of this pixel: 2^(22 - exponent of the largest |gradient|); warp-uniform.  Falls back to the
     // float path for non-finite or vanishing gradients.
     float fxp_scale = 0.0f, fxp_inv = 0.0f;
-    if (FXP) {
+    {
       float mx = fmaxf(fmaxf(fabsf(ga0), fabsf(ga1)), has1 ? fmaxf(fabsf(gb0), fabsf(gb1)) : 0.0f);
       // NaN sampling positions make NaN weights, which must propagate like in the reference: float path.  (Infinite or
       // huge positions are gated out -- a gated-in tap has a fraction in [0, 1), so |w g| <= |g|.)
@@ -568,7 +567,7 @@ lookup_fused_bwd_kernel(const __grid_constant__ FusedMaps maps, const FusedLooku
         fxp_inv = __int_as_float((127 - 22 + ex) << 23);
       }
     }
-    const bool fxp = FXP && fxp_scale != 0.0f;
+    const bool fxp = fxp_scale != 0.0f;
     const int xb0 = box_origin_x(floor_to_int(x0), 7, prm.W2[0]), yb0 = box_origin_y(floor_to_int(y0), 7, prm.H2[0]);
     const int xb1 = box_origin_x(floor_to_int(x1c), 7, prm.W2[1]), yb1 = box_origin_y(floor_to_int(y1c), 7, prm.H2[1]);
     auto deform_bwd = [&](int l, const float* bx, int xb, int yb, float cx, float cy, float2 oa, float2 ob, BTap& ta,
@@ -928,24 +927,16 @@ static int lgu::launch_lookup_fused_bwd(const float* lvl0, const float* lvl1, co
   // Schedule.  Accumulate mode (footprint-only reductions): persistent, two CTAs per SM, every CTA the same number of
   // tiles (4608 tiles -> 288 CTAs x 16) -- 431 -> 373 us at E = 48.  Dense mode (every slice streamed once, write-bound):
   // one tile per CTA -- persistent CTAs run in lock step and write in phase (690 us against 601 us); the hardware's CTA
-  // scheduler staggers them.  LGU_BWD_TILES_PER_CTA overrides (experiments).
-  long long per_cta = accumulate ? (ntiles + 2LL * sms - 1) / (2LL * sms) : 1;
-  if (const char* gk = getenv("LGU_BWD_TILES_PER_CTA")) {
-    const long long v = atoll(gk);
-    if (v > 0) per_cta = v;
-  }
+  // scheduler staggers them.
+  const long long per_cta = accumulate ? (ntiles + 2LL * sms - 1) / (2LL * sms) : 1;
   const long long nblk = (ntiles + per_cta - 1) / per_cta;
-  // bulk zero-fill needs row bands that tile a warp (W2 / 4 divides 32 at levels 0 and 1)
-  const char* nb = getenv("LGU_BWD_NOBULK");
-  const bool bulk = !accumulate && (W == 64 || W == 128) && !(nb != nullptr && nb[0] != '\0' && nb[0] != '0');
-  // LGU_BWD_FLOAT_ATOMICS=1: the first version's float compare-and-swap scatter instead of the fixed-point one
-  const char* fa = getenv("LGU_BWD_FLOAT_ATOMICS");
-  const bool fxp = !(fa != nullptr && fa[0] != '\0' && fa[0] != '0');
-  auto kern = accumulate ? (fxp ? lookup_fused_bwd_kernel<true, false, true> : lookup_fused_bwd_kernel<true, false, false>)
-              : bulk     ? (fxp ? lookup_fused_bwd_kernel<false, true, true> : lookup_fused_bwd_kernel<false, true, false>)
-                         : (fxp ? lookup_fused_bwd_kernel<false, false, true> : lookup_fused_bwd_kernel<false, false, false>);
-  if (gauss)   // dense mode only (the fixed-point scatter always: the float-atomics switch is an experiment of the plain form)
-    kern = bulk ? lookup_fused_bwd_kernel<false, true, true, true> : lookup_fused_bwd_kernel<false, false, true, true>;
+  // bulk zero-fill (-4 %) needs row bands that tile a warp (W2 / 4 divides 32 at levels 0 and 1)
+  const bool bulk = !accumulate && (W == 64 || W == 128);
+  auto kern = accumulate ? lookup_fused_bwd_kernel<true, false>
+              : bulk     ? lookup_fused_bwd_kernel<false, true>
+                         : lookup_fused_bwd_kernel<false, false>;
+  if (gauss)   // dense mode only
+    kern = bulk ? lookup_fused_bwd_kernel<false, true, true> : lookup_fused_bwd_kernel<false, false, true>;
   if (int rc = optin_smem(reinterpret_cast<const void*>(kern), flb::kSmemBytes, "lgu_corr_lookup_fused_backward")) return rc;
   kern<<<(unsigned)nblk, fl::kThreads, flb::kSmemBytes, (cudaStream_t)stream>>>(maps, prm);
   return check_launch("lgu_corr_lookup_fused_backward");

@@ -45,11 +45,6 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void*
                "r"(smem_u32(src)), "r"(c0), "r"(c1)
                : "memory");
 }
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, const void* src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.tile.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(map),
-               "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2)
-               : "memory");
-}
 __device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void tma_wait_read() {
@@ -195,36 +190,6 @@ static inline int make_map_2d(CUtensorMap* map, CUtensorMapDataType dt, int elem
                   swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     set_error("cuTensorMapEncodeTiled failed with CUresult %d (rows=%llu cols=%llu)", (int)r,
-              (unsigned long long)rows, (unsigned long long)cols);
-    return LGU_ERR_LAUNCH;
-  }
-  map_cache_put(key, map);
-  return LGU_OK;
-}
-
-// Row-major fp32 matrix [rows, cols] (cols % 32 == 0) seen as {32 floats, rows, cols / 32 chunks}: one box of
-// {32, box_rows, box_chunks} moves box_chunks * 128 CONTIGUOUS bytes per row (128B-swizzled 4 KB sub-tiles in smem).
-static inline int make_map_chunked(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint32_t box_rows,
-                                   uint32_t box_chunks) {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const MapKey key = {{3u, (uint64_t)dev, (uint64_t)reinterpret_cast<uintptr_t>(base), rows, cols, box_rows, box_chunks, 0,
-                       0, 0, 0, 0}};
-  if (map_cache_get(key, map)) return LGU_OK;
-  EncodeTiledFn fn = get_encode_fn();
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return LGU_ERR_LAUNCH;
-  }
-  const cuuint64_t dims[3] = {32, rows, cols / 32};
-  const cuuint64_t strides[2] = {cols * 4, 128};
-  const cuuint32_t box[3] = {32, box_rows, box_chunks};
-  const cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (chunked) failed with CUresult %d (rows=%llu cols=%llu)", (int)r,
               (unsigned long long)rows, (unsigned long long)cols);
     return LGU_ERR_LAUNCH;
   }
