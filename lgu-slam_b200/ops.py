@@ -7,8 +7,6 @@ unpack with `x, = op(...)`); the only checks the reference performs are `is_cont
 (droid.cpp:48-49) and the accessor's dtype/ndim checks, which surface as RuntimeError -- same here,
 plus explicit device/shape checks.  torch is used only for allocation and the current stream.
 """
-import ctypes
-
 import torch
 
 from . import _lib
@@ -27,16 +25,58 @@ def _chk(t, name, ndim, dtype=torch.float32):
         raise RuntimeError(f"{name}: expected {ndim} dimensions, got {t.dim()}")
 
 
-def _p(t):
-    return ctypes.c_void_p(t.data_ptr())
+def _launch(name, device, *args):
+    """Call entry point `name` on `device` with the device's current stream appended; a non-zero status raises."""
+    with torch.cuda.device(device):
+        return _lib.call(name, *args, torch.cuda.current_stream(device).cuda_stream)
 
 
-def _stream(t):
-    return ctypes.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
+def _check_levels(levels, S, H, W, name, skip=()):
+    """Pyramid levels [S,H,W,H>>l,W>>l] (fp32, contiguous, CUDA); the levels listed in `skip` are not read."""
+    for l, t in enumerate(levels):
+        if l not in skip:
+            _chk(t, f"{name}[{l}]", 5)
+            if tuple(t.shape) != (S, H, W, H >> l, W >> l):
+                raise RuntimeError(f"{name}[{l}] shape {tuple(t.shape)} != {(S, H, W, H >> l, W >> l)}")
 
 
-def _i(v):
-    return ctypes.c_int(int(v))
+def _check_offsets(numel, exact=True, **offsets):
+    """Offset tensors [*,H,W,98] / [*,H,W,7,7,2]: contiguous fp32 CUDA with `numel` elements (at least `numel` if not
+    exact)."""
+    for name, o in offsets.items():
+        if not (isinstance(o, torch.Tensor) and o.is_cuda and o.is_contiguous() and o.dtype == torch.float32
+                and (o.numel() == numel if exact else o.numel() >= numel)):
+            raise RuntimeError(f"{name} must be a contiguous fp32 CUDA tensor with {'' if exact else '>= '}{numel} elements")
+
+
+def _check_index(t, name, n=None):
+    """A contiguous CUDA int32 vector (edge / slot / row indices), with n entries if n is given."""
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.int32 and t.dim() == 1 and t.is_contiguous()
+            and (n is None or t.numel() == n)):
+        raise RuntimeError(f"{name} must be a contiguous CUDA int32 vector" + ("" if n is None else f" with {n} entries"))
+
+
+def _check_plane(t, name):
+    """A channels-last fp16 plane [T,P,C] as pack_fmaps returns it."""
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float16 and t.dim() == 3 and t.is_contiguous()):
+        raise RuntimeError(f"{name} must be a contiguous CUDA fp16 tensor [T,P,C] (see pack_fmaps)")
+
+
+def _check_means_covs(means, covs, E, H, W):
+    """The Gaussian parameters: means, covs [E,H,W,2] (channel 0 = x, 1 = y)."""
+    _chk(means, "means", 4); _chk(covs, "covs", 4)
+    if tuple(means.shape) != (E, H, W, 2) or tuple(covs.shape) != (E, H, W, 2):
+        raise RuntimeError(f"means/covs must be [E,H,W,2] = {[E, H, W, 2]}")
+
+
+def _encoder_weight(weight):
+    """corr_encoder[0].weight [128,196] or [128,196,1,1] -> contiguous [128,196], the only shape the kernels implement."""
+    if not (isinstance(weight, torch.Tensor) and weight.is_cuda and weight.dtype == torch.float32):
+        raise RuntimeError("weight must be a CUDA fp32 tensor")
+    w = weight.detach().reshape(weight.shape[0], -1).contiguous()
+    if tuple(w.shape) != (128, 196):
+        raise RuntimeError(f"only the 196 -> 128 corr_encoder is implemented, got weight {tuple(weight.shape)}")
+    return w
 
 
 def corr_index_forward(volume, coords, radius):
@@ -47,10 +87,7 @@ def corr_index_forward(volume, coords, radius):
         raise RuntimeError(f"coords shape {tuple(coords.shape)} != {(E, 2, H1, W1)}")
     rd = 2 * int(radius) + 1
     corr = torch.empty(E, rd, rd, H1, W1, dtype=volume.dtype, device=volume.device)
-    with torch.cuda.device(volume.device):
-        st = _lib.lib().lgu_corr_index_forward(_p(volume), _p(coords), _p(corr), _i(E), _i(H1), _i(W1), _i(H2),
-                                               _i(W2), _i(radius), _stream(volume))
-    _lib.check(st, "corr_index_forward")
+    _launch("lgu_corr_index_forward", volume.device, volume, coords, corr, E, H1, W1, H2, W2, int(radius))
     return [corr]
 
 
@@ -62,10 +99,7 @@ def corr_index_backward(volume, coords, corr_grad, radius):
     if tuple(corr_grad.shape) != (E, rd, rd, H1, W1):
         raise RuntimeError(f"corr_grad shape {tuple(corr_grad.shape)} != {(E, rd, rd, H1, W1)}")
     volume_grad = torch.empty_like(volume)
-    with torch.cuda.device(volume.device):
-        st = _lib.lib().lgu_corr_index_backward(_p(coords), _p(corr_grad), _p(volume_grad), _i(E), _i(H1), _i(W1),
-                                                _i(H2), _i(W2), _i(radius), _stream(volume))
-    _lib.check(st, "corr_index_backward")
+    _launch("lgu_corr_index_backward", volume.device, coords, corr_grad, volume_grad, E, H1, W1, H2, W2, int(radius))
     return [volume_grad]
 
 
@@ -79,10 +113,7 @@ def defCorr_index_forward(volume, coords, offset, radius):
     if tuple(coords.shape) != (E, 2, H1, W1):
         raise RuntimeError(f"coords shape {tuple(coords.shape)} != {(E, 2, H1, W1)}")
     corr = torch.empty(E, rd, rd, H1, W1, dtype=volume.dtype, device=volume.device)
-    with torch.cuda.device(volume.device):
-        st = _lib.lib().lgu_defcorr_index_forward(_p(volume), _p(coords), _p(offset), _p(corr), _i(E), _i(H1),
-                                                  _i(W1), _i(H2), _i(W2), _i(radius), _stream(volume))
-    _lib.check(st, "defCorr_index_forward")
+    _launch("lgu_defcorr_index_forward", volume.device, volume, coords, offset, corr, E, H1, W1, H2, W2, int(radius))
     return [corr]
 
 
@@ -97,43 +128,32 @@ def defCorr_index_backward(volume, coords, offset, corr_grad, radius):
         raise RuntimeError(f"corr_grad shape {tuple(corr_grad.shape)} != {(E, rd, rd, H1, W1)}")
     volume_grad = torch.empty_like(volume)
     offset_grad = torch.empty_like(offset)
-    with torch.cuda.device(volume.device):
-        st = _lib.lib().lgu_defcorr_index_backward(_p(volume), _p(coords), _p(offset), _p(corr_grad),
-                                                   _p(volume_grad), _p(offset_grad), _i(E), _i(H1), _i(W1), _i(H2),
-                                                   _i(W2), _i(radius), _stream(volume))
-    _lib.check(st, "defCorr_index_backward")
+    _launch("lgu_defcorr_index_backward", volume.device, volume, coords, offset, corr_grad, volume_grad, offset_grad, E,
+            H1, W1, H2, W2, int(radius))
     return [volume_grad, offset_grad]
 
 
 def gaussianMask(means, covs, volume, radius):
     """droid.cpp:100-110.  means, covs [E,H1,W1,2] -> [volume1] (dense, zero outside the window)."""
-    _chk(means, "means", 4); _chk(covs, "covs", 4); _chk(volume, "volume", 5)
+    _chk(volume, "volume", 5)
     E, H1, W1, H2, W2 = volume.shape
-    if tuple(means.shape) != (E, H1, W1, 2) or tuple(covs.shape) != (E, H1, W1, 2):
-        raise RuntimeError("means/covs must be [E,H1,W1,2]")
+    _check_means_covs(means, covs, E, H1, W1)
     out = torch.empty_like(volume)
-    with torch.cuda.device(volume.device):
-        st = _lib.lib().lgu_gaussian_mask_forward(_p(means), _p(covs), _p(volume), _p(out), _i(E), _i(H1), _i(W1),
-                                                  _i(H2), _i(W2), _i(radius), _stream(volume))
-    _lib.check(st, "gaussianMask")
+    _launch("lgu_gaussian_mask_forward", volume.device, means, covs, volume, out, E, H1, W1, H2, W2, int(radius))
     return [out]
 
 
 def gaussianMask_backward(means, covs, volume, volume1_grad, radius):
     """droid.cpp:112-123 -> [means_grad, covs_grad]."""
-    _chk(means, "means", 4); _chk(covs, "covs", 4); _chk(volume, "volume", 5); _chk(volume1_grad, "volume_grad", 5)
+    _chk(volume, "volume", 5); _chk(volume1_grad, "volume_grad", 5)
     E, H1, W1, H2, W2 = volume.shape
-    if tuple(means.shape) != (E, H1, W1, 2) or tuple(covs.shape) != (E, H1, W1, 2):
-        raise RuntimeError("means/covs must be [E,H1,W1,2]")
+    _check_means_covs(means, covs, E, H1, W1)
     if volume1_grad.shape != volume.shape:
         raise RuntimeError("volume_grad must have the volume's shape")
     gm = torch.empty_like(means)
     gc = torch.empty_like(covs)
-    with torch.cuda.device(volume.device):
-        st = _lib.lib().lgu_gaussian_mask_backward(_p(means), _p(covs), _p(volume), _p(volume1_grad), _p(gm), _p(gc),
-                                                   _i(E), _i(H1), _i(W1), _i(H2), _i(W2), _i(radius),
-                                                   _stream(volume))
-    _lib.check(st, "gaussianMask_backward")
+    _launch("lgu_gaussian_mask_backward", volume.device, means, covs, volume, volume1_grad, gm, gc, E, H1, W1, H2, W2,
+            int(radius))
     return [gm, gc]
 
 
@@ -158,17 +178,17 @@ def release_workspace():
 
 
 def _ws_bytes(B, N, H1, W1, H2, W2, C, radius):
-    L = _lib.lib()
-    L.lgu_lowmem_workspace_bytes.restype = ctypes.c_longlong
-    return int(L.lgu_lowmem_workspace_bytes(_i(B), _i(N), _i(H1), _i(W1), _i(H2), _i(W2), _i(C), _i(radius)))
+    return _lib.call("lgu_lowmem_workspace_bytes", B, N, H1, W1, H2, W2, C, radius)
 
 
-def _sub_batches(B, per_call_bytes_fn):
-    """Split B edges into runs whose workspace fits LOWMEM_WORKSPACE_CAP (usually one run)."""
+def _tensor_core_runs(device, B, N, H1, W1, H2, W2, C, radius):
+    """Split B edges into runs whose workspace fits LOWMEM_WORKSPACE_CAP (usually one run): yields (b0, b1, workspace)."""
     step = B
-    while step > 1 and per_call_bytes_fn(step) > LOWMEM_WORKSPACE_CAP:
+    while step > 1 and _ws_bytes(step, N, H1, W1, H2, W2, C, radius) > LOWMEM_WORKSPACE_CAP:
         step = (step + 1) // 2
-    return [(s0, min(B, s0 + step)) for s0 in range(0, B, step)]
+    for b0 in range(0, B, step):
+        b1 = min(B, b0 + step)
+        yield b0, b1, _workspace(device, _ws_bytes(b1 - b0, N, H1, W1, H2, W2, C, radius))
 
 
 def lowMem_defSample(fmap1, fmap2, coords, offset, radius, strict_ref=True, tensor_cores=True):
@@ -189,24 +209,15 @@ def lowMem_defSample(fmap1, fmap2, coords, offset, radius, strict_ref=True, tens
     if tuple(offset.shape[1:]) != (H1, W1, rd, rd, 2) or offset.shape[0] < need:
         raise RuntimeError(f"offset shape {tuple(offset.shape)} incompatible with {(need, H1, W1, rd, rd, 2)}")
     corr = torch.empty(B, N, rd, rd, H1, W1, dtype=fmap1.dtype, device=fmap1.device)
+    radius, strict = int(radius), 1 if strict_ref else 0
     if tensor_cores and B > 0 and _ws_bytes(B, N, H1, W1, H2, W2, C, radius) > 0:
-        runs = _sub_batches(B, lambda b: _ws_bytes(b, N, H1, W1, H2, W2, C, radius))
-        with torch.cuda.device(fmap1.device):
-            for b0, b1 in runs:
-                nb = _ws_bytes(b1 - b0, N, H1, W1, H2, W2, C, radius)
-                ws = _workspace(fmap1.device, nb)
-                off = offset if strict_ref else offset[b0:]          # strict: every run reads slab 0 of the call (Q2)
-                st = _lib.lib().lgu_lowmem_defsample_forward_ws(
-                    _p(fmap1[b0:b1]), _p(fmap2[b0:b1]), _p(coords[b0:b1]), _p(off), _p(corr[b0:b1]), _i(b1 - b0), _i(N),
-                    _i(H1), _i(W1), _i(H2), _i(W2), _i(C), _i(radius), _i(1 if strict_ref else 0), _p(ws),
-                    ctypes.c_longlong(ws.numel()), _stream(fmap1))
-                _lib.check(st, "lowMem_defSample (tensor cores)")
-        return [corr]
-    with torch.cuda.device(fmap1.device):
-        st = _lib.lib().lgu_lowmem_defsample_forward(_p(fmap1), _p(fmap2), _p(coords), _p(offset), _p(corr), _i(B),
-                                                     _i(N), _i(H1), _i(W1), _i(H2), _i(W2), _i(C), _i(radius),
-                                                     _i(1 if strict_ref else 0), _stream(fmap1))
-    _lib.check(st, "lowMem_defSample")
+        for b0, b1, ws in _tensor_core_runs(fmap1.device, B, N, H1, W1, H2, W2, C, radius):
+            off = offset if strict_ref else offset[b0:]              # strict: every run reads slab 0 of the call (Q2)
+            _launch("lgu_lowmem_defsample_forward_ws", fmap1.device, fmap1[b0:b1], fmap2[b0:b1], coords[b0:b1], off,
+                    corr[b0:b1], b1 - b0, N, H1, W1, H2, W2, C, radius, strict, ws, ws.numel())
+    else:
+        _launch("lgu_lowmem_defsample_forward", fmap1.device, fmap1, fmap2, coords, offset, corr, B, N, H1, W1, H2, W2, C,
+                radius, strict)
     return [corr]
 
 
@@ -222,20 +233,13 @@ def altcorr_forward(fmap1, fmap2, coords, radius, tensor_cores=True):
     if B2 != B or C2 != C or Bc != B or (Hc, Wc, two) != (H1, W1, 2):
         raise RuntimeError("altcorr_forward: inconsistent fmap/coords shapes")
     corr = torch.empty(B, N, rd * rd, H1, W1, dtype=fmap1.dtype, device=fmap1.device)
+    radius = int(radius)
     if tensor_cores and B > 0 and _ws_bytes(B, N, H1, W1, H2, W2, C, radius) > 0:
-        runs = _sub_batches(B, lambda b: _ws_bytes(b, N, H1, W1, H2, W2, C, radius))
-        with torch.cuda.device(fmap1.device):
-            for b0, b1 in runs:
-                ws = _workspace(fmap1.device, _ws_bytes(b1 - b0, N, H1, W1, H2, W2, C, radius))
-                st = _lib.lib().lgu_altcorr_forward_ws(
-                    _p(fmap1[b0:b1]), _p(fmap2[b0:b1]), _p(coords[b0:b1]), _p(corr[b0:b1]), _i(b1 - b0), _i(N), _i(H1),
-                    _i(W1), _i(H2), _i(W2), _i(C), _i(radius), _p(ws), ctypes.c_longlong(ws.numel()), _stream(fmap1))
-                _lib.check(st, "altcorr_forward (tensor cores)")
-        return [corr]
-    with torch.cuda.device(fmap1.device):
-        st = _lib.lib().lgu_altcorr_forward(_p(fmap1), _p(fmap2), _p(coords), _p(corr), _i(B), _i(N), _i(H1), _i(W1),
-                                            _i(H2), _i(W2), _i(C), _i(radius), _stream(fmap1))
-    _lib.check(st, "altcorr_forward")
+        for b0, b1, ws in _tensor_core_runs(fmap1.device, B, N, H1, W1, H2, W2, C, radius):
+            _launch("lgu_altcorr_forward_ws", fmap1.device, fmap1[b0:b1], fmap2[b0:b1], coords[b0:b1], corr[b0:b1], b1 - b0,
+                    N, H1, W1, H2, W2, C, radius, ws, ws.numel())
+    else:
+        _launch("lgu_altcorr_forward", fmap1.device, fmap1, fmap2, coords, corr, B, N, H1, W1, H2, W2, C, radius)
     return [corr]
 
 
@@ -254,10 +258,7 @@ def offset_heads(c0, c1, eps=1e-5):
     off0 = torch.empty(E, H, W, CH, dtype=torch.float32, device=c0.device)
     off1 = torch.empty_like(off0)
     stats = torch.empty(E, 4, dtype=torch.float32, device=c0.device)
-    with torch.cuda.device(c0.device):
-        st = _lib.lib().lgu_offset_heads(_p(c0), _p(c1), _p(off0), _p(off1), _p(stats), _i(E), _i(CH), _i(H), _i(W),
-                                         ctypes.c_float(eps), _stream(c0))
-    _lib.check(st, "offset_heads")
+    _launch("lgu_offset_heads", c0.device, c0, c1, off0, off1, stats, E, CH, H, W, eps)
     return off0, off1
 
 
@@ -272,11 +273,7 @@ def pack_fmaps(fmaps, split=False):
     T, C, H, W = fmaps.shape
     hi = torch.empty(T, H * W, C, dtype=torch.float16, device=fmaps.device)
     lo = torch.empty_like(hi) if split else None
-    with torch.cuda.device(fmaps.device):
-        st = _lib.lib().lgu_pack_fmaps(_p(fmaps), _i(fmaps.dtype == torch.float16), _p(hi),
-                                       _p(lo) if split else ctypes.c_void_p(0), _i(T), _i(C), _i(H * W),
-                                       _stream(fmaps))
-    _lib.check(st, "pack_fmaps")
+    _launch("lgu_pack_fmaps", fmaps.device, fmaps, fmaps.dtype == torch.float16, hi, lo, T, C, H * W)
     return hi, lo
 
 
@@ -288,61 +285,45 @@ def build_pyramid(hi, lo, ii, jj, H, W, means=None, covs=None, den=None, num_lev
     Returns [lvl0 [E,H,W,H,W], lvl1 [E,H,W,H/2,W/2], ...].
     Edge-slot pool: out = the pool's level storages [S,H,W,H>>l,W>>l] and out_slots = int32 [E] slot of each edge;
     the levels are then written in place (nothing is allocated) and `out` is returned."""
-    if hi.dtype != torch.float16 or not hi.is_cuda or hi.dim() != 3 or not hi.is_contiguous():
-        raise RuntimeError("hi must be a contiguous CUDA fp16 tensor [T,H*W,C] (see pack_fmaps)")
+    _check_plane(hi, "hi")
     T, P, C = hi.shape
     if P != H * W:
         raise RuntimeError(f"hi has {P} pixels per map, expected H*W = {H * W}")
-    if precision is None:
-        precision = 2 if lo is not None else 1
-    if precision == 2 and (lo is None or lo.shape != hi.shape or lo.dtype != torch.float16):
-        raise RuntimeError("precision 2 needs the lo plane from pack_fmaps(split=True)")
-    for t, name in ((ii, "ii"), (jj, "jj")):
-        if not (t.is_cuda and t.dtype == torch.int32 and t.dim() == 1 and t.is_contiguous()):
-            raise RuntimeError(f"{name} must be a contiguous CUDA int32 vector")
+    precision = int(precision) if precision is not None else 2 if lo is not None else 1
+    if precision == 2:
+        _check_plane(lo, "lo")
+        if lo.shape != hi.shape:
+            raise RuntimeError("precision 2 needs the lo plane from pack_fmaps(split=True)")
+    else:
+        lo = None
+    _check_index(ii, "ii")
     E = ii.numel()
-    if jj.numel() != E:
-        raise RuntimeError("ii and jj must have the same length")
-    use_gauss = gauss_radius > 0 and means is not None
-    if use_gauss:
-        _chk(means, "means", 4); _chk(covs, "covs", 4)
-        if tuple(means.shape) != (E, H, W, 2) or tuple(covs.shape) != (E, H, W, 2):
-            raise RuntimeError("means/covs must be [E,H,W,2]")
+    _check_index(jj, "jj", E)
+    gauss_radius = int(gauss_radius) if gauss_radius > 0 and means is not None else 0
+    if gauss_radius:
+        _check_means_covs(means, covs, E, H, W)
         if den is not None:                      # None: the kernel forms 6.28*sqrt(cov_x*cov_y) in its prologue
             _chk(den, "den", 3)
             if tuple(den.shape) != (E, H, W):
                 raise RuntimeError("den must be [E,H,W]")
+    else:
+        means = covs = den = None
     if not 1 <= num_levels <= 4:
         raise RuntimeError("num_levels must be in 1..4")
-    null = ctypes.c_void_p(0)
-    if out is not None:
-        if out_slots is None or not (out_slots.is_cuda and out_slots.dtype == torch.int32 and out_slots.numel() == E
-                                     and out_slots.is_contiguous()):
-            raise RuntimeError("out_slots must be a contiguous CUDA int32 vector with one slot per edge")
-        S = out[0].shape[0]
-        for l, t in enumerate(out[:num_levels]):
-            _chk(t, f"out[{l}]", 5)
-            if tuple(t.shape) != (S, H, W, H >> l, W >> l):
-                raise RuntimeError(f"out[{l}] shape {tuple(t.shape)} != {(S, H, W, H >> l, W >> l)}")
-        lv = list(out[:num_levels])
-        ptr = [_p(t) for t in lv] + [null] * (4 - num_levels)
-        with torch.cuda.device(hi.device):
-            st = _lib.lib().lgu_build_pyramid_slots(
-                _p(hi), _p(lo) if precision == 2 else null, _p(ii), _p(jj), _p(means) if use_gauss else null,
-                _p(covs) if use_gauss else null, _p(den) if (use_gauss and den is not None) else null, ptr[0], ptr[1], ptr[2],
-                ptr[3], _p(out_slots), _i(S), _i(T), _i(E), _i(H), _i(W), _i(C), _i(gauss_radius if use_gauss else 0),
-                _i(precision), _i(1 if round_half else 0), _stream(hi))
-        _lib.check(st, "build_pyramid (slots)")
+    rh = 1 if round_half else 0
+    if out is None:
+        lv = [torch.empty(E, H, W, H >> l, W >> l, dtype=torch.float32, device=hi.device) for l in range(num_levels)]
+        p = lv + [None] * (4 - num_levels)
+        _launch("lgu_build_pyramid", hi.device, hi, lo, ii, jj, means, covs, den, p[0], p[1], p[2], p[3], T, E, H, W, C,
+                gauss_radius, precision, rh)
         return lv
-    lv = [torch.empty(E, H, W, H >> l, W >> l, dtype=torch.float32, device=hi.device) for l in range(num_levels)]
-    ptr = [_p(t) for t in lv] + [null] * (4 - num_levels)
-    with torch.cuda.device(hi.device):
-        st = _lib.lib().lgu_build_pyramid(_p(hi), _p(lo) if precision == 2 else null, _p(ii), _p(jj),
-                                          _p(means) if use_gauss else null, _p(covs) if use_gauss else null,
-                                          _p(den) if (use_gauss and den is not None) else null, ptr[0], ptr[1], ptr[2], ptr[3],
-                                          _i(T), _i(E), _i(H), _i(W), _i(C), _i(gauss_radius if use_gauss else 0),
-                                          _i(precision), _i(1 if round_half else 0), _stream(hi))
-    _lib.check(st, "build_pyramid")
+    _check_index(out_slots, "out_slots", E)
+    S = out[0].shape[0]
+    lv = list(out[:num_levels])
+    _check_levels(lv, S, H, W, "out")
+    p = lv + [None] * (4 - num_levels)
+    _launch("lgu_build_pyramid_slots", hi.device, hi, lo, ii, jj, means, covs, den, p[0], p[1], p[2], p[3], out_slots, S, T,
+            E, H, W, C, gauss_radius, precision, rh)
     return lv
 
 
@@ -357,62 +338,40 @@ def corr_lookup_fused(pyramid, coords, off0, off1, radius=3, return_mask=False, 
     if len(pyramid) != 4:
         raise RuntimeError("corr_lookup_fused needs a 4-level pyramid")
     S, H, W = pyramid[0].shape[:3]                    # S = storage slots (== edges without a pool)
-    for l, t in enumerate(pyramid):
-        _chk(t, f"pyramid[{l}]", 5)
-        if tuple(t.shape) != (S, H, W, H >> l, W >> l):
-            raise RuntimeError(f"pyramid[{l}] shape {tuple(t.shape)} != {(S, H, W, H >> l, W >> l)}")
+    _check_levels(pyramid, S, H, W, "pyramid")
     _chk(coords, "coords", 4)
     E = coords.shape[0] if slots is not None else S
-    if slots is not None and not (slots.is_cuda and slots.dtype == torch.int32 and slots.is_contiguous()
-                                  and slots.numel() == E):
-        raise RuntimeError("slots must be a contiguous CUDA int32 vector with one slot per edge of coords")
+    if slots is not None:
+        _check_index(slots, "slots", E)
     if tuple(coords.shape) != (E, H, W, 2):
         raise RuntimeError(f"coords shape {tuple(coords.shape)} != {(E, H, W, 2)}")
-    rd = 2 * int(radius) + 1
-    for name, o in (("off0", off0), ("off1", off1)):
-        if not (isinstance(o, torch.Tensor) and o.is_cuda and o.is_contiguous() and o.dtype == torch.float32):
-            raise RuntimeError(f"{name} must be a contiguous fp32 CUDA tensor")
-        if o.numel() != S * H * W * rd * rd * 2:
-            raise RuntimeError(f"{name} has {o.numel()} elements, expected {S * H * W * rd * rd * 2}")
+    radius = int(radius)
+    rd = 2 * radius + 1
+    _check_offsets(S * H * W * rd * rd * 2, off0=off0, off1=off1)
     corr = torch.empty(E, 4 * rd * rd, H, W, dtype=torch.float32, device=coords.device)
     mask = torch.empty(E, H, W, dtype=torch.float32, device=coords.device) if return_mask else None
+    p = pyramid
     if cum_mask is not None:
         _chk(cum_mask, "cum_mask", 3)
         if tuple(cum_mask.shape) != (S, H, W):
             raise RuntimeError(f"cum_mask shape {tuple(cum_mask.shape)} != {(S, H, W)}")
-    with torch.cuda.device(coords.device):
-        if cum_mask is not None:
-            st = _lib.lib().lgu_corr_lookup_fused_cum(_p(pyramid[0]), _p(pyramid[1]), _p(pyramid[2]), _p(pyramid[3]),
-                                                      _p(coords), _p(off0), _p(off1), _p(cum_mask), _p(corr),
-                                                      _p(mask) if return_mask else ctypes.c_void_p(0),
-                                                      _p(slots) if slots is not None else ctypes.c_void_p(0),
-                                                      _i(S), _i(E), _i(H), _i(W), _i(4), _i(radius), _stream(coords))
-        elif slots is not None:
-            st = _lib.lib().lgu_corr_lookup_fused_slots(_p(pyramid[0]), _p(pyramid[1]), _p(pyramid[2]), _p(pyramid[3]),
-                                                        _p(coords), _p(off0), _p(off1), _p(corr),
-                                                        _p(mask) if return_mask else ctypes.c_void_p(0), _p(slots),
-                                                        _i(S), _i(E), _i(H), _i(W), _i(4), _i(radius), _stream(coords))
-        else:
-            st = _lib.lib().lgu_corr_lookup_fused(_p(pyramid[0]), _p(pyramid[1]), _p(pyramid[2]), _p(pyramid[3]),
-                                                  _p(coords), _p(off0), _p(off1), _p(corr),
-                                                  _p(mask) if return_mask else ctypes.c_void_p(0),
-                                                  _i(E), _i(H), _i(W), _i(4), _i(radius), _stream(coords))
-    _lib.check(st, "corr_lookup_fused")
+        _launch("lgu_corr_lookup_fused_cum", coords.device, p[0], p[1], p[2], p[3], coords, off0, off1, cum_mask, corr,
+                mask, slots, S, E, H, W, 4, radius)
+    elif slots is not None:
+        _launch("lgu_corr_lookup_fused_slots", coords.device, p[0], p[1], p[2], p[3], coords, off0, off1, corr, mask, slots,
+                S, E, H, W, 4, radius)
+    else:
+        _launch("lgu_corr_lookup_fused", coords.device, p[0], p[1], p[2], p[3], coords, off0, off1, corr, mask, E, H, W, 4,
+                radius)
     return (corr, mask) if return_mask else corr
 
 
 def pack_conv1x1(weight):
     """corr_encoder[0].weight [128,196] (or [128,196,1,1]) -> the tensor-core operand fragments of the fused encoder
     epilogue (TF32 hi/lo split, m16n8k8 A-fragment order): a float32 tensor of 8*25*32*8 elements."""
-    if not (isinstance(weight, torch.Tensor) and weight.is_cuda and weight.dtype == torch.float32):
-        raise RuntimeError("weight must be a CUDA fp32 tensor")
-    w = weight.detach().reshape(weight.shape[0], -1).contiguous()
-    if tuple(w.shape) != (128, 196):
-        raise RuntimeError(f"only the 196 -> 128 corr_encoder is implemented, got weight {tuple(weight.shape)}")
+    w = _encoder_weight(weight)
     frag = torch.empty(8 * 25 * 32 * 8, dtype=torch.float32, device=w.device)
-    with torch.cuda.device(w.device):
-        st = _lib.lib().lgu_pack_conv1x1(_p(w), _p(frag), _i(128), _i(196), _stream(w))
-    _lib.check(st, "pack_conv1x1")
+    _launch("lgu_pack_conv1x1", w.device, w, frag, 128, 196)
     return frag
 
 
@@ -425,18 +384,14 @@ def corr_lookup_fused_enc(pyramid, coords, off0, off1, cum_mask, wfrag, bias=Non
     if len(pyramid) != 4:
         raise RuntimeError("corr_lookup_fused_enc needs a 4-level pyramid")
     S, H, W = pyramid[0].shape[:3]
-    for l, t in enumerate(pyramid):
-        _chk(t, f"pyramid[{l}]", 5)
-        if tuple(t.shape) != (S, H, W, H >> l, W >> l):
-            raise RuntimeError(f"pyramid[{l}] shape {tuple(t.shape)} != {(S, H, W, H >> l, W >> l)}")
+    _check_levels(pyramid, S, H, W, "pyramid")
     _chk(coords, "coords", 4); _chk(cum_mask, "cum_mask", 3)
     E = coords.shape[0] if slots is not None else S
     if tuple(coords.shape) != (E, H, W, 2) or tuple(cum_mask.shape) != (S, H, W):
         raise RuntimeError("corr_lookup_fused_enc: inconsistent coords / cum_mask shapes")
-    for name, o in (("off0", off0), ("off1", off1)):
-        if not (isinstance(o, torch.Tensor) and o.is_cuda and o.is_contiguous() and o.dtype == torch.float32
-                and o.numel() == S * H * W * 98):
-            raise RuntimeError(f"{name} must be a contiguous fp32 CUDA tensor with {S * H * W * 98} elements")
+    if slots is not None:
+        _check_index(slots, "slots", E)
+    _check_offsets(S * H * W * 98, off0=off0, off1=off1)
     if not (wfrag.is_cuda and wfrag.dtype == torch.float32 and wfrag.numel() == 8 * 25 * 32 * 8 and wfrag.is_contiguous()):
         raise RuntimeError("wfrag must come from pack_conv1x1")
     if bias is not None and not (bias.is_cuda and bias.dtype == torch.float32 and bias.numel() == 128 and bias.is_contiguous()):
@@ -445,14 +400,9 @@ def corr_lookup_fused_enc(pyramid, coords, off0, off1, cum_mask, wfrag, bias=Non
         raise RuntimeError("enc_half needs keep_corr=False")
     corr = torch.empty(E, 196, H, W, dtype=torch.float32, device=coords.device) if keep_corr else None
     enc = torch.empty(E, 128, H, W, dtype=torch.float16 if enc_half else torch.float32, device=coords.device)
-    null = ctypes.c_void_p(0)
-    with torch.cuda.device(coords.device):
-        st = _lib.lib().lgu_corr_lookup_fused_enc(
-            _p(pyramid[0]), _p(pyramid[1]), _p(pyramid[2]), _p(pyramid[3]), _p(coords), _p(off0), _p(off1), _p(cum_mask),
-            _p(corr) if keep_corr else null, _p(enc), _p(wfrag), _p(bias) if bias is not None else null,
-            _i(1 if relu else 0), _i(1 if enc_half else 0), null, _p(slots) if slots is not None else null, _i(S), _i(E),
-            _i(H), _i(W), _i(4), _i(3), _stream(coords))
-    _lib.check(st, "corr_lookup_fused_enc")
+    p = pyramid
+    _launch("lgu_corr_lookup_fused_enc", coords.device, p[0], p[1], p[2], p[3], coords, off0, off1, cum_mask, corr, enc,
+            wfrag, bias, 1 if relu else 0, 1 if enc_half else 0, None, slots, S, E, H, W, 4, 3)
     return corr, enc
 
 
@@ -474,82 +424,57 @@ def corr_lookup_fused_backward(pyramid, coords, off0, off1_out, mask, corr_grad,
     build_backward_gauss(means, covs, den, pyramid[0], this call's level gradients, 4)
     (lgu_corr_lookup_fused_backward_gauss)."""
     E, H, W = pyramid[0].shape[:3]
-    for l, t in enumerate(pyramid):
-        _chk(t, f"pyramid[{l}]", 5)
+    _check_levels(pyramid, E, H, W, "pyramid")
     _chk(coords, "coords", 4); _chk(mask, "mask", 3); _chk(corr_grad, "corr_grad", 4)
     if tuple(corr_grad.shape) != (E, 196, H, W) or tuple(mask.shape) != (E, H, W) or tuple(coords.shape) != (E, H, W, 2):
         raise RuntimeError("corr_lookup_fused_backward: inconsistent shapes")
-    for name, o in (("off0", off0), ("off1_out", off1_out), ("off1_out_grad", off1_out_grad)):
-        if o is None and name == "off1_out_grad":
-            continue
-        if not (isinstance(o, torch.Tensor) and o.is_cuda and o.is_contiguous() and o.dtype == torch.float32
-                and o.numel() == E * H * W * 98):
-            raise RuntimeError(f"{name} must be a contiguous fp32 CUDA tensor with {E * H * W * 98} elements")
+    _check_offsets(E * H * W * 98, off0=off0, off1_out=off1_out)
+    if off1_out_grad is not None:
+        _check_offsets(E * H * W * 98, off1_out_grad=off1_out_grad)
     if accumulate_into is not None:
         gv = list(accumulate_into)
-        for l, (a, t) in enumerate(zip(gv, pyramid)):
-            _chk(a, f"accumulate_into[{l}]", 5)
-            if a.shape != t.shape or a.device != t.device:
-                raise RuntimeError(f"accumulate_into[{l}] must match pyramid[{l}]")
-        fn = _lib.lib().lgu_corr_lookup_fused_backward_accumulate
+        _check_levels(gv, E, H, W, "accumulate_into")
+        if any(a.device != t.device for a, t in zip(gv, pyramid)):
+            raise RuntimeError("accumulate_into must be on the pyramid's device")
     else:
         gv = [torch.empty_like(t) for t in pyramid]
-        fn = _lib.lib().lgu_corr_lookup_fused_backward
-    g0 = torch.empty(E, H, W, 98, dtype=torch.float32, device=coords.device)
-    g1 = torch.empty_like(g0)
     if cum_mask is not None:
         _chk(cum_mask, "cum_mask", 3)
         if tuple(cum_mask.shape) != (E, H, W):
             raise RuntimeError("cum_mask must be [E,H,W]")
-        if gauss_head is not None:
-            if accumulate_into is not None or gauss_window_means is not None:
-                raise RuntimeError("corr_lookup_fused_backward: gauss_head needs the dense form (and excludes the window record)")
-            means, covs, den = gauss_head
-            _chk(means, "means", 4); _chk(covs, "covs", 4); _chk(den, "den", 3)
-            if tuple(means.shape) != (E, H, W, 2) or tuple(covs.shape) != (E, H, W, 2) or tuple(den.shape) != (E, H, W):
-                raise RuntimeError("gauss_head must be (means [E,H,W,2], covs [E,H,W,2], den [E,H,W])")
-            gm, gc, gd = torch.empty_like(means), torch.empty_like(covs), torch.empty_like(den)
-            with torch.cuda.device(coords.device):
-                st = _lib.lib().lgu_corr_lookup_fused_backward_gauss(
-                    _p(pyramid[0]), _p(pyramid[1]), _p(coords), _p(off0), _p(off1_out), _p(cum_mask), _p(mask),
-                    _p(corr_grad), _p(off1_out_grad) if off1_out_grad is not None else ctypes.c_void_p(0),
-                    _p(means), _p(covs), _p(den), _p(gv[0]), _p(gv[1]), _p(gv[2]), _p(gv[3]), _p(g0), _p(g1),
-                    _p(gm), _p(gc), _p(gd), _i(E), _i(H), _i(W), _i(4), _i(3), _i(4), _stream(coords))
-            _lib.check(st, "corr_lookup_fused_backward (gauss)")
-            return gv[0], gv[1], gv[2], gv[3], g0, g1, gm, gc, gd
-        if gauss_window_means is not None:
-            if accumulate_into is not None:
-                raise RuntimeError("corr_lookup_fused_backward: the Gaussian window record needs the dense form")
-            _chk(gauss_window_means, "gauss_window_means", 4)
-            if tuple(gauss_window_means.shape) != (E, H, W, 2):
-                raise RuntimeError("gauss_window_means must be [E,H,W,2]")
-            gwin = torch.empty(E, H, W, 81, dtype=torch.float32, device=coords.device)
-            with torch.cuda.device(coords.device):
-                st = _lib.lib().lgu_corr_lookup_fused_backward_win(
-                    _p(pyramid[0]), _p(pyramid[1]), _p(coords), _p(off0), _p(off1_out), _p(cum_mask), _p(mask),
-                    _p(corr_grad), _p(off1_out_grad) if off1_out_grad is not None else ctypes.c_void_p(0),
-                    _p(gauss_window_means), _p(gv[0]), _p(gv[1]), _p(gv[2]), _p(gv[3]), _p(g0), _p(g1), _p(gwin),
-                    _i(E), _i(H), _i(W), _i(4), _i(3), _stream(coords))
-            _lib.check(st, "corr_lookup_fused_backward (window)")
-            return gv[0], gv[1], gv[2], gv[3], g0, g1, gwin
-        with torch.cuda.device(coords.device):
-            st = _lib.lib().lgu_corr_lookup_fused_backward_cum(
-                _p(pyramid[0]), _p(pyramid[1]), _p(coords), _p(off0), _p(off1_out), _p(cum_mask), _p(mask), _p(corr_grad),
-                _p(off1_out_grad) if off1_out_grad is not None else ctypes.c_void_p(0),
-                _p(gv[0]), _p(gv[1]), _p(gv[2]), _p(gv[3]), _p(g0), _p(g1), _i(E), _i(H), _i(W), _i(4), _i(3),
-                _i(1 if accumulate_into is not None else 0), _stream(coords))
-        _lib.check(st, "corr_lookup_fused_backward (cum)")
-        return gv[0], gv[1], gv[2], gv[3], g0, g1
-    if gauss_window_means is not None or gauss_head is not None:
-        raise RuntimeError("corr_lookup_fused_backward: gauss_window_means / gauss_head need cum_mask (the cumulative-mask form)")
-    with torch.cuda.device(coords.device):
-        st = fn(
-            _p(pyramid[0]), _p(pyramid[1]), _p(coords), _p(off0), _p(off1_out), _p(mask), _p(corr_grad),
-            _p(off1_out_grad) if off1_out_grad is not None else ctypes.c_void_p(0),
-            _p(gv[0]), _p(gv[1]), _p(gv[2]), _p(gv[3]), _p(g0), _p(g1), _i(E), _i(H), _i(W), _i(4), _i(3),
-            _stream(coords))
-    _lib.check(st, "corr_lookup_fused_backward")
-    return gv[0], gv[1], gv[2], gv[3], g0, g1
+    if (gauss_window_means is not None or gauss_head is not None) and \
+            (cum_mask is None or accumulate_into is not None or (gauss_window_means is not None and gauss_head is not None)):
+        raise RuntimeError("corr_lookup_fused_backward: gauss_window_means / gauss_head need the dense cumulative-mask form "
+                           "(cum_mask, no accumulate_into) and exclude each other")
+    g0 = torch.empty(E, H, W, 98, dtype=torch.float32, device=coords.device)
+    g1 = torch.empty_like(g0)
+    p0, p1, dev, out = pyramid[0], pyramid[1], coords.device, (gv[0], gv[1], gv[2], gv[3], g0, g1)
+    if gauss_head is not None:
+        means, covs, den = gauss_head
+        _check_means_covs(means, covs, E, H, W)
+        _chk(den, "den", 3)
+        if tuple(den.shape) != (E, H, W):
+            raise RuntimeError("gauss_head must be (means [E,H,W,2], covs [E,H,W,2], den [E,H,W])")
+        gm, gc, gd = torch.empty_like(means), torch.empty_like(covs), torch.empty_like(den)
+        _launch("lgu_corr_lookup_fused_backward_gauss", dev, p0, p1, coords, off0, off1_out, cum_mask, mask, corr_grad,
+                off1_out_grad, means, covs, den, gv[0], gv[1], gv[2], gv[3], g0, g1, gm, gc, gd, E, H, W, 4, 3, 4)
+        return out + (gm, gc, gd)
+    if gauss_window_means is not None:
+        _chk(gauss_window_means, "gauss_window_means", 4)
+        if tuple(gauss_window_means.shape) != (E, H, W, 2):
+            raise RuntimeError("gauss_window_means must be [E,H,W,2]")
+        gwin = torch.empty(E, H, W, 81, dtype=torch.float32, device=coords.device)
+        _launch("lgu_corr_lookup_fused_backward_win", dev, p0, p1, coords, off0, off1_out, cum_mask, mask, corr_grad,
+                off1_out_grad, gauss_window_means, gv[0], gv[1], gv[2], gv[3], g0, g1, gwin, E, H, W, 4, 3)
+        return out + (gwin,)
+    accumulate = accumulate_into is not None
+    if cum_mask is not None:
+        _launch("lgu_corr_lookup_fused_backward_cum", dev, p0, p1, coords, off0, off1_out, cum_mask, mask, corr_grad,
+                off1_out_grad, gv[0], gv[1], gv[2], gv[3], g0, g1, E, H, W, 4, 3, 1 if accumulate else 0)
+    else:
+        _launch("lgu_corr_lookup_fused_backward_accumulate" if accumulate else "lgu_corr_lookup_fused_backward", dev, p0, p1,
+                coords, off0, off1_out, mask, corr_grad, off1_out_grad, gv[0], gv[1], gv[2], gv[3], g0, g1, E, H, W, 4, 3)
+    return out
 
 
 def build_backward_gauss(means, covs, den, lvl0, level_grads, radius, window=None):
@@ -558,36 +483,22 @@ def build_backward_gauss(means, covs, den, lvl0, level_grads, radius, window=Non
     window [E,H,W,81]: the record corr_lookup_fused_backward(gauss_window_means=means) returned -- used INSTEAD of
     level_grads (radius 4; same result bit for bit, one contiguous read per pixel).
     Returns (means_grad, covs_grad, den_grad); see lgu_build_backward_gauss in include/lgu_corr.h."""
-    _chk(means, "means", 4); _chk(covs, "covs", 4); _chk(den, "den", 3); _chk(lvl0, "lvl0", 5)
+    _chk(den, "den", 3); _chk(lvl0, "lvl0", 5)
     E, H, W = lvl0.shape[:3]
-    if tuple(lvl0.shape) != (E, H, W, H, W) or tuple(means.shape) != (E, H, W, 2) or tuple(covs.shape) != (E, H, W, 2) \
-            or tuple(den.shape) != (E, H, W):
+    _check_means_covs(means, covs, E, H, W)
+    if tuple(lvl0.shape) != (E, H, W, H, W) or tuple(den.shape) != (E, H, W):
         raise RuntimeError("build_backward_gauss: inconsistent shapes")
+    gm, gc, gd = torch.empty_like(means), torch.empty_like(covs), torch.empty_like(den)
     if window is not None:
         _chk(window, "window", 4)
         if tuple(window.shape) != (E, H, W, 81) or radius != 4:
             raise RuntimeError("build_backward_gauss: window must be [E,H,W,81] and radius 4")
-        gm, gc, gd = torch.empty_like(means), torch.empty_like(covs), torch.empty_like(den)
-        with torch.cuda.device(lvl0.device):
-            st = _lib.lib().lgu_build_backward_gauss_window(_p(means), _p(covs), _p(den), _p(lvl0), _p(window), _p(gm),
-                                                            _p(gc), _p(gd), _i(E), _i(H), _i(W), _stream(lvl0))
-        _lib.check(st, "build_backward_gauss (window)")
+        _launch("lgu_build_backward_gauss_window", lvl0.device, means, covs, den, lvl0, window, gm, gc, gd, E, H, W)
         return gm, gc, gd
-    ptrs = []
-    for l, g in enumerate(level_grads):
-        if g is None:
-            ptrs.append(ctypes.c_void_p(0))
-            continue
-        _chk(g, f"level_grads[{l}]", 5)
-        if tuple(g.shape) != (E, H, W, H >> l, W >> l):
-            raise RuntimeError(f"level_grads[{l}] must be [E,H,W,{H >> l},{W >> l}]")
-        ptrs.append(_p(g))
-    gm, gc, gd = torch.empty_like(means), torch.empty_like(covs), torch.empty_like(den)
-    with torch.cuda.device(lvl0.device):
-        st = _lib.lib().lgu_build_backward_gauss(_p(means), _p(covs), _p(den), _p(lvl0), ptrs[0], ptrs[1], ptrs[2],
-                                                 ptrs[3], _p(gm), _p(gc), _p(gd), _i(E), _i(H), _i(W), _i(radius),
-                                                 _stream(lvl0))
-    _lib.check(st, "build_backward_gauss")
+    g = list(level_grads)
+    _check_levels(g, E, H, W, "level_grads", skip=[l for l, t in enumerate(g) if t is None])
+    _launch("lgu_build_backward_gauss", lvl0.device, means, covs, den, lvl0, g[0], g[1], g[2], g[3], gm, gc, gd, E, H, W,
+            int(radius))
     return gm, gc, gd
 
 
@@ -597,10 +508,7 @@ def tf32_split(x, scale=1.0):
         raise RuntimeError("tf32_split: fp32 CUDA tensor expected")
     x = x.contiguous()
     hi, lo = torch.empty_like(x), torch.empty_like(x)
-    with torch.cuda.device(x.device):
-        st = _lib.lib().lgu_tf32_split(_p(x), ctypes.c_float(scale), _p(hi), _p(lo), ctypes.c_longlong(x.numel()),
-                                       _stream(x))
-    _lib.check(st, "tf32_split")
+    _launch("lgu_tf32_split", x.device, x, scale, hi, lo, x.numel())
     return hi, lo
 
 
@@ -610,7 +518,10 @@ def build_backward_fmaps(level_grads, f1, f2):
     Returns (g_f1, g_f2) [E,C,H,W] fp32: g_f1 = g_V f2 / 16, g_f2 = g_V^T f1 / 16 with g_V = sum_l avg_pool^T(level_grads[l])."""
     import torch.nn.functional as F
     E, C, H, W = f1.shape
+    if not isinstance(f2, torch.Tensor) or f2.shape != f1.shape or f2.device != f1.device:
+        raise RuntimeError(f"f2 must have f1's shape {tuple(f1.shape)} and device")
     L = len(level_grads)
+    _check_levels(level_grads, E, H, W, "level_grads", skip=[l for l, g in enumerate(level_grads) if g is None])
     f1h, f1l = tf32_split(f1.float().reshape(E, C, H * W), 1.0 / 16.0)
     planes, cur = [], f2.float()
     for l in range(L):
@@ -620,21 +531,9 @@ def build_backward_fmaps(level_grads, f1, f2):
     g_f1 = torch.empty(E, C, H * W, dtype=torch.float32, device=f1.device)
     g_f2l = [torch.empty(E, C, (H >> l) * (W >> l), dtype=torch.float32, device=f1.device) if level_grads[l] is not None
              else None for l in range(L)]
-    arr = ctypes.c_void_p * L
-
-    def ptrs(ts):
-        return arr(*[t.data_ptr() if t is not None else None for t in ts])
-
-    for l, g in enumerate(level_grads):
-        if g is not None:
-            _chk(g, f"level_grads[{l}]", 5)
-            if tuple(g.shape) != (E, H, W, H >> l, W >> l):
-                raise RuntimeError(f"level_grads[{l}] must be [E,H,W,{H >> l},{W >> l}]")
-    with torch.cuda.device(f1.device):
-        st = _lib.lib().lgu_build_backward_fmaps(ptrs(level_grads), _p(f1h), _p(f1l), ptrs([p[0] for p in planes]),
-                                                 ptrs([p[1] for p in planes]), _p(g_f1), ptrs(g_f2l), _i(L), _i(E), _i(H),
-                                                 _i(W), _i(C), _stream(f1))
-    _lib.check(st, "build_backward_fmaps")
+    arr = _lib.pointer_array
+    _launch("lgu_build_backward_fmaps", f1.device, arr(level_grads), f1h, f1l, arr([p[0] for p in planes]),
+            arr([p[1] for p in planes]), g_f1, arr(g_f2l), L, E, H, W, C)
     g_f2 = None
     for l, t in enumerate(g_f2l):
         if t is None:
@@ -653,9 +552,7 @@ def volume_half_mask(coords, level=0):
     _chk(coords, "coords", 4)
     E, H, W, _ = coords.shape
     mask = torch.empty(E * H * W // 128, dtype=torch.int32, device=coords.device)
-    with torch.cuda.device(coords.device):
-        st = _lib.lib().lgu_volume_half_mask(_p(coords), _p(mask), _i(E), _i(H), _i(W), _i(level), _stream(coords))
-    _lib.check(st, "volume_half_mask")
+    _launch("lgu_volume_half_mask", coords.device, coords, mask, E, H, W, int(level))
     return mask
 
 
@@ -666,23 +563,16 @@ def build_boxes(f1_hi, f2_hi, ii, jj, coords, half_mask=None, level=0):
     level = 1: f2_hi holds the level-1 pooled maps [T2,P/4,C]; the result goes to altcorr_lookup_fused(..., boxes1=)."""
     _chk(coords, "coords", 4)
     E, H, W, _ = coords.shape
-    for t, name in ((f1_hi, "f1_hi"), (f2_hi, "f2_hi")):
-        if not (t.is_cuda and t.dtype == torch.float16 and t.dim() == 3 and t.is_contiguous()):
-            raise RuntimeError(f"{name} must be a contiguous CUDA fp16 tensor [T,P,C]")
+    _check_plane(f1_hi, "f1_hi"); _check_plane(f2_hi, "f2_hi")
     T1, P, C = f1_hi.shape
     T2, Q, C2 = f2_hi.shape
     if C2 != C or P != H * W or Q != (H >> level) * (W >> level) or level not in (0, 1):
         raise RuntimeError("build_boxes: f1 [T,H*W,C] and f2 [T,(H>>level)*(W>>level),C] expected, level 0 or 1")
-    for t, name in ((ii, "ii"), (jj, "jj")):
-        if not (t.is_cuda and t.dtype == torch.int32 and t.dim() == 1 and t.is_contiguous() and t.numel() == E):
-            raise RuntimeError(f"{name} must be a contiguous CUDA int32 vector with one entry per edge")
+    _check_index(ii, "ii", E); _check_index(jj, "jj", E)
     if half_mask is None:
         half_mask = volume_half_mask(coords, level)
     boxes = torch.empty(E, P, 16, 20, dtype=torch.float32, device=coords.device)
-    with torch.cuda.device(coords.device):
-        st = _lib.lib().lgu_build_boxes(_p(f1_hi), _p(f2_hi), _p(ii), _p(jj), _p(coords), _p(half_mask), _p(boxes), _i(T1),
-                                        _i(T2), _i(E), _i(H), _i(W), _i(C), _i(level), _stream(coords))
-    _lib.check(st, "build_boxes")
+    _launch("lgu_build_boxes", coords.device, f1_hi, f2_hi, ii, jj, coords, half_mask, boxes, T1, T2, E, H, W, C, level)
     return boxes
 
 
@@ -692,43 +582,38 @@ def build_volume(f1_hi, f1_lo, f2_hi, f2_lo, ii, jj, half_mask=None):
     Returns [E,P,Q] fp32.  The backend path's per-level volume (source level 0 x pooled target level l).
     half_mask (volume_half_mask): sparse form -- only the named halves are computed; the rest of the result is
     UNINITIALISED memory that the fused backend lookup at those coords never reads."""
-    for t, name in ((f1_hi, "f1_hi"), (f2_hi, "f2_hi")):
-        if not (t.is_cuda and t.dtype == torch.float16 and t.dim() == 3 and t.is_contiguous()):
-            raise RuntimeError(f"{name} must be a contiguous CUDA fp16 tensor [T,P,C]")
+    _check_plane(f1_hi, "f1_hi"); _check_plane(f2_hi, "f2_hi")
     split = f1_lo is not None
-    if split and (f2_lo is None or f1_lo.shape != f1_hi.shape or f2_lo.shape != f2_hi.shape):
-        raise RuntimeError("precision 2 needs lo planes for both map sets")
+    if split:
+        _check_plane(f1_lo, "f1_lo"); _check_plane(f2_lo, "f2_lo")
+        if f1_lo.shape != f1_hi.shape or f2_lo.shape != f2_hi.shape:
+            raise RuntimeError("precision 2 needs lo planes for both map sets")
+    else:
+        f2_lo = None
     T1, P, C = f1_hi.shape
     T2, Q, C2 = f2_hi.shape
     if C2 != C:
         raise RuntimeError("channel mismatch")
-    for t, name in ((ii, "ii"), (jj, "jj")):
-        if not (t.is_cuda and t.dtype == torch.int32 and t.dim() == 1 and t.is_contiguous()):
-            raise RuntimeError(f"{name} must be a contiguous CUDA int32 vector")
+    _check_index(ii, "ii")
     E = ii.numel()
+    _check_index(jj, "jj", E)
     vol = torch.empty(E, P, Q, dtype=torch.float32, device=f1_hi.device)
-    null = ctypes.c_void_p(0)
-    if half_mask is not None:
-        if not (half_mask.is_cuda and half_mask.dtype == torch.int32 and half_mask.is_contiguous()
-                and half_mask.numel() == E * (P // 128)):
-            raise RuntimeError(f"half_mask must be a contiguous CUDA int32 vector of {E * (P // 128)} words")
-        with torch.cuda.device(f1_hi.device):
-            st = _lib.lib().lgu_build_volume_sparse(_p(f1_hi), _p(f1_lo) if split else null, _p(f2_hi),
-                                                    _p(f2_lo) if split else null, _p(ii), _p(jj), _p(half_mask), _p(vol),
-                                                    _i(T1), _i(T2), _i(E), _i(P), _i(Q), _i(C), _i(2 if split else 1),
-                                                    _stream(f1_hi))
-        _lib.check(st, "build_volume (sparse)")
-        return vol
-    with torch.cuda.device(f1_hi.device):
-        st = _lib.lib().lgu_build_volume(_p(f1_hi), _p(f1_lo) if split else null, _p(f2_hi), _p(f2_lo) if split else null,
-                                         _p(ii), _p(jj), _p(vol), _i(T1), _i(T2), _i(E), _i(P), _i(Q), _i(C),
-                                         _i(2 if split else 1), _stream(f1_hi))
-    _lib.check(st, "build_volume")
+    if half_mask is None:
+        _launch("lgu_build_volume", f1_hi.device, f1_hi, f1_lo, f2_hi, f2_lo, ii, jj, vol, T1, T2, E, P, Q, C,
+                2 if split else 1)
+    else:
+        _check_index(half_mask, "half_mask", E * (P // 128))
+        _launch("lgu_build_volume_sparse", f1_hi.device, f1_hi, f1_lo, f2_hi, f2_lo, ii, jj, half_mask, vol, T1, T2, E, P,
+                Q, C, 2 if split else 1)
     return vol
 
 
-def _check_altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1):
-    """Shapes / dtypes / layout of the backend lookup's inputs; returns (E, H, W)."""
+def _altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1, out, out_index, C, out_dtype,
+                    return_mask):
+    """Input handling of the backend lookups: checks shapes / dtypes / layout, allocates out [E,C,H,W] (out_dtype) and
+    drops out_index when no destination is given, else checks the caller's rows [E_out,C,H,W] (fp32 / fp16) and their
+    optional int32 row index (one row per edge).  Returns (E, H, W, levels, out, out_index, mask); levels[l] is
+    volumes[l], or None where boxes replace it."""
     E, H, W = volumes[2].shape[:3]
     if boxes1 is not None and boxes0 is None:
         raise RuntimeError("boxes1 needs boxes0")
@@ -737,32 +622,24 @@ def _check_altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, b
             _chk(bx, name, 4)
             if tuple(bx.shape) != (E, H * W, 16, 20):
                 raise RuntimeError(f"{name} must be [E,H*W,16,20], got {tuple(bx.shape)}")
-    for l, t in enumerate(volumes):
-        if (l == 0 and boxes0 is not None) or (l == 1 and boxes1 is not None):
-            continue
-        _chk(t, f"volumes[{l}]", 5)
-        if tuple(t.shape) != (E, H, W, H >> l, W >> l):
-            raise RuntimeError(f"volumes[{l}] shape {tuple(t.shape)} != {(E, H, W, H >> l, W >> l)}")
+    boxed = [l for l, bx in enumerate((boxes0, boxes1)) if bx is not None]
+    _check_levels(volumes, E, H, W, "volumes", skip=boxed)
     _chk(coords, "coords", 4)
-    need = H * W * 98 * (1 if shared_offsets else E)
-    for name, o in (("off0", off0), ("off1", off1)):
-        if not (isinstance(o, torch.Tensor) and o.is_cuda and o.is_contiguous() and o.dtype == torch.float32
-                and o.numel() >= need):
-            raise RuntimeError(f"{name} must be a contiguous fp32 CUDA tensor with >= {need} elements")
-    return E, H, W
-
-
-def _check_out_rows(out, out_index, E, C, H, W, device):
-    """A caller-owned destination [E_out,C,H,W] (fp32 / fp16) and its optional int32 row index, one row per edge."""
-    if not (isinstance(out, torch.Tensor) and out.is_cuda and out.is_contiguous() and out.dim() == 4
-            and tuple(out.shape[1:]) == (C, H, W) and out.dtype in (torch.float32, torch.float16)):
-        raise RuntimeError(f"out must be a contiguous CUDA tensor [E_out,{C},H,W], fp32 or fp16")
-    if out_index is not None:
-        if not (out_index.is_cuda and out_index.dtype == torch.int32 and out_index.is_contiguous()
-                and out_index.numel() == E and out_index.device == device):
-            raise RuntimeError("out_index must be a contiguous CUDA int32 vector with one row per edge")
-    elif out.shape[0] < E:
-        raise RuntimeError(f"out has {out.shape[0]} rows, {E} edges")
+    _check_offsets(H * W * 98 * (1 if shared_offsets else E), exact=False, off0=off0, off1=off1)
+    if out is None:
+        out, out_index = torch.empty(E, C, H, W, dtype=out_dtype, device=coords.device), None
+    else:
+        if not (isinstance(out, torch.Tensor) and out.is_cuda and out.is_contiguous() and out.dim() == 4
+                and tuple(out.shape[1:]) == (C, H, W) and out.dtype in (torch.float32, torch.float16)):
+            raise RuntimeError(f"out must be a contiguous CUDA tensor [E_out,{C},H,W], fp32 or fp16")
+        if out_index is not None:
+            _check_index(out_index, "out_index", E)
+            if out_index.device != coords.device:
+                raise RuntimeError("out_index must be on the coords' device")
+        elif out.shape[0] < E:
+            raise RuntimeError(f"out has {out.shape[0]} rows, {E} edges")
+    mask = torch.empty(E, H, W, dtype=torch.float32, device=coords.device) if return_mask else None
+    return E, H, W, [None if l in boxed else volumes[l] for l in range(4)], out, out_index, mask
 
 
 def altcorr_lookup_fused(volumes, coords, off0, off1, radius=3, shared_offsets=False, apply_mask=True,
@@ -774,44 +651,16 @@ def altcorr_lookup_fused(volumes, coords, off0, off1, radius=3, shared_offsets=F
     into this process; out_index int32 [E]: row of `out` that receives edge e (default: e).  Returns `out` then.
     boxes0 [E,H*W,16,20] (build_boxes): level 0 as compact per-pixel boxes; volumes[0] is then ignored (may be None);
     boxes1: the same for level 1 (needs boxes0)."""
-    E, H, W = _check_altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1)
-    mask = torch.empty(E, H, W, dtype=torch.float32, device=coords.device) if return_mask else None
-    if out is not None:
-        _check_out_rows(out, out_index, E, 196, H, W, coords.device)
-        null = ctypes.c_void_p(0)
-        if boxes0 is not None:
-            head = (_p(boxes0), _p(boxes1) if boxes1 is not None else null, _p(volumes[1]) if boxes1 is None else null)
-            fn = _lib.lib().lgu_altcorr_lookup_boxes_into
-        else:
-            head = (_p(volumes[0]), _p(volumes[1]))
-            fn = _lib.lib().lgu_altcorr_lookup_fused_into
-        with torch.cuda.device(coords.device):
-            st = fn(
-                *head, _p(volumes[2]), _p(volumes[3]), _p(coords), _p(off0), _p(off1), _p(out),
-                _p(out_index) if out_index is not None else ctypes.c_void_p(0), _i(out.dtype == torch.float16),
-                _p(mask) if return_mask else ctypes.c_void_p(0), _i(E), _i(H), _i(W), _i(4), _i(radius),
-                _i(1 if shared_offsets else 0), _i(1 if apply_mask else 0), _stream(coords))
-        _lib.check(st, "altcorr_lookup_fused (into)")
-        return (out, mask) if return_mask else out
-    corr = torch.empty(E, 196, H, W, dtype=torch.float32, device=coords.device)
+    E, H, W, lv, out, out_index, mask = _altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1, out,
+                                                        out_index, 196, torch.float32, return_mask)
+    half, so, am = out.dtype == torch.float16, 1 if shared_offsets else 0, 1 if apply_mask else 0
     if boxes0 is not None:
-        with torch.cuda.device(coords.device):
-            null = ctypes.c_void_p(0)
-            st = _lib.lib().lgu_altcorr_lookup_boxes_into(
-                _p(boxes0), _p(boxes1) if boxes1 is not None else null, _p(volumes[1]) if boxes1 is None else null,
-                _p(volumes[2]), _p(volumes[3]), _p(coords), _p(off0), _p(off1), _p(corr),
-                ctypes.c_void_p(0), _i(0), _p(mask) if return_mask else ctypes.c_void_p(0), _i(E), _i(H), _i(W), _i(4),
-                _i(radius), _i(1 if shared_offsets else 0), _i(1 if apply_mask else 0), _stream(coords))
-        _lib.check(st, "altcorr_lookup_fused (boxes)")
-        return (corr, mask) if return_mask else corr
-    with torch.cuda.device(coords.device):
-        st = _lib.lib().lgu_altcorr_lookup_fused(_p(volumes[0]), _p(volumes[1]), _p(volumes[2]), _p(volumes[3]),
-                                                 _p(coords), _p(off0), _p(off1), _p(corr),
-                                                 _p(mask) if return_mask else ctypes.c_void_p(0), _i(E), _i(H), _i(W),
-                                                 _i(4), _i(radius), _i(1 if shared_offsets else 0),
-                                                 _i(1 if apply_mask else 0), _stream(coords))
-    _lib.check(st, "altcorr_lookup_fused")
-    return (corr, mask) if return_mask else corr
+        _launch("lgu_altcorr_lookup_boxes_into", coords.device, boxes0, boxes1, lv[1], lv[2], lv[3], coords, off0, off1,
+                out, out_index, half, mask, E, H, W, 4, int(radius), so, am)
+    else:
+        _launch("lgu_altcorr_lookup_fused_into", coords.device, lv[0], lv[1], lv[2], lv[3], coords, off0, off1, out,
+                out_index, half, mask, E, H, W, 4, int(radius), so, am)
+    return (out, mask) if return_mask else out
 
 
 CONV1X1_F16_BYTES = 53760            # LGU_CONV1X1_F16_BYTES
@@ -821,21 +670,14 @@ def pack_conv1x1_f16(weight, bias=None):
     """corr_encoder[0] weight [128,196] (or [128,196,1,1]) and bias [128] (or None) -> the fp16 operands of the backend
     lookup's encoder epilogue (altcorr_lookup_encoded): both rounded to fp16 as autocast does, weight in m16n8k16
     A-fragment order.  A uint8 CUDA tensor of CONV1X1_F16_BYTES bytes."""
-    if not (isinstance(weight, torch.Tensor) and weight.is_cuda and weight.dtype == torch.float32):
-        raise RuntimeError("weight must be a CUDA fp32 tensor")
-    w = weight.detach().reshape(weight.shape[0], -1).contiguous()
-    if tuple(w.shape) != (128, 196):
-        raise RuntimeError(f"only the 196 -> 128 corr_encoder is implemented, got weight {tuple(weight.shape)}")
+    w = _encoder_weight(weight)
     if bias is not None:
         if not (isinstance(bias, torch.Tensor) and bias.is_cuda and bias.dtype == torch.float32 and bias.numel() == 128
                 and bias.device == w.device):
             raise RuntimeError("bias must be a CUDA fp32 vector of 128 on the weight's device")
         bias = bias.detach().contiguous()
     packed = torch.empty(CONV1X1_F16_BYTES, dtype=torch.uint8, device=w.device)
-    with torch.cuda.device(w.device):
-        st = _lib.lib().lgu_pack_conv1x1_f16(_p(w), _p(bias) if bias is not None else ctypes.c_void_p(0), _p(packed),
-                                             _i(128), _i(196), _stream(w))
-    _lib.check(st, "pack_conv1x1_f16")
+    _launch("lgu_pack_conv1x1_f16", w.device, w, bias, packed, 128, 196)
     return packed
 
 
@@ -846,29 +688,16 @@ def altcorr_lookup_encoded(volumes, coords, off0, off1, radius=3, shared_offsets
     only the 128-channel result leaves the SM.  packed: from pack_conv1x1_f16.  Same inputs, side effects and row
     placement as altcorr_lookup_fused; out: [E_out,128,H,W] fp16 or fp32.  Without out, returns a new
     [E,128,H,W] fp16 tensor."""
-    E, H, W = _check_altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1)
+    E, H, W, lv, out, out_index, mask = _altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1, out,
+                                                        out_index, 128, torch.float16, return_mask)
     if not (isinstance(packed, torch.Tensor) and packed.is_cuda and packed.dtype == torch.uint8 and packed.is_contiguous()
             and packed.numel() == CONV1X1_F16_BYTES and packed.device == coords.device):
         raise RuntimeError("packed must come from pack_conv1x1_f16 (on the coords' device)")
     if packed.data_ptr() % 16:
         raise RuntimeError("packed must be 16-byte aligned")
-    if out is None:
-        out = torch.empty(E, 128, H, W, dtype=torch.float16, device=coords.device)
-        out_index = None
-    else:
-        _check_out_rows(out, out_index, E, 128, H, W, coords.device)
     if out.data_ptr() % 8:
         raise RuntimeError("out must be 8-byte aligned")
-    mask = torch.empty(E, H, W, dtype=torch.float32, device=coords.device) if return_mask else None
-    null = ctypes.c_void_p(0)
-    vol = lambda l: null if volumes[l] is None or (l == 0 and boxes0 is not None) or (l == 1 and boxes1 is not None) \
-        else _p(volumes[l])
-    with torch.cuda.device(coords.device):
-        st = _lib.lib().lgu_altcorr_lookup_enc_into(
-            _p(boxes0) if boxes0 is not None else null, _p(boxes1) if boxes1 is not None else null, vol(0), vol(1), vol(2),
-            vol(3), _p(coords), _p(off0), _p(off1), _p(packed), _p(out),
-            _p(out_index) if out_index is not None else null, _i(out.dtype == torch.float16),
-            _p(mask) if return_mask else null, _i(E), _i(H), _i(W), _i(4), _i(radius), _i(1 if shared_offsets else 0),
-            _i(1 if apply_mask else 0), _stream(coords))
-    _lib.check(st, "altcorr_lookup_encoded")
+    _launch("lgu_altcorr_lookup_enc_into", coords.device, boxes0, boxes1, lv[0], lv[1], lv[2], lv[3], coords, off0, off1,
+            packed, out, out_index, out.dtype == torch.float16, mask, E, H, W, 4, int(radius), 1 if shared_offsets else 0,
+            1 if apply_mask else 0)
     return (out, mask) if return_mask else out

@@ -21,6 +21,7 @@ Collectives (only these; the lookups themselves exchange nothing):
 Everything here is host logic on top of `torch.distributed`; the `compute` callable is the AltCorrBlock of
 lgu-slam_b200/corr.py on a GPU box and may be any function with the same signature in CPU (gloo) tests.
 """
+import ctypes
 from dataclasses import dataclass, field
 from typing import Callable, List, Optional
 
@@ -198,25 +199,20 @@ class PeerOutput:
         if self.world > 1:
             dist.barrier(group=group)                       # the zero-fill on `dst` precedes every remote store
 
-    # ---- raw device memory through the C ABI (lgu_peer_*): a plain cudaMalloc allocation + its CUDA IPC handle
+    # ---- raw device memory through the C ABI (lgu_peer_*): a plain cudaMalloc allocation + its CUDA IPC handle.  The
+    # package is imported here, not at the top: the CPU tests load this module on its own.
     @staticmethod
-    def _lib():
-        import ctypes
+    def _native_alloc(nbytes):
         from . import _lib
-        return _lib, ctypes
-
-    @classmethod
-    def _native_alloc(cls, nbytes):
-        _lib, ctypes = cls._lib()
         ptr, handle = ctypes.c_void_p(0), ctypes.create_string_buffer(64)
-        _lib.check(_lib.lib().lgu_peer_alloc(ctypes.c_longlong(nbytes), ctypes.byref(ptr), handle), "peer_alloc")
+        _lib.call("lgu_peer_alloc", nbytes, ctypes.byref(ptr), handle)
         return ptr.value, handle.raw
 
-    @classmethod
-    def _native_open(cls, handle):
-        _lib, ctypes = cls._lib()
+    @staticmethod
+    def _native_open(handle):
+        from . import _lib
         ptr = ctypes.c_void_p(0)
-        _lib.check(_lib.lib().lgu_peer_open(ctypes.create_string_buffer(handle, 64), ctypes.byref(ptr)), "peer_open")
+        _lib.call("lgu_peer_open", ctypes.create_string_buffer(handle, 64), ctypes.byref(ptr))
         return ptr.value
 
     @staticmethod
@@ -233,23 +229,27 @@ class PeerOutput:
         return self.buffer[None] if self.rank == self.dst else None
 
     def close(self):
+        """Collective.  A failed unmap or free raises LguError; a failed unmap raises only after the barrier that orders
+        the unmaps before the free, so no other rank is left waiting in it."""
         if self.world > 1:
             dist.barrier(group=self.group)
         ptr = getattr(self, "_ptr", None)
-        self.buffer = None
-        if self.device.type == "cuda" and ptr is not None:
-            _lib, ctypes = self._lib()
+        native = self.device.type == "cuda" and ptr is not None
+        if native:
+            from . import _lib
+        self.buffer, self._ptr = None, None
+        try:
+            if native:
+                with torch.cuda.device(self.device):
+                    torch.cuda.synchronize(self.device)
+                    if self._opened:
+                        _lib.call("lgu_peer_close", ptr)   # drop the mapping before the owner frees the memory
+        finally:
+            if self.world > 1:
+                dist.barrier(group=self.group)
+        if native and not self._opened:
             with torch.cuda.device(self.device):
-                torch.cuda.synchronize(self.device)
-                if self._opened:
-                    _lib.lib().lgu_peer_close(ctypes.c_void_p(ptr))   # drop the mapping before the owner frees the memory
-            self._ptr = None
-        if self.world > 1:
-            dist.barrier(group=self.group)
-        if self.device.type == "cuda" and ptr is not None and not self._opened:
-            _lib, ctypes = self._lib()
-            with torch.cuda.device(self.device):
-                _lib.lib().lgu_peer_free(ctypes.c_void_p(ptr))
+                _lib.call("lgu_peer_free", ptr)
         self._own = None
         if self._path is not None:
             import os

@@ -401,3 +401,25 @@ def test_fused_lookup_with_corr_encoder_epilogue(ops, keep_corr, half):
         assert err <= 2.0 ** -10 * scale, f"fp16 enc: {err} (scale {scale})"
     else:
         assert err <= 1e-5 * scale, f"enc: {err} (scale {scale})"
+
+
+def test_backward_entry_points_refuse_mismatched_shapes_before_any_launch(ops):
+    """The kernels size their reads and writes from pyramid[0]'s [E,H,W] and from f1: corr_lookup_fused_backward must
+    refuse a pyramid level that is not [E,H,W,H>>l,W>>l] and build_backward_fmaps an f2 that is not f1's shape, with
+    nothing launched.  The tensors are oversized, so a launch that went ahead would stay inside them."""
+    import lgu_slam_b200
+    E, H, W, dev = 1, 16, 32, "cuda"
+    pyr = [torch.zeros(E, H, W, H >> l, W >> l, device=dev) for l in range(4)]
+    coords = torch.zeros(E, H, W, 2, device=dev)
+    off0, off1 = torch.zeros(E, H, W, 98, device=dev), torch.zeros(E, H, W, 98, device=dev)
+    mask, g_corr = torch.ones(E, H, W, device=dev), torch.zeros(E, 196, H, W, device=dev)
+    f1 = torch.zeros(E, 128, H, W, device=dev)
+    launches = lgu_slam_b200._lib.LAUNCHES
+    for l, shape in ((1, (E, H, W, H // 2 + 1, W // 2)), (0, (E, H, W, H + 1, W))):
+        bad = list(pyr)
+        bad[l] = torch.zeros(shape, device=dev)
+        with pytest.raises(RuntimeError, match=rf"pyramid\[{l}\]"):
+            ops.corr_lookup_fused_backward(bad, coords, off0, off1, mask, g_corr)
+    with pytest.raises(RuntimeError, match="f2"):
+        ops.build_backward_fmaps([torch.zeros_like(p) for p in pyr], f1, torch.zeros(E, 128, H + 2, W, device=dev))
+    assert lgu_slam_b200._lib.LAUNCHES == launches
