@@ -418,7 +418,8 @@ LGU_API int lgu_pack_fmaps(const void* fmaps, int src_is_half, void* hi, void* l
  * c0 [E,CH,H,W] = ofsMap(t), c1 [E,CH,H/2,W/2] = ofs_residual(avg_pool2d(t, 2)) (the conv outputs; the nearest-neighbour
  * upsampling of c1 is done by indexing, its statistics equal the low-resolution ones), mean/var per edge over
  * (CH,H,W), biased variance, eps = 1e-5.  off0, off1 [E,H,W,CH]: the channels-last layout the lookups read.
- * stats [E,4] fp32 receives (mean0, rstd0, mean1, rstd1).  Forward only (inference paths); CH <= 128, W % 32 == 0, H even.
+ * stats [E,4] fp32 receives (mean0, sigma0, mean1, sigma1), sigma = sqrt(var + eps) -- the divisor itself, not a
+ * reciprocal; lgu_offset_heads_backward (lgu_corr_ext.h) takes it as it is.  CH <= 128, W % 32 == 0, H even.
  * ------------------------------------------------------------------------ */
 LGU_API int lgu_offset_heads(const float* c0, const float* c1, float* off0, float* off1, float* stats,
                      int E, int CH, int H, int W, float eps, void* stream);

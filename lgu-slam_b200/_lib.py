@@ -88,7 +88,13 @@ SIGNATURES = (
     ("lgu_peer_close", _P),
     ("lgu_peer_free", _P),
 )
-_RETURNS_STATUS = {name for name, _, *ret in SIGNATURES if not ret}
+# The same for include/lgu_corr_ext.h, the entry points added after the version-1 set of lgu_corr.h (which SIGNATURES
+# mirrors as released); tests/test_binding_ext_cpu.py keeps this table and that header in step.  Called via call_ext.
+EXT_SIGNATURES = (
+    ("lgu_offset_heads_backward", _P * 8 + _I * 4 + _P),
+)
+_RETURNS_STATUS = {name for name, _, *ret in SIGNATURES + EXT_SIGNATURES if not ret}
+_EXT_NAMES = {name for name, *_ in EXT_SIGNATURES}
 
 
 def build(verbose=False):
@@ -112,7 +118,7 @@ def lib():
                 "Run `python -c 'import __graft_entry__ as g; g.build()'` (or `make -C lgu-slam_b200/csrc`). "
                 "There is no CPU fallback.")
         L = ctypes.CDLL(LIB_PATH)
-        for name, argtypes, *ret in SIGNATURES:
+        for name, argtypes, *ret in SIGNATURES + EXT_SIGNATURES:
             fn = getattr(L, name)
             fn.argtypes = argtypes
             fn.restype = ret[0] if ret else ctypes.c_int
@@ -149,3 +155,10 @@ def call(name, *args):
     if name in _RETURNS_STATUS:
         check(res, name)
     return res
+
+
+def call_ext(name, *args):
+    """`call` for an entry point of include/lgu_corr_ext.h (EXT_SIGNATURES); any other name raises KeyError."""
+    if name not in _EXT_NAMES:
+        raise KeyError(f"{name} is not an entry point of lgu_corr_ext.h")
+    return call(name, *args)

@@ -237,6 +237,29 @@ class FusedBuild(torch.autograd.Function):
         return (g_f1.to(f1.dtype), g_f2.view_as(f2).to(f2.dtype), g_mean, g_cov, g_det, None, None)
 
 
+class OffsetHeads(torch.autograd.Function):
+    """The offset heads' glue (corr.py:117-135, per_Corr_Normalization :44-51) as ONE differentiable op: forward = the two
+    lgu_offset_heads launches (c0 = ofsMap(t) [E,CH,H,W], c1 = ofs_residual(avg_pool2d(t)) [E,CH,H/2,W/2] -> contiguous
+    off0, off1 [E,H,W,CH], bit-identical to the inference path), backward = one lgu_offset_heads_backward call.  A missing
+    output gradient reaches the kernel as NULL (a zero gradient) instead of a materialised zero tensor."""
+
+    @staticmethod
+    def forward(ctx, c0, c1):
+        c0, c1 = c0.contiguous(), c1.contiguous()
+        off0, off1, stats = ops.offset_heads(c0, c1, return_stats=True)
+        ctx.save_for_backward(c0, c1, stats)
+        ctx.set_materialize_grads(False)
+        return off0, off1
+
+    @staticmethod
+    def backward(ctx, g_off0, g_off1):
+        if g_off0 is None and g_off1 is None:
+            return None, None
+        c0, c1, stats = ctx.saved_tensors
+        return ops.offset_heads_backward(c0, c1, stats, None if g_off0 is None else g_off0.contiguous(),
+                                         None if g_off1 is None else g_off1.contiguous())
+
+
 def per_Corr_Normalization(x, normalIndex, eps=1e-5):
     """corr.py:44-51 / gaussianMask_cuda.py:26-33: standardise over `normalIndex` (biased variance + eps)."""
     mean = torch.mean(x, dim=normalIndex, keepdim=True)
@@ -288,17 +311,24 @@ class GaussianMask(nn.Module):
 # ------------------------------------------------------------------------------------------------
 # offsets (corr.py:117-135 / 217-235)
 # ------------------------------------------------------------------------------------------------
-def _generate_offsets(ofsMap, ofs_residual, t):
-    """t [E,256,h,w] -> 4 per-level offset tensors [E,h,w,98]; levels 2 and 3 are zeros."""
+def _generate_offsets(ofsMap, ofs_residual, t, fused_lookup=False):
+    """t [E,256,h,w] -> 4 per-level offset tensors [E,h,w,98]; levels 2 and 3 are zeros.  fused_lookup: the caller's
+    lookups take the fused path (CorrBlock._fused_lookup_shape), which never writes the records' centre taps."""
     _, _, h, w = t.shape
     o0 = ofsMap(t)
     r1 = ofs_residual(F.avg_pool2d(t, kernel_size=2, stride=2))
-    if (not torch.is_grad_enabled() or not (o0.requires_grad or r1.requires_grad)) and o0.is_cuda and w % 32 == 0 \
-            and h % 2 == 0 and o0.shape[1] <= 128 and o0.dtype == torch.float32:
+    kernel = o0.is_cuda and w % 32 == 0 and h % 2 == 0 and o0.shape[1] <= 128 and o0.dtype == torch.float32
+    if kernel and (not torch.is_grad_enabled() or not (o0.requires_grad or r1.requires_grad)):
         # inference: normalise -> 4 tanh -> level-1 average -> upsample -> NHWC in two launches (lgu_offset_heads) instead of
         # ~14 torch kernels; the records come out contiguous [E,h,w,98] (the reference holds permuted views here, so its
         # stored centre taps survive the first per-operator call; they are read as 0 either way, quirk Q5)
         off0, off1 = ops.offset_heads(o0.detach().contiguous(), r1.detach().contiguous())
+        return [off0, off1, torch.zeros_like(off0), torch.zeros_like(off0)]
+    if kernel and fused_lookup:
+        # training with fused lookups: the same two launches, differentiable (OffsetHeads).  Contiguous records are safe
+        # here because the fused lookup reads the centre tap as 0 and never zeroes it in memory (quirk Q5); the
+        # per-operator sampler does zero it in place, so every other caller keeps the permuted views below
+        off0, off1 = OffsetHeads.apply(o0, r1)
         return [off0, off1, torch.zeros_like(off0), torch.zeros_like(off0)]
     o1 = F.interpolate(r1, (h, w))
     o0 = torch.tanh(per_Corr_Normalization(o0, [1, 2, 3])) * 4
@@ -414,7 +444,7 @@ class CorrBlock:
             autocast_rounding = False
 
         t = torch.cat((fmap1.reshape(E, c, h, w), fmap2.reshape(E, c, h, w)), dim=1)
-        self.offset = _Offsets(_generate_offsets(ofsMap, ofs_residual, t.float()))
+        self.offset = _Offsets(_generate_offsets(ofsMap, ofs_residual, t.float(), self._fused_lookup_shape(h, w)))
         self.t = t.permute(0, 2, 3, 1).contiguous()
 
         if fused:
@@ -437,10 +467,13 @@ class CorrBlock:
         self.mean_n = mean.view(b, n, h, w, 2)
         self.theta = 2 * det.view(b, n, h, w)
 
+    def _fused_lookup_shape(self, ht, wd):
+        """The grids and settings the fused lookup covers (lgu_corr_lookup_fused)."""
+        return self.fused_lookup and self.num_levels == 4 and self.radius == 3 and wd % 32 == 0 and ht % 8 == 0
+
     def _can_fuse_lookup(self, coords):
         ht, wd = coords.shape[2:4]
-        return (self.fused_lookup and self.num_levels == 4 and self.radius == 3 and wd % 32 == 0 and ht % 8 == 0
-                and all(t.dtype == torch.float32 for t in self.corr_pyramid))
+        return self._fused_lookup_shape(ht, wd) and all(t.dtype == torch.float32 for t in self.corr_pyramid)
 
     def _needs_grad(self, coords):
         return torch.is_grad_enabled() and any(t.requires_grad for t in self.corr_pyramid + [

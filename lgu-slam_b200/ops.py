@@ -31,6 +31,12 @@ def _launch(name, device, *args):
         return _lib.call(name, *args, torch.cuda.current_stream(device).cuda_stream)
 
 
+def _launch_ext(name, device, *args):
+    """_launch for an entry point of include/lgu_corr_ext.h (the additions to the version-1 C ABI)."""
+    with torch.cuda.device(device):
+        return _lib.call_ext(name, *args, torch.cuda.current_stream(device).cuda_stream)
+
+
 def _check_levels(levels, S, H, W, name, skip=()):
     """Pyramid levels [S,H,W,H>>l,W>>l] (fp32, contiguous, CUDA); the levels listed in `skip` are not read."""
     for l, t in enumerate(levels):
@@ -246,20 +252,43 @@ def altcorr_forward(fmap1, fmap2, coords, radius, tensor_cores=True):
 # ----------------------------------------------------------------------------------------------
 # Fused ops (no single reference operator; they replace sequences of the reference's Python glue)
 # ----------------------------------------------------------------------------------------------
-def offset_heads(c0, c1, eps=1e-5):
-    """The offset heads' glue (corr.py:117-135 / 217-235) in two launches: c0 [E,CH,H,W] = ofsMap(t), c1 [E,CH,H/2,W/2] =
-    ofs_residual(avg_pool2d(t, 2)) -> (off0, off1) [E,H,W,CH], channels-last and contiguous:
-    off0 = 4 tanh(norm(c0)), off1 = (4 tanh(norm(upsample(c1))) + off0) / 2, norm = per-edge standardisation over
-    (CH,H,W) with biased variance + eps (per_Corr_Normalization, corr.py:44-51).  Forward only."""
+def _check_heads_inputs(c0, c1):
     _chk(c0, "c0", 4); _chk(c1, "c1", 4)
     E, CH, H, W = c0.shape
     if tuple(c1.shape) != (E, CH, H // 2, W // 2):
         raise RuntimeError(f"c1 shape {tuple(c1.shape)} != {(E, CH, H // 2, W // 2)}")
+    return E, CH, H, W
+
+
+def offset_heads(c0, c1, eps=1e-5, return_stats=False):
+    """The offset heads' glue (corr.py:117-135 / 217-235) in two launches: c0 [E,CH,H,W] = ofsMap(t), c1 [E,CH,H/2,W/2] =
+    ofs_residual(avg_pool2d(t, 2)) -> (off0, off1) [E,H,W,CH], channels-last and contiguous:
+    off0 = 4 tanh(norm(c0)), off1 = (4 tanh(norm(upsample(c1))) + off0) / 2, norm = per-edge standardisation over
+    (CH,H,W) with biased variance + eps (per_Corr_Normalization, corr.py:44-51).  With return_stats, also the per-edge
+    statistics [E,4] = (mean0, sigma0, mean1, sigma1), sigma = sqrt(var + eps), which offset_heads_backward takes."""
+    E, CH, H, W = _check_heads_inputs(c0, c1)
     off0 = torch.empty(E, H, W, CH, dtype=torch.float32, device=c0.device)
     off1 = torch.empty_like(off0)
     stats = torch.empty(E, 4, dtype=torch.float32, device=c0.device)
     _launch("lgu_offset_heads", c0.device, c0, c1, off0, off1, stats, E, CH, H, W, eps)
-    return off0, off1
+    return (off0, off1, stats) if return_stats else (off0, off1)
+
+
+def offset_heads_backward(c0, c1, stats, g_off0, g_off1):
+    """Backward of offset_heads in two launches: the forward's inputs c0, c1 and statistics, and the gradients of off0 /
+    off1 ([E,H,W,CH], either may be None = zero) -> (g_c0 [E,CH,H,W], g_c1 [E,CH,H/2,W/2]).  Bit-identical from run to
+    run (fp64 per-edge sums in a fixed order, no atomics)."""
+    E, CH, H, W = _check_heads_inputs(c0, c1)
+    _chk(stats, "stats", 2)
+    if tuple(stats.shape) != (E, 4):
+        raise RuntimeError(f"stats shape {tuple(stats.shape)} != {(E, 4)}")
+    grads = {k: v for k, v in (("g_off0", g_off0), ("g_off1", g_off1)) if v is not None}
+    _check_offsets(E * H * W * CH, **grads)
+    g_c0 = torch.empty_like(c0)
+    g_c1 = torch.empty_like(c1)
+    scratch = torch.empty(max(1, E * (H // 2) * (W // 32)) * 4, dtype=torch.float64, device=c0.device)
+    _launch_ext("lgu_offset_heads_backward", c0.device, c0, c1, stats, g_off0, g_off1, g_c0, g_c1, scratch, E, CH, H, W)
+    return g_c0, g_c1
 
 
 def pack_fmaps(fmaps, split=False):

@@ -9,10 +9,12 @@ num_steps x CorrBlock.__call__, backward to the feature maps and the offset / Ga
   acc      this repo, fused build + fused lookups, level gradients accumulated in persistent buffers (the default)
   dense    this repo, fused build + fused lookups, one dense gradient per lookup summed by autograd
   per_op   this repo's drop-in operators inside the reference's per-operator graph (fused=False)
+  acc_chain  `acc` with the offset heads' torch chain patched back in (permuted views, autograd backward): the same-process
+           comparison for corr.OffsetHeads
   ref_cuda the reference's OWN kernels recompiled unmodified for sm_100 (oracle/_ref) inside the same per-operator
            graph (skipped when oracle/_ref is absent)
 
-    python tools/bench_train.py [--batch 4] [--edges 24] [--steps 9] [--iters 3] [--arms acc,dense,per_op,ref_cuda]
+    python tools/bench_train.py [--batch 4] [--edges 24] [--steps 9] [--iters 3] [--arms acc,dense,per_op,acc_chain,ref_cuda]
 
 Prints one JSON line per arm (CUDA events around whole training steps, median).  Inputs are synthetic (fp32 maps, as
 in training), TF32 off.  The conv heads (ofsMap / ofs_residual, cuDNN) are part of every arm alike.
@@ -61,14 +63,15 @@ def main():
     params = list(ofsMap.parameters()) + list(ofs_residual.parameters()) + list(GA.parameters())
 
     real_ops = corr.ops
+    real_offsets = corr._generate_offsets
 
     def train_step(kind):
         f1, f2 = fm1.clone().requires_grad_(), fm2.clone().requires_grad_()
         for p in params:
             p.grad = None
-        fused = kind in ("acc", "dense")
+        fused = kind in ("acc", "dense", "acc_chain")
         blk = corr.CorrBlock(ofsMap, ofs_residual, GA, f1, f2, fused=fused, fused_lookup=fused,
-                             accumulate_grads=(kind == "acc"))
+                             accumulate_grads=(kind in ("acc", "acc_chain")))
         loss = 0.0
         for c, w in zip(coords, wts):
             out, mean_n, theta = blk(c)
@@ -85,6 +88,8 @@ def main():
                 print(json.dumps({"arm": kind, "unavailable": "oracle/_ref/defCorrSample_ref.so is absent"}))
                 continue
             corr.ops = ref                                   # the 6 operator names CorrBlock's per-op graph calls
+        if kind == "acc_chain":
+            corr._generate_offsets = lambda ofsMap, ofs_residual, t, fused_lookup=False: real_offsets(ofsMap, ofs_residual, t)
         try:
             torch.cuda.reset_peak_memory_stats()
             g1, _ = train_step(kind)
@@ -108,6 +113,7 @@ def main():
             print(json.dumps(line), flush=True)
         finally:
             corr.ops = real_ops
+            corr._generate_offsets = real_offsets
         torch.cuda.empty_cache()
 
 
