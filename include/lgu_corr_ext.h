@@ -34,6 +34,41 @@ LGU_API int lgu_offset_heads_backward(const float* c0, const float* c1, const fl
                               const float* g_off1, float* g_c0, float* g_c1, double* scratch,
                               int E, int CH, int H, int W, void* stream);
 
+/* The offset heads' 3x3 convolutions (ofsMap / ofs_residual: nn.Conv2d(C_in, C_out, 3, padding=1), stride 1, zero
+ * padding, bias) and their input and weight gradients, in fp32 accuracy on tensor cores: every product is
+ * hi*hi + hi*lo + lo*hi of tf32 hi / lo splits (~2^-21 relative), accumulated in fp32 in chunks of K = 128.
+ * Activations and gradients are NCHW fp32; the weight is [C_out, C_in, 3, 3] as nn.Conv2d holds it, packed by each
+ * call.  Sizes, checked by every entry point: C_in % 32 == 0, 0 < C_out <= 128, W % 32 == 0 with W dividing 128 or a
+ * multiple of 128, H*W % 128 == 0, E >= 0.  LGU_ERR_BAD_ARG names a NULL or misaligned pointer, a bad size or a short
+ * workspace before any device work; E = 0 is a no-op.  No float atomics: results are bit-identical from run to run. */
+
+/* Workspace bytes that any of the three operations below needs at these sizes (-1 for unsupported sizes). */
+LGU_API long long lgu_conv3x3_workspace_bytes(int E, int C_in, int C_out, int H, int W);
+
+/* x [E,C,H,W] -> tf32 hi / lo planes [E,H,W,Cp], channels-last, Cp = C rounded up to 32, padded channels 0.
+ * hi = x with the low 13 mantissa bits cleared, lo = x - hi; a +-inf or NaN x gives hi = 0, lo = x.
+ * hi, lo 16-byte aligned.  The forward packs x (C = C_in), the input gradient packs g_y (C = C_out). */
+LGU_API int lgu_conv3x3_pack(const float* x, float* hi, float* lo, int E, int C, int H, int W, void* stream);
+
+/* y [E,C_out,H,W] = conv3x3(x, weight) + bias, from x's planes (lgu_conv3x3_pack).  bias may be NULL (no bias).
+ * workspace: lgu_conv3x3_workspace_bytes, 256-byte aligned. */
+LGU_API int lgu_conv3x3_forward(const float* x_hi, const float* x_lo, const float* weight, const float* bias, float* y,
+                                void* workspace, long long workspace_bytes, int E, int C_in, int C_out, int H, int W,
+                                void* stream);
+
+/* g_x [E,C_in,H,W] = conv3x3(g_y, weight flipped and transposed), from g_y's planes (lgu_conv3x3_pack, C = C_out). */
+LGU_API int lgu_conv3x3_backward_input(const float* gy_hi, const float* gy_lo, const float* weight, float* g_x,
+                                       void* workspace, long long workspace_bytes, int E, int C_in, int C_out, int H,
+                                       int W, void* stream);
+
+/* g_w [C_out,C_in,3,3] = sum over e, y, x of g_y[e,co,y,x] x[e,ci,y+ky-1,x+kx-1] (x's planes from lgu_conv3x3_pack) and
+ * g_b [C_out] = sum of g_y over e, y, x (in fp64).  Either g_w or g_b may be NULL (not computed), not both; x_hi, x_lo
+ * and the workspace are read only for g_w.  The pixel sum is split over CTAs by a partition that depends only on the
+ * sizes, and the partial sums are added in a fixed order. */
+LGU_API int lgu_conv3x3_backward_weight(const float* x_hi, const float* x_lo, const float* g_y, float* g_w, float* g_b,
+                                        void* workspace, long long workspace_bytes, int E, int C_in, int C_out, int H,
+                                        int W, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -92,6 +92,11 @@ SIGNATURES = (
 # mirrors as released); tests/test_binding_ext_cpu.py keeps this table and that header in step.  Called via call_ext.
 EXT_SIGNATURES = (
     ("lgu_offset_heads_backward", _P * 8 + _I * 4 + _P),
+    ("lgu_conv3x3_workspace_bytes", _I * 5, ctypes.c_longlong),
+    ("lgu_conv3x3_pack", _P * 3 + _I * 4 + _P),
+    ("lgu_conv3x3_forward", _P * 6 + _LL + _I * 5 + _P),
+    ("lgu_conv3x3_backward_input", _P * 5 + _LL + _I * 5 + _P),
+    ("lgu_conv3x3_backward_weight", _P * 6 + _LL + _I * 5 + _P),
 )
 _RETURNS_STATUS = {name for name, _, *ret in SIGNATURES + EXT_SIGNATURES if not ret}
 _EXT_NAMES = {name for name, *_ in EXT_SIGNATURES}

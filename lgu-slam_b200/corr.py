@@ -11,7 +11,8 @@ instead.  What differs is underneath:
     the per-op path (`fused=False`) is kept and is what the fused path is tested against;
   * every lookup goes through the C ABI in include/lgu_corr.h; there is no CPU path.
 
-The learned heads (ofsMap / ofs_residual convs, the GaussianMask MLP) stay torch modules, as in the reference.
+The learned heads (ofsMap / ofs_residual convs, the GaussianMask MLP) stay torch modules, as in the reference;
+`OffsetConv` is an nn.Conv2d for the two offset convs that runs them on the library's tensor-core kernels.
 """
 import functools
 import math
@@ -258,6 +259,48 @@ class OffsetHeads(torch.autograd.Function):
         c0, c1, stats = ctx.saved_tensors
         return ops.offset_heads_backward(c0, c1, stats, None if g_off0 is None else g_off0.contiguous(),
                                          None if g_off1 is None else g_off1.contiguous())
+
+
+class OffsetConvFunction(torch.autograd.Function):
+    """conv3x3 (ops.conv3x3) as a differentiable op: forward = pack + implicit GEMM, backward = the input, weight and bias
+    gradients that autograd asks for, nothing else."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias):
+        ctx.save_for_backward(x, weight)
+        return ops.conv3x3(x, weight, bias)
+
+    @staticmethod
+    def backward(ctx, g_y):
+        x, weight = ctx.saved_tensors
+        need_x, need_w, need_b = ctx.needs_input_grad
+        return ops.conv3x3_backward(x, weight, g_y.contiguous(), need_x, need_w, need_b)
+
+
+class OffsetConv(nn.Conv2d):
+    """nn.Conv2d(in_channels, out_channels, 3, padding=1) -- the offset heads ofsMap / ofs_residual (droid_net.py) --
+    whose forward and backward run on the library's tensor-core kernels (OffsetConvFunction) in fp32 accuracy when the
+    input allows: a CUDA fp32 [E,C_in,H,W] tensor outside CUDA autocast, at sizes ops.conv3x3_supported accepts (both
+    grids of the heads, 48x64 and 24x32).  Any other input takes nn.Conv2d.forward unchanged.  Parameters and state_dict
+    are nn.Conv2d's, so the reference's checkpoints load."""
+
+    def __init__(self, in_channels, out_channels, device=None, dtype=None):
+        super().__init__(in_channels, out_channels, 3, stride=1, padding=1, dilation=1, groups=1, bias=True,
+                         padding_mode="zeros", device=device, dtype=dtype)
+
+    def _library_path(self, x):
+        w, b = self.weight, self.bias
+        return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 4
+                and not torch.is_autocast_enabled("cuda") and w.dtype == torch.float32 and w.device == x.device
+                and b is not None and b.dtype == torch.float32 and self.padding_mode == "zeros"
+                and tuple(self.kernel_size) == (3, 3) and tuple(self.stride) == (1, 1) and tuple(self.padding) == (1, 1)
+                and tuple(self.dilation) == (1, 1) and self.groups == 1 and x.shape[1] == self.in_channels
+                and ops.conv3x3_supported(self.in_channels, self.out_channels, x.shape[2], x.shape[3]))
+
+    def forward(self, x):
+        if self._library_path(x):
+            return OffsetConvFunction.apply(x.contiguous(), self.weight.contiguous(), self.bias.contiguous())
+        return super().forward(x)
 
 
 def per_Corr_Normalization(x, normalIndex, eps=1e-5):

@@ -291,6 +291,90 @@ def offset_heads_backward(c0, c1, stats, g_off0, g_off1):
     return g_c0, g_c1
 
 
+def _conv3x3_inputs(x, weight, bias=None):
+    """Checks of conv3x3 / conv3x3_backward: x [E,C_in,H,W], weight [C_out,C_in,3,3], bias [C_out] or None, contiguous
+    fp32 on one CUDA device, sizes the kernels implement."""
+    _chk(x, "x", 4); _chk(weight, "weight", 4)
+    E, C_in, H, W = x.shape
+    C_out = weight.shape[0]
+    if tuple(weight.shape) != (C_out, C_in, 3, 3):
+        raise RuntimeError(f"weight shape {tuple(weight.shape)} != {(C_out, C_in, 3, 3)}")
+    if bias is not None:
+        _chk(bias, "bias", 1)
+        if tuple(bias.shape) != (C_out,):
+            raise RuntimeError(f"bias shape {tuple(bias.shape)} != {(C_out,)}")
+    if any(t is not None and t.device != x.device for t in (weight, bias)):
+        raise RuntimeError("x, weight and bias must be on one device")
+    if not conv3x3_supported(C_in, C_out, H, W):
+        raise RuntimeError(f"conv3x3: unsupported sizes C_in={C_in} C_out={C_out} H={H} W={W} (needs C_in % 32 == 0, "
+                           "C_out <= 128, W % 32 == 0 dividing 128 or a multiple of 128, H*W % 128 == 0)")
+    return E, C_in, C_out, H, W
+
+
+def conv3x3_supported(C_in, C_out, H, W):
+    """Whether the conv3x3 kernels implement these sizes (OffsetConv takes the library path only then)."""
+    return (C_in > 0 and C_in % 32 == 0 and 0 < C_out <= 128 and W > 0 and W % 32 == 0
+            and (128 % W == 0 or W % 128 == 0) and H > 0 and (H * W) % 128 == 0)
+
+
+def _conv3x3_planes(t):
+    """NCHW fp32 -> tf32 hi / lo planes [E,H,W,round_up(C,32)] (lgu_conv3x3_pack)."""
+    E, C, H, W = t.shape
+    hi = torch.empty(E, H, W, (C + 31) // 32 * 32, dtype=torch.float32, device=t.device)
+    lo = torch.empty_like(hi)
+    _launch_ext("lgu_conv3x3_pack", t.device, t, hi, lo, E, C, H, W)
+    return hi, lo
+
+
+def _conv3x3_workspace(device, E, C_in, C_out, H, W):
+    nbytes = _lib.call_ext("lgu_conv3x3_workspace_bytes", E, C_in, C_out, H, W)
+    return torch.empty(max(1, nbytes), dtype=torch.uint8, device=device), nbytes
+
+
+def conv3x3(x, weight, bias=None):
+    """F.conv2d(x, weight, bias, padding=1) for a 3x3 kernel (the offset heads, ofsMap / ofs_residual) in fp32 accuracy
+    on tensor cores: x [E,C_in,H,W], weight [C_out,C_in,3,3], bias [C_out] or None -> y [E,C_out,H,W].  Two launches
+    pack x into tf32 hi / lo planes, then one packs the weight and one runs the implicit GEMM."""
+    E, C_in, C_out, H, W = _conv3x3_inputs(x, weight, bias)
+    y = torch.empty(E, C_out, H, W, dtype=torch.float32, device=x.device)
+    if E == 0:
+        return y
+    x_hi, x_lo = _conv3x3_planes(x)
+    ws, nbytes = _conv3x3_workspace(x.device, E, C_in, C_out, H, W)
+    _launch_ext("lgu_conv3x3_forward", x.device, x_hi, x_lo, weight, bias, y, ws, nbytes, E, C_in, C_out, H, W)
+    return y
+
+
+def conv3x3_backward(x, weight, g_y, need_input=True, need_weight=True, need_bias=None):
+    """Backward of conv3x3: the forward's x and weight and the output gradient g_y [E,C_out,H,W] -> (g_x [E,C_in,H,W],
+    g_w [C_out,C_in,3,3], g_b [C_out]), each None unless asked for (need_bias defaults to need_weight).  Bit-identical
+    from run to run (the weight gradient's pixel sum is split by the sizes alone and reduced in a fixed order)."""
+    E, C_in, C_out, H, W = _conv3x3_inputs(x, weight)
+    _chk(g_y, "g_y", 4)
+    if tuple(g_y.shape) != (E, C_out, H, W) or g_y.device != x.device:
+        raise RuntimeError(f"g_y shape {tuple(g_y.shape)} != {(E, C_out, H, W)} (on x's device)")
+    need_bias = need_weight if need_bias is None else need_bias
+    g_x = torch.empty_like(x) if need_input else None
+    g_w = torch.empty_like(weight) if need_weight else None
+    g_b = torch.empty(C_out, dtype=torch.float32, device=x.device) if need_bias else None
+    if E == 0:
+        for t in (g_x, g_w, g_b):
+            if t is not None:
+                t.zero_()
+        return g_x, g_w, g_b
+    if not (need_input or need_weight or need_bias):
+        return g_x, g_w, g_b
+    ws, nbytes = _conv3x3_workspace(x.device, E, C_in, C_out, H, W)
+    if need_input:
+        gy_hi, gy_lo = _conv3x3_planes(g_y)
+        _launch_ext("lgu_conv3x3_backward_input", x.device, gy_hi, gy_lo, weight, g_x, ws, nbytes, E, C_in, C_out, H, W)
+        del gy_hi, gy_lo
+    if need_weight or need_bias:
+        x_hi, x_lo = _conv3x3_planes(x) if need_weight else (None, None)
+        _launch_ext("lgu_conv3x3_backward_weight", x.device, x_hi, x_lo, g_y, g_w, g_b, ws, nbytes, E, C_in, C_out, H, W)
+    return g_x, g_w, g_b
+
+
 def pack_fmaps(fmaps, split=False):
     """fmaps [T,C,H,W] (fp32 or fp16 CUDA, as the encoders emit) -> channels-last fp16 planes for the
     tcgen05 build: hi [T,H*W,C] = fp16(x/4) and, if split, lo = fp16(x/4 - hi) (else None).

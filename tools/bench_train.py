@@ -11,13 +11,15 @@ num_steps x CorrBlock.__call__, backward to the feature maps and the offset / Ga
   per_op   this repo's drop-in operators inside the reference's per-operator graph (fused=False)
   acc_chain  `acc` with the offset heads' torch chain patched back in (permuted views, autograd backward): the same-process
            comparison for corr.OffsetHeads
+  acc_conv `acc` with corr.OffsetConv heads (the same parameters): the offset convolutions on the library's tensor-core
+           kernels instead of cuDNN fp32
   ref_cuda the reference's OWN kernels recompiled unmodified for sm_100 (oracle/_ref) inside the same per-operator
            graph (skipped when oracle/_ref is absent)
 
-    python tools/bench_train.py [--batch 4] [--edges 24] [--steps 9] [--iters 3] [--arms acc,dense,per_op,acc_chain,ref_cuda]
+    python tools/bench_train.py [--batch 4] [--edges 24] [--steps 9] [--iters 3] [--arms acc,dense,per_op,acc_chain,acc_conv,ref_cuda]
 
 Prints one JSON line per arm (CUDA events around whole training steps, median).  Inputs are synthetic (fp32 maps, as
-in training), TF32 off.  The conv heads (ofsMap / ofs_residual, cuDNN) are part of every arm alike.
+in training), TF32 off.  The conv heads (ofsMap / ofs_residual, cuDNN fp32) are part of every arm alike, except acc_conv.
 """
 import argparse
 import json
@@ -60,7 +62,10 @@ def main():
     ofsMap = nn.Conv2d(256, 98, 3, padding=1).to(dev)
     ofs_residual = nn.Conv2d(256, 98, 3, padding=1).to(dev)
     GA = corr.GaussianMask(H, W).to(dev)
-    params = list(ofsMap.parameters()) + list(ofs_residual.parameters()) + list(GA.parameters())
+    conv_heads = [corr.OffsetConv(256, 98).to(dev) for _ in range(2)]
+    for h, ref_h in zip(conv_heads, (ofsMap, ofs_residual)):
+        h.load_state_dict(ref_h.state_dict())
+    params = [p for m in (ofsMap, ofs_residual, GA, *conv_heads) for p in m.parameters()]
 
     real_ops = corr.ops
     real_offsets = corr._generate_offsets
@@ -69,9 +74,10 @@ def main():
         f1, f2 = fm1.clone().requires_grad_(), fm2.clone().requires_grad_()
         for p in params:
             p.grad = None
-        fused = kind in ("acc", "dense", "acc_chain")
-        blk = corr.CorrBlock(ofsMap, ofs_residual, GA, f1, f2, fused=fused, fused_lookup=fused,
-                             accumulate_grads=(kind in ("acc", "acc_chain")))
+        fused = kind in ("acc", "dense", "acc_chain", "acc_conv")
+        heads = conv_heads if kind == "acc_conv" else (ofsMap, ofs_residual)
+        blk = corr.CorrBlock(*heads, GA, f1, f2, fused=fused, fused_lookup=fused,
+                             accumulate_grads=(kind in ("acc", "acc_chain", "acc_conv")))
         loss = 0.0
         for c, w in zip(coords, wts):
             out, mean_n, theta = blk(c)
@@ -110,6 +116,8 @@ def main():
                     "fmap1_grad_rms": float(g1.square().mean().sqrt())}
             if "per_op" in results and kind != "per_op":
                 line["fmap1_grad_max_err_vs_per_op"] = float((g1 - results["per_op"]).abs().max())
+            if kind == "acc_conv" and "acc" in results:
+                line["fmap1_grad_max_err_vs_acc"] = float((g1 - results["acc"]).abs().max())
             print(json.dumps(line), flush=True)
         finally:
             corr.ops = real_ops
