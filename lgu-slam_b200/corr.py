@@ -881,7 +881,9 @@ class AltCorrBlock:
         outs, masks, new_off1 = [], [], []
         for s, s_end in bounds:
             e = slice(s, s_end)
-            vols = ent["vols"].get(s) if ent is not None else None
+            # keyed by the pass's edge range: a later call with another pass schedule must not pick up volumes built
+            # for different edges
+            vols = ent["vols"].get((s, s_end)) if ent is not None else None
             boxes0 = None
             if vols is None:
                 # Level 0 is 3/4 of the volume bytes, and the lookup below reads it only inside a 20 x 16 box per source
@@ -899,7 +901,7 @@ class AltCorrBlock:
                         for l in range(self.num_levels)]
                 nbytes = sum(v.numel() * 4 for v in vols if v is not None)
                 if ent is not None and self._vol_bytes + nbytes <= self._vol_budget:
-                    ent["vols"][s] = vols
+                    ent["vols"][(s, s_end)] = vols
                     self._vol_bytes += nbytes
             # out / out_index: this pass's edges are written straight to their rows of the caller's buffer
             dst = dict(out=out, out_index=(out_index[e].contiguous() if out_index is not None else

@@ -738,6 +738,8 @@ def _altcorr_inputs(volumes, coords, off0, off1, shared_offsets, boxes0, boxes1,
     boxed = [l for l, bx in enumerate((boxes0, boxes1)) if bx is not None]
     _check_levels(volumes, E, H, W, "volumes", skip=boxed)
     _chk(coords, "coords", 4)
+    if tuple(coords.shape) != (E, H, W, 2):                   # the kernels index coords with the volumes' E, H, W
+        raise RuntimeError(f"coords must be [E,H,W,2] = {[E, H, W, 2]}, got {list(coords.shape)}")
     _check_offsets(H * W * 98 * (1 if shared_offsets else E), exact=False, off0=off0, off1=off1)
     if out is None:
         out, out_index = torch.empty(E, C, H, W, dtype=out_dtype, device=coords.device), None
