@@ -1,4 +1,5 @@
 // abi.cu -- library identification + error plumbing of the C ABI (include/lgu_corr.h).
+#include <array>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -54,39 +55,87 @@ int optin_smem(const void* kernel, int bytes, const char* who) {
 }
 
 namespace {
+// The device, then every argument that reaches the encoder: rank-dependent entries past `rank` stay zero.
+constexpr int kMaxRank = 5;
+typedef std::array<uint64_t, 6 + 3 * kMaxRank> MapKey;
 struct KeyHash {
   size_t operator()(const MapKey& k) const {
     uint64_t h = 1469598103934665603ull;
-    for (uint64_t x : k.v) h = (h ^ x) * 1099511628211ull;
+    for (uint64_t x : k) h = (h ^ x) * 1099511628211ull;
     return (size_t)h;
   }
 };
-struct KeyEq {
-  bool operator()(const MapKey& a, const MapKey& b) const { return memcmp(a.v, b.v, sizeof(a.v)) == 0; }
-};
-struct Map128 {
-  unsigned char b[128];
-};
 constexpr size_t kMapCacheMax = 512;
-std::unordered_map<MapKey, Map128, KeyHash, KeyEq>& map_cache() {
-  static std::unordered_map<MapKey, Map128, KeyHash, KeyEq> c;
-  return c;
-}
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 }  // namespace
 
-bool map_cache_get(const MapKey& key, void* map128) {
+int encode_tensor_map(CUtensorMap* map, CUtensorMapDataType dt, int rank, const void* base, const uint64_t* dims,
+                      const uint64_t* strides_bytes, const uint32_t* box, CUtensorMapSwizzle swz, CUtensorMapL2promotion l2) {
+  static std::unordered_map<MapKey, CUtensorMap, KeyHash> cache;
+  static const EncodeTiledFn encode = [] {                       // resolved once; static initialisation is thread-safe
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+                    q == cudaDriverEntryPointSuccess;
+    return ok ? reinterpret_cast<EncodeTiledFn>(p) : nullptr;
+  }();
+  if (rank < 1 || rank > kMaxRank) {
+    set_error("encode_tensor_map: rank %d is outside 1..%d", rank, kMaxRank);
+    return LGU_ERR_LAUNCH;
+  }
+  int dev = 0;
+  cudaGetDevice(&dev);
+  MapKey key{(uint64_t)dev, (uint64_t)reinterpret_cast<uintptr_t>(base), (uint64_t)dt, (uint64_t)rank, (uint64_t)swz,
+             (uint64_t)l2};
+  for (int i = 0; i < rank; ++i) {
+    key[6 + i] = dims[i];
+    key[6 + kMaxRank + i] = box[i];
+  }
+  for (int i = 0; i + 1 < rank; ++i) key[6 + 2 * kMaxRank + i] = strides_bytes[i];
+  {
+    std::lock_guard<std::mutex> lk(g_plumb_mutex);
+    auto it = cache.find(key);
+    if (it != cache.end()) {
+      *map = it->second;
+      return LGU_OK;
+    }
+  }
+  if (encode == nullptr) {
+    set_error("cuTensorMapEncodeTiled is not available from the driver");
+    return LGU_ERR_LAUNCH;
+  }
+  const cuuint32_t elem_strides[kMaxRank] = {1, 1, 1, 1, 1};
+  const CUresult r = encode(map, dt, (cuuint32_t)rank, const_cast<void*>(base), dims, strides_bytes, box, elem_strides,
+                            CU_TENSOR_MAP_INTERLEAVE_NONE, swz, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    char d[128];
+    int n = 0;
+    for (int i = 0; i < rank; ++i) n += snprintf(d + n, sizeof(d) - n, i ? " x %llu" : "%llu", (unsigned long long)dims[i]);
+    set_error("cuTensorMapEncodeTiled failed with CUresult %d (rank %d, dims %s)", (int)r, rank, d);
+    return LGU_ERR_LAUNCH;
+  }
   std::lock_guard<std::mutex> lk(g_plumb_mutex);
-  auto it = map_cache().find(key);
-  if (it == map_cache().end()) return false;
-  memcpy(map128, it->second.b, 128);
-  return true;
+  if (cache.size() >= kMapCacheMax) cache.clear();               // geometry churn: start over (maps are cheap to redo)
+  cache[key] = *map;
+  return LGU_OK;
 }
-void map_cache_put(const MapKey& key, const void* map128) {
+
+int num_sms() {
+  struct Known { int dev, sms; };
+  static std::vector<Known> known;
+  int dev = 0, sms = 0;
+  cudaGetDevice(&dev);
+  {
+    std::lock_guard<std::mutex> lk(g_plumb_mutex);
+    for (const auto& k : known)
+      if (k.dev == dev) return k.sms;
+  }
+  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return kNumSMs;
   std::lock_guard<std::mutex> lk(g_plumb_mutex);
-  if (map_cache().size() >= kMapCacheMax) map_cache().clear();   // geometry churn: start over (maps are cheap to redo)
-  Map128 m;
-  memcpy(m.b, map128, 128);
-  map_cache()[key] = m;
+  known.push_back({dev, sms});
+  return sms;
 }
 }  // namespace lgu
 

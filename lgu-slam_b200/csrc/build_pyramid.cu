@@ -449,9 +449,7 @@ static int launch_build(const CUtensorMap& mh, const CUtensorMap& ml, const CUte
   using Cfg = BpCfg<PREC>;
   auto kern = build_pyramid_kernel<PREC>;
   if (int rc = optin_smem(reinterpret_cast<const void*>(kern), Cfg::kSmemBytes, "lgu_build_pyramid")) return rc;
-  int dev = 0, sms = kNumSMs;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int grid = prm.num_units < sms ? prm.num_units : sms;
   kern<<<grid, kBpThreads, Cfg::kSmemBytes, st>>>(mh, ml, mbh, mbl, m0, m1, prm);
   return check_launch("lgu_build_pyramid");

@@ -394,9 +394,7 @@ build_pyramid16_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_
 int launch_build16(const CUtensorMap& mh, const CUtensorMap& mb, const BpParams& prm, bool flat, cudaStream_t st) {
   auto kern = flat ? build_pyramid16_kernel<true> : build_pyramid16_kernel<false>;
   if (int rc = optin_smem(reinterpret_cast<const void*>(kern), b16::kSmemBytes, "lgu_build_pyramid")) return rc;
-  int dev = 0, sms = kNumSMs;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int grid = prm.num_units < sms ? prm.num_units : sms;
   kern<<<grid, b16::kThreads, b16::kSmemBytes, st>>>(mh, mb, prm);
   return check_launch(flat ? "lgu_build_volume(16)" : "lgu_build_pyramid(16)");

@@ -1,5 +1,6 @@
 // common.cuh -- shared helpers for the sm_100a correlation kernels.
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "../../include/lgu_corr.h"
@@ -24,14 +25,15 @@ constexpr int kNumSMs = 148;  // B200: 2 dies x 74 SMs
 
 // Host-side launch plumbing that is paid ONCE, not per call (abi.cu):
 //  * the opt-in to more than 48 KB of dynamic shared memory is a per-(device, kernel) function attribute;
-//  * a CUtensorMap depends only on (device, base pointer, geometry): encoded maps are kept in a small table, so the
-//    steady state of a frontend / backend loop (same pyramid storage, same shapes) re-encodes nothing.
+//  * a CUtensorMap depends only on the device and the encoder's arguments: encoded maps are kept in a small table, so the
+//    steady state of a frontend / backend loop (same pyramid storage, same shapes) re-encodes nothing;
+//  * the SM count that sizes the persistent grids is read once per device (kNumSMs if the query fails).
 int optin_smem(const void* kernel, int bytes, const char* who);
-struct MapKey {
-  uint64_t v[12];
-};
-bool map_cache_get(const MapKey& key, void* map128);          // map128: CUtensorMap (128 bytes)
-void map_cache_put(const MapKey& key, const void* map128);
+// Tiled map of a tensor of rank <= 5: dims innermost first, strides_bytes of dims 1 .. rank-1, element strides 1, no
+// interleave, out-of-bounds elements read as zero.
+int encode_tensor_map(CUtensorMap* map, CUtensorMapDataType dt, int rank, const void* base, const uint64_t* dims,
+                      const uint64_t* strides_bytes, const uint32_t* box, CUtensorMapSwizzle swz, CUtensorMapL2promotion l2);
+int num_sms();
 
 __device__ __forceinline__ bool in_bounds(int h, int w, int H, int W) {
   return h >= 0 && h < H && w >= 0 && w < W;

@@ -520,41 +520,13 @@ __global__ void __launch_bounds__(256) conv_bias_grad_kernel(const float* __rest
 // ---------------------------------------------------------------------------------------------
 static inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 
-// Row-major tensor of 3 or 4 fp32 dimensions (dims innermost first, dense), box `box`, cached like make_map_2d.
+// Row-major tensor of 3 or 4 fp32 dimensions (dims innermost first, dense), box `box`.
 static int make_map_nd(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint32_t* box,
                        CUtensorMapSwizzle swz) {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  MapKey key = {{(uint64_t)(16 + rank), (uint64_t)dev, (uint64_t)reinterpret_cast<uintptr_t>(base), (uint64_t)swz, 0, 0, 0, 0,
-                 0, 0, 0, 0}};
-  for (int i = 0; i < rank; ++i) {
-    key.v[4 + i] = dims[i];
-    key.v[8] |= (uint64_t)box[i] << (16 * i);
-  }
-  if (map_cache_get(key, map)) return LGU_OK;
-  EncodeTiledFn fn = get_encode_fn();
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return LGU_ERR_LAUNCH;
-  }
-  cuuint64_t gd[4], gs[3];
-  cuuint32_t bx[4], es[4];
-  uint64_t stride = 4;
-  for (int i = 0; i < rank; ++i) {
-    gd[i] = dims[i];
-    bx[i] = box[i];
-    es[i] = 1;
-    if (i > 0) gs[i - 1] = stride;
-    stride *= dims[i];
-  }
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed with CUresult %d (rank %d)", (int)r, rank);
-    return LGU_ERR_LAUNCH;
-  }
-  map_cache_put(key, map);
-  return LGU_OK;
+  uint64_t strides[3] = {dims[0] * 4, 0, 0};
+  for (int i = 1; i + 1 < rank; ++i) strides[i] = strides[i - 1] * dims[i];
+  return encode_tensor_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank, base, dims, strides, box, swz,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
 }
 
 struct ConvShape {

@@ -116,77 +116,13 @@ struct FusedMaps {
   CUtensorMap m[4];
 };
 
-typedef CUresult (*FlEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
+// The slices [nslices, H2, W2] of a pyramid level as a 3-D fp32 tensor, box bw x bh of one slice, no swizzle.
 static inline int make_slice_map(CUtensorMap* map, const float* base, long long nslices, int H2, int W2, int bw, int bh) {
-  static_assert(sizeof(CUtensorMap) == 128, "CUtensorMap is expected to be 128 bytes");
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const MapKey key = {{1u, (uint64_t)dev, (uint64_t)reinterpret_cast<uintptr_t>(base), (uint64_t)nslices, (uint64_t)H2,
-                       (uint64_t)W2, (uint64_t)bw, (uint64_t)bh, 0, 0, 0, 0}};
-  if (map_cache_get(key, map)) return LGU_OK;
-  static FlEncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<FlEncodeTiledFn>(p);
-  }
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return LGU_ERR_LAUNCH;
-  }
-  const cuuint64_t dims[3] = {(cuuint64_t)W2, (cuuint64_t)H2, (cuuint64_t)nslices};
-  const cuuint64_t strides[2] = {(cuuint64_t)W2 * 4, (cuuint64_t)W2 * H2 * 4};
-  const cuuint32_t box[3] = {(cuuint32_t)bw, (cuuint32_t)bh, 1};
-  const cuuint32_t es[3] = {1, 1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed with CUresult %d (slices=%lld H2=%d W2=%d box=%dx%d)", (int)r, nslices, H2,
-              W2, bw, bh);
-    return LGU_ERR_LAUNCH;
-  }
-  map_cache_put(key, map);
-  return LGU_OK;
-}
-
-// Row-major fp32 matrix [rows, cols] as a 2-D tensor, box = [box_rows, box_cols] (box_cols * 4 a multiple of 16), no swizzle.
-static inline int make_rows_map(CUtensorMap* map, const float* base, long long rows, long long cols, int box_cols, int box_rows) {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const MapKey key = {{4u, (uint64_t)dev, (uint64_t)reinterpret_cast<uintptr_t>(base), (uint64_t)rows, (uint64_t)cols,
-                       (uint64_t)box_cols, (uint64_t)box_rows, 0, 0, 0, 0, 0}};
-  if (map_cache_get(key, map)) return LGU_OK;
-  static FlEncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<FlEncodeTiledFn>(p);
-  }
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return LGU_ERR_LAUNCH;
-  }
-  const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  const cuuint64_t strides[1] = {(cuuint64_t)cols * 4};
-  const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  const cuuint32_t es[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed with CUresult %d (rows=%lld cols=%lld box=%dx%d)", (int)r, rows, cols, box_rows, box_cols);
-    return LGU_ERR_LAUNCH;
-  }
-  map_cache_put(key, map);
-  return LGU_OK;
+  const uint64_t dims[3] = {(uint64_t)W2, (uint64_t)H2, (uint64_t)nslices};
+  const uint64_t strides[2] = {(uint64_t)W2 * 4, (uint64_t)W2 * H2 * 4};
+  const uint32_t box[3] = {(uint32_t)bw, (uint32_t)bh, 1};
+  return encode_tensor_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE,
+                           CU_TENSOR_MAP_L2_PROMOTION_NONE);
 }
 
 }  // namespace lgu

@@ -902,7 +902,10 @@ static int lgu::launch_lookup_fused_bwd(const float* lvl0, const float* lvl1, co
     if (rc) return rc;
   }
   {  // the upstream gradient [E*196, P] as a 2-D tensor: one box = 196 channel rows x 4 pixels (this warp's strip)
-    const int rc = make_rows_map(&maps.m[2], corr_grad, (long long)E * fl::CH, P, fl::kPixPerWarp, fl::CH);
+    const uint64_t dims[2] = {(uint64_t)P, (uint64_t)E * fl::CH}, strides[1] = {(uint64_t)P * 4};
+    const uint32_t box[2] = {fl::kPixPerWarp, fl::CH};
+    const int rc = encode_tensor_map(&maps.m[2], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, corr_grad, dims, strides, box,
+                                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE);
     if (rc) return rc;
   }
   maps.m[3] = maps.m[0];
@@ -921,9 +924,7 @@ static int lgu::launch_lookup_fused_bwd(const float* lvl0, const float* lvl1, co
   const long long ntiles = (long long)E * prm.tiles_per_edge;
   LGU_REQUIRE(ntiles < 2147483647LL, "lgu_corr_lookup_fused_backward: too many tiles (%lld)", ntiles);
   prm.num_tiles = (int)ntiles;
-  int dev = 0, sms = kNumSMs;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   // Schedule.  Accumulate mode (footprint-only reductions): persistent, two CTAs per SM, every CTA the same number of
   // tiles (4608 tiles -> 288 CTAs x 16) -- 431 -> 373 us at E = 48.  Dense mode (every slice streamed once, write-bound):
   // one tile per CTA -- persistent CTAs run in lock step and write in phase (690 us against 601 us); the hardware's CTA

@@ -152,49 +152,13 @@ __host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N) {
 // ---------------------------------------------------------------------------------------------
 // Host side: tensor maps
 // ---------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static inline EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
-// 2-D row-major tensor [rows, cols] of `elem_bytes`-byte elements, box [box_rows, box_cols], 128B swizzle.
+// 2-D row-major tensor [rows, cols] of `elem_bytes`-byte elements, box [box_rows, box_cols], 128B swizzle by default.
 static inline int make_map_2d(CUtensorMap* map, CUtensorMapDataType dt, int elem_bytes, const void* base, uint64_t rows,
                        uint64_t cols, uint32_t box_rows, uint32_t box_cols,
                        CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B) {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const MapKey key = {{2u, (uint64_t)dev, (uint64_t)reinterpret_cast<uintptr_t>(base), (uint64_t)dt, (uint64_t)elem_bytes,
-                       rows, cols, box_rows, box_cols, (uint64_t)swz, 0, 0}};
-  if (map_cache_get(key, map)) return LGU_OK;
-  EncodeTiledFn fn = get_encode_fn();
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return LGU_ERR_LAUNCH;
-  }
-  const cuuint64_t dims[2] = {cols, rows};
-  const cuuint64_t strides[1] = {cols * (uint64_t)elem_bytes};
-  const cuuint32_t box[2] = {box_cols, box_rows};
-  const cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, dt, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed with CUresult %d (rows=%llu cols=%llu)", (int)r,
-              (unsigned long long)rows, (unsigned long long)cols);
-    return LGU_ERR_LAUNCH;
-  }
-  map_cache_put(key, map);
-  return LGU_OK;
+  const uint64_t dims[2] = {cols, rows}, strides[1] = {cols * (uint64_t)elem_bytes};
+  const uint32_t box[2] = {box_cols, box_rows};
+  return encode_tensor_map(map, dt, 2, base, dims, strides, box, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
 }
 
 }  // namespace lgu
