@@ -57,7 +57,9 @@ __device__ __forceinline__ void gauss_window_grads(const float (&v)[3], const fl
     float vraw = v[ps];
     if (FUSED) {
       vraw = __fdividef(v[ps], __fmaf_rn(__fmul_rn(k3, cE), rE, 1.0f));   // the raw volume (== v outside the window)
-      if (live) gd = __fmaf_rn(g[ps], __fsub_rn(v[ps], vraw), gd);
+      // the residual corr1 / den = v - vraw, formed as vraw 3 e / den: the difference cancels to a few bits where e is
+      // small (a window far from its mean keeps 2^-24 / (3 e / den) of its relative accuracy)
+      if (live) gd = __fmaf_rn(g[ps], __fmul_rn(vraw, __fmul_rn(__fmul_rn(k3, cE), rE)), gd);
     }
     const float w = live ? __fmul_rn(__fmul_rn(vraw, 3.0f), g[ps]) : 0.0f;
     const float wa = __fmul_rn(w, rE), wb = __fmul_rn(w, cE);

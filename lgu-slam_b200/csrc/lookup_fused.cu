@@ -394,7 +394,8 @@ lookup_fused_kernel(const __grid_constant__ FusedMaps maps, const FusedLookupPar
         const float mm = prm.cum_mask != nullptr ? __fmul_rn(cum, m) : m;
         if (lane >= 17) o[1] = make_float2(__fmul_rn(o[1].x, mm), __fmul_rn(o[1].y, mm));
         o[2] = make_float2(__fmul_rn(o[2].x, mm), __fmul_rn(o[2].y, mm));
-        o[3] = make_float2(__fmul_rn(o[3].x, mm), __fmul_rn(o[3].y, mm));       // lanes >= 2 hold zeros
+        // lanes >= 2 are level-2 taps: their zero offsets stay zero (0 * a NaN mask would move them to F2I(NaN) = 0)
+        if (lane < 2) o[3] = make_float2(__fmul_rn(o[3].x, mm), __fmul_rn(o[3].y, mm));
         if (prm.cum_mask != nullptr) {
           if (lane == 0) prm.cum_mask[(size_t)ns * P + p] = mm;
         } else {

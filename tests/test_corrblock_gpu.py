@@ -339,8 +339,10 @@ def test_training_clip_fused_lookup_equals_per_op_autograd(accumulate):
         assert (a - bb).abs().max().item() <= 2e-5, f"lookup {k}"
     names = ("fmap1", "fmap2", "ofsMap.weight", "ofs_residual.weight", "GA.map.weight", "GA.covMap.weight",
              "GA.meanMap.weight")
-    # both graphs are pinned directly against the reference's compiled kernels in tests/test_dropin_gpu.py; here the two
-    # paths of this repo must agree to the same bar: |err| <= 1e-5 * max(1, max|per-op gradient|)
+    # the fused path -- build, lookups, their backward and the training chain's leaf gradients (maps, mean / cov / det,
+    # offsets) -- is judged against an fp64 statement in tests/test_frontend_scale_gpu.py, which also checks that
+    # CorrBlock(fused=True) wires its modules into those ops.  Here the two paths of this repo must agree:
+    # |err| <= 1e-5 * max(1, max|per-op gradient|)
     # (learned-parameter gradients are cuDNN / cuBLAS reductions of the per-pixel gradients over N = E*H*W positions:
     # rounding-level differences of the summands accumulate as sqrt(N) -> 8 * 2^-24 * sqrt(N) relative, see test_dropin_gpu)
     n_pos = b * n * 48 * 64

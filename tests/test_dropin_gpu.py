@@ -14,6 +14,10 @@ unmodified modules are executed three ways in one process:
 Compared: outputs over >= 3 consecutive calls (cumulative offset[1] mask, quirk Q7), the in-place offset state
 (quirk Q5), and every autograd gradient (feature maps, offset heads, Gaussian head).
 
+The whole file skips unless oracle/_ref has been built and staged.  Without it, the fused build, lookup, lookup
+backward and training chain at the bench shape are judged against the float64 statement in tests/frontend_ref.py
+(tests/test_frontend_scale_gpu.py), and that statement against the CPU oracle (tests/test_frontend_reference_cpu.py).
+
 Bars (fp32): forward values of A vs B bit-exact (same torch glue, bit-exact kernels); everything else
 |err| <= 1e-5 * max(1, max|reference|) -- 1e-5 abs for the O(1) quantities the contract names, the same 1e-5 relative
 to the tensor's largest entry where accumulated values exceed 1 (fp32 cannot resolve 1e-5 abs beyond |v| ~ 100).
